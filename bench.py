@@ -3,6 +3,7 @@
 
     python bench.py --gpus N --steps K --warmup W            # this repo's CUDA path
     python bench.py --impl reference --gpus N --steps K ...   # reference CPU implementation (oracle port)
+    python bench.py ... --dump-outputs DIR                    # + the last timed step's tokens / log-probabilities as .npy
 
 One "step" = one batch of synthetic 6 x 224 x 224 clips through the whole path: CLIP ViT-B/16 encode with temporal
 embeddings, decoder pass over the visual tokens (K/V cache fill), 14 greedy decode steps (beam_size=1, max_steps=15,
@@ -97,7 +98,8 @@ class ClockSampler:
 def run_reference_cpu(steps: int, warmup: int, clips_per_step: int = 1):
     """Reference CPU implementation of the path = the oracle port in reference-faithful mode (per-frame ViT calls,
     hidden-state history with per-step K/V re-projection, Python search loop, per-step logits -> numpy), fp32, all host
-    threads (BASELINE.md section 4; the reference itself cannot be imported: SURVEY.md 8c)."""
+    threads (BASELINE.md section 4; the reference itself cannot be imported: SURVEY.md 8c).  The result's "outputs" are
+    the last step's (tokens [clips, 1, 15], logprobs [clips, 1])."""
     import torch
     from oracle import git_oracle as go
     from oracle import search_oracle as so
@@ -111,13 +113,14 @@ def run_reference_cpu(steps: int, warmup: int, clips_per_step: int = 1):
     with torch.no_grad():
         for i in range(warmup + steps):
             t0 = time.perf_counter()
-            for c in clips:  # the reference captions one clip at a time (model.py:765-770)
-                so.caption_clip(sd, cfg, c, per_frame_calls=True, beam_size=1, max_steps=15)
+            # the reference captions one clip at a time (model.py:765-770)
+            res = [so.caption_clip(sd, cfg, c, per_frame_calls=True, beam_size=1, max_steps=15) for c in clips]
             dt = time.perf_counter() - t0
             if i >= warmup:
                 times.append(dt)
     total = sum(times)
-    return {"value": clips_per_step * len(times) / total, "ms_per_step": 1e3 * total / len(times),
+    outputs = (torch.cat([r["predictions"] for r in res])[:, None], torch.cat([r["logprobs"] for r in res]))
+    return {"value": clips_per_step * len(times) / total, "ms_per_step": 1e3 * total / len(times), "outputs": outputs,
             "cores": torch.get_num_threads(), "p50_ms": 1e3 * statistics.median(times) / clips_per_step,
             "sample": f"{len(times)} steps x {clips_per_step} clip(s), greedy (beam 1, max_steps 15), fp32, after {warmup} warm-up"}
 
@@ -142,6 +145,15 @@ def emit(line: dict) -> None:
         os.write(1, data)
     else:
         os.write(_JSON_FD, data)
+
+
+def dump_outputs(out_dir: str, tokens, logprobs) -> None:
+    """tokens [clips, keep, max_steps] (integer ids) -> tokens.npy (float64: every int32 id exactly); logprobs [clips, keep] ->
+    logprobs.npy (float32).  At the default geometry that is 512 x 15 tokens and 512 scores per GPU, well under 1 MB."""
+    import numpy as np
+    os.makedirs(out_dir, exist_ok=True)
+    np.save(os.path.join(out_dir, "tokens.npy"), tokens.cpu().numpy().astype(np.float64))
+    np.save(os.path.join(out_dir, "logprobs.npy"), logprobs.cpu().numpy().astype(np.float32))
 
 
 def pin_rank_to_cores(local_rank: int, world: int):
@@ -369,11 +381,22 @@ def distill_leg(g, gm, torch, dist, world, rank, local_rank, dev, steps=10, warm
     return out
 
 
+def _count(least: int):
+    """argparse type: an integer >= least."""
+    def parse(text: str) -> int:
+        v = int(text)
+        if v < least:
+            raise argparse.ArgumentTypeError(f"must be >= {least}, got {v}")
+        return v
+    return parse
+
+
 def main():
     ap = argparse.ArgumentParser()
     ap.add_argument("--gpus", type=int, default=1)
-    ap.add_argument("--steps", type=int, default=6)
-    ap.add_argument("--warmup", type=int, default=3)
+    ap.add_argument("--steps", type=_count(1), default=6, help="timed steps (>= 1)")
+    ap.add_argument("--warmup", type=_count(0), default=3, help="warm-up steps before the timed ones (the CUDA arm runs at least 4: "
+                    "each of its two frame buffers is captured into CUDA graphs on its second use)")
     ap.add_argument("--impl", default="b200", choices=["b200", "reference"])
     ap.add_argument("--batch", type=int, default=512, help="clips per GPU per step (512: +3.5 %% over 256, the decode-step weights amortise over more rows)")
     ap.add_argument("--beam", type=int, default=1)
@@ -391,6 +414,10 @@ def main():
     ap.add_argument("--early-exit", type=int, default=-1, help="poll the device's finished-clip count every N decode steps (-1: library default 4; 0: never)")
     ap.add_argument("--fuse-ln", action="store_true", help="opt-in: LayerNorms written by the residual GEMMs as a second output (DESIGN.md dead ends)")
     ap.add_argument("--no-graphs", action="store_true", help="A/B: eager launches instead of the CUDA graphs of encode / visual pass / decode segments")
+    ap.add_argument("--dump-outputs", metavar="DIR", help="write the last timed step's result to DIR/tokens.npy and "
+                    "DIR/logprobs.npy, so that two builds can be compared output for output on the same seeded weights and clips: "
+                    "all ranks' caption tokens and log-probabilities as the token gather returns them (with --impl reference: the "
+                    "oracle's caption of its one clip, whose weights and clip are seeded apart from the CUDA arm's)")
     args = ap.parse_args()
     claim_stdout()
 
@@ -413,11 +440,11 @@ def main():
     if args.impl == "reference":
         if rank != 0:
             return 0
-        warm = max(1, min(args.warmup, 1))
-        steps = max(1, min(args.steps, 5))
-        r = run_reference_cpu(steps, warm, 1)
-        line = {"impl": "reference", "metric": METRIC, "value": r["value"], "unit": UNIT, "n_gpus": args.gpus, "steps": steps,
-                "warmup": warm, "ms_per_step": r["ms_per_step"], "higher_is_better": True, "scaling": "weak", "vs_baseline": None,
+        r = run_reference_cpu(args.steps, args.warmup, 1)
+        if args.dump_outputs:
+            dump_outputs(args.dump_outputs, *r["outputs"])
+        line = {"impl": "reference", "metric": METRIC, "value": r["value"], "unit": UNIT, "n_gpus": args.gpus, "steps": args.steps,
+                "warmup": args.warmup, "ms_per_step": r["ms_per_step"], "higher_is_better": True, "scaling": "weak", "vs_baseline": None,
                 "dtype": "fp32", "data": "synthetic", "config": dict(config, clips_per_gpu_per_step=1, parallelism="cpu"),
                 "cpu_baseline": {"value": r["value"], "unit": UNIT, "cores": r["cores"], "kind": "port", "sample": r["sample"]},
                 "e2e": {"value": r["value"], "unit": UNIT, "h2d_bytes_per_step": 0, "d2h_bytes_per_step": 0},
@@ -496,6 +523,8 @@ def main():
     sync_all()
     ms = e0.elapsed_time(e1)
     graph_replays_timed = int(eng.lib.gitb200_graph_launches(eng.h)) - graph0
+    if args.dump_outputs and rank == 0:
+        dump_outputs(args.dump_outputs, *handles[-1].wait())
     # every kernel of the step is this library's: a step issues `per_step_launches` of them (counted on the first, eager warm-up
     # step), whether they reach the GPU one by one or inside graph replays
     launches = per_step_launches * args.steps

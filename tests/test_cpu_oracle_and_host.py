@@ -268,6 +268,17 @@ def test_bench_emits_exactly_one_json_line_on_stdout(tmp_path):
     assert "NCCL version banner" in r.stderr and "chatter" in r.stderr
 
 
+def test_bench_dump_outputs_round_trips_tokens_and_scores(tmp_path):
+    """--dump-outputs: the gathered tokens (int32) come back exactly as float64, the log-probabilities bit for bit as float32."""
+    import bench
+    tok = torch.tensor([[[101, 30521, 2 ** 31 - 1, 102]], [[101, 7, 102, 102]]], dtype=torch.int32)
+    lp = torch.tensor([[-1.25], [-0.1]])
+    bench.dump_outputs(str(tmp_path / "out"), tok, lp)
+    t, l = np.load(tmp_path / "out" / "tokens.npy"), np.load(tmp_path / "out" / "logprobs.npy")
+    assert t.dtype == np.float64 and l.dtype == np.float32 and t.shape == (2, 1, 4) and l.shape == (2, 1)
+    assert np.array_equal(t.astype(np.int64), tok.numpy()) and np.array_equal(l, lp.numpy())
+
+
 def test_module_tree_and_state_dict_names_match_upstream():
     m = g.get_git_model(g.SyntheticTokenizer(), {"num_image_with_embedding": 6})
     sd = m.state_dict()
