@@ -212,6 +212,43 @@ int gitb200_stream_frames(const gitb200_ctx* ctx);
 int gitb200_stream_caption(gitb200_ctx* ctx, const gitb200_search_params* sp, int32_t* tokens_dev, float* logprobs_dev,
                            void* stream);
 
+/* ---- multi-stream pool: many cameras on one context ------------------------------------------------------------
+ * A pool of n_streams windows next to the single window above (which it does not touch), each window the same ring of
+ * num_image_with_embedding per-frame ViT features: bf16 [n_streams][cap][T][Dv] (GIT-base, 6 frames: 1.82 MB per stream).
+ * Stream ids are 0 .. n_streams-1.  configure empties every window; a different count also reallocates the pool.
+ * Every call below checks its id list on the host before it enqueues anything and fails, naming the offending id, on an
+ * unknown id or an id given twice (GITB200_ERR_INVALID), k < 1 (GITB200_ERR_INVALID), or a call before configure
+ * (GITB200_ERR_STATE); a rejected call changes no window.  Which frames each window holds is host-side bookkeeping. */
+int gitb200_streams_configure(gitb200_ctx* ctx, int n_streams);
+/* ONE frame for each of k distinct streams, encoded as one ViT batch (the launch sequence of gitb200_encode_images on the same
+ * k frames, in sub-batches of gitb200_set_sweep_rows): ln_post writes each frame's T rows straight into its stream's ring
+ * slot.  frames_dev fp32 [k, 3, R, R] (preprocessed) or, for _u8, uint8 [k, height, width, 3] BGR with image_transform()
+ * fused into the patch-embed loader (as gitb200_stream_push_u8); ids_host int32 [k]: frame j goes to stream ids_host[j].
+ * Calls of up to gitb200_set_graph_max_clips frames (larger ones too while graph segments are on) on a non-default stream
+ * are captured into a CUDA graph keyed by shape only (k, frame buffer, height / width): the same shape replays whichever
+ * streams it pushes to, because the per-call slot table is copied (cudaMemcpyAsync, from host memory the call owns) into a
+ * context-owned device buffer before the graph launch. */
+int gitb200_streams_push(gitb200_ctx* ctx, const int32_t* ids_host, int k, const float* frames_dev, void* stream);
+int gitb200_streams_push_u8(gitb200_ctx* ctx, const int32_t* ids_host, int k, const uint8_t* frames_dev, int height, int width,
+                            void* stream);
+/* Decoder + search over the windows of k distinct streams that hold the SAME number of frames n (temporal embeddings by
+ * arrival order, oldest = position 0, exactly as gitb200_stream_caption): tokens_dev int32 [k, num_keep_best, max_steps],
+ * logprobs_dev fp32 [k, num_keep_best], row j = stream ids_host[j].  Fails with GITB200_ERR_STATE on an empty stream and
+ * GITB200_ERR_INVALID when the streams hold different frame counts (caption those in separate calls).  Afterwards the
+ * context's current visual features are these k windows [k, n*T, Dv], as after gitb200_stream_caption.  Up to
+ * gitb200_set_graph_max_clips windows the whole call is one CUDA graph (one window with beam <= 4 takes the persistent
+ * decode kernel); larger calls graph the window assembly + visual pass and the decode segments.  The caption of a stream
+ * does not depend on which other streams share the call or in which order. */
+int gitb200_streams_caption(gitb200_ctx* ctx, const int32_t* ids_host, int k, const gitb200_search_params* sp,
+                            int32_t* tokens_dev, float* logprobs_dev, void* stream);
+/* Empties the windows of k distinct streams (the reference's frames.clear() after a caption, real_time_inference.py:61). */
+int gitb200_streams_reset(gitb200_ctx* ctx, const int32_t* ids_host, int k);
+/* Frames held by one stream's window (0 .. num_image_with_embedding); GITB200_ERR_INVALID for an unknown id. */
+int gitb200_streams_frames(const gitb200_ctx* ctx, int stream_id);
+/* One stream's window as the decoder sees it: temporal embeddings added, bf16 values written as fp32 [n*T, Dv] (the
+ * visual features gitb200_streams_caption decodes for that stream).  Does not change the context's current features. */
+int gitb200_streams_window(gitb200_ctx* ctx, int stream_id, float* out_dev, void* stream);
+
 /* ---- frame preprocessing: image_transform(), src/utils/dataloader.py:18-32 (= real_time_inference.py:16-28) ----
  * frames_dev: uint8 [n_frames, height, width, 3] in OpenCV's BGR HWC layout; out_dev: fp32 [n_frames, 3, size, size]
  * (RGB, CLIP-normalised): bicubic resize of the smaller edge to `size` (no antialias, like the pinned torchvision

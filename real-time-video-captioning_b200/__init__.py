@@ -9,7 +9,7 @@ All compute runs in libgitb200.so (include/gitb200.h); importing works without a
 from ._lib import GitB200Error, LIB_PATH  # noqa: F401
 from .engine import Engine, SearchConfig, make_config, preprocess_frames, VIT_CONFIGS  # noqa: F401
 from .model import (BeamHypotheses, CLIPVisionTower, GenerativeImageTextModel, GenerativeImageTextTeacher,  # noqa: F401
-                    GeneratorWithBeamSearchV2, LazyLogits, StreamingCaptioner, SyntheticTokenizer, TransformerDecoderTextualHead,
+                    GeneratorWithBeamSearchV2, LazyLogits, MultiStreamCaptioner, StreamingCaptioner, SyntheticTokenizer, TransformerDecoderTextualHead,
                     get_git_model)
 from .student import DistillationTrainer, StudentCandidateV1  # noqa: F401
 from .metrics import calculate_bleu_score_corpus  # noqa: F401
@@ -18,4 +18,4 @@ from .dist import all_reduce_bucket, caption_sharded, finish_all_reduce, shard_r
 __all__ = ["Engine", "SearchConfig", "GenerativeImageTextModel", "GenerativeImageTextTeacher",
            "GeneratorWithBeamSearchV2", "get_git_model", "calculate_bleu_score_corpus", "shard_range",
            "caption_sharded", "GitB200Error", "StudentCandidateV1", "DistillationTrainer", "all_reduce_bucket",
-           "finish_all_reduce"]
+           "finish_all_reduce", "MultiStreamCaptioner"]

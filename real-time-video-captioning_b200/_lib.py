@@ -99,6 +99,13 @@ SIGNATURES = {
     "gitb200_stream_push_u8": (c_int, [c_void_p, c_void_p, c_int, c_int, c_void_p]),
     "gitb200_stream_frames": (c_int, [c_void_p]),
     "gitb200_stream_caption": (c_int, [c_void_p, POINTER(SearchParams), c_void_p, c_void_p, c_void_p]),
+    "gitb200_streams_configure": (c_int, [c_void_p, c_int]),
+    "gitb200_streams_push": (c_int, [c_void_p, c_void_p, c_int, c_void_p, c_void_p]),
+    "gitb200_streams_push_u8": (c_int, [c_void_p, c_void_p, c_int, c_void_p, c_int, c_int, c_void_p]),
+    "gitb200_streams_caption": (c_int, [c_void_p, c_void_p, c_int, POINTER(SearchParams), c_void_p, c_void_p, c_void_p]),
+    "gitb200_streams_reset": (c_int, [c_void_p, c_void_p, c_int]),
+    "gitb200_streams_frames": (c_int, [c_void_p, c_int]),
+    "gitb200_streams_window": (c_int, [c_void_p, c_int, c_void_p, c_void_p]),
     "gitb200_preprocess": (c_int, [c_void_p, c_int, c_int, c_int, c_int, c_void_p, c_void_p]),
     "gitb200_op_gemm": (c_int, [c_void_p, c_void_p, c_int, c_int, c_int, c_void_p, c_void_p, c_int, c_void_p, c_void_p,
                                 c_int, c_void_p]),

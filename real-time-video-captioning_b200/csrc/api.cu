@@ -161,6 +161,15 @@ struct gitb200_ctx {
   Buf<bf16> ring;
   int ring_count = 0, ring_head = 0;
 
+  // multi-stream pool (gitb200_streams_*): one window of num_image_with_embedding frames per camera stream, bf16
+  // [pool_streams][cap][T][W], same per-frame features as `ring`.  head / count of every window are kept here on the host.
+  // The per-call tables (ln_post output row of every pushed frame, oldest ring slot of every captioned window) are copied
+  // into pool_rows / pool_oldest at fixed addresses, so a captured graph replays for any set of streams of the same shape.
+  Buf<bf16> pool;
+  int pool_streams = 0;
+  std::vector<int> pool_head, pool_count;
+  Buf<int> pool_rows, pool_oldest;
+
   // forward-hook taps on image_encoder.transformer.resblocks[i] (model.py:847): outputs copied out by the next encodes
   std::vector<int> tap_layers;
   float* tap_out = nullptr;
@@ -316,7 +325,8 @@ int sweep_clips(int sweep_rows, int rows_per_clip, int n_clips) {
 // clip_offset / total_clips: the visual features of this call land at clip index `clip_offset` of a buffer sized for
 // `total_clips` clips (host path: chunks are encoded as their frames arrive, then decoded together).
 // frame_out != nullptr: streaming mode -- write ln_post(x) WITHOUT temporal embeddings to frame_out and leave the
-// context's visual features untouched.
+// context's visual features untouched.  out_rows != nullptr (device table, one entry per frame): frame f's T rows go to
+// frame_out rows out_rows[f] .. out_rows[f] + T - 1 (a multi-stream push: each frame straight into its stream's ring slot).
 // raw != nullptr: `frames` is ignored and the patch matrix is filled straight from raw uint8 BGR video frames
 // (image_transform() fused into the patch-embed loader, preprocess.cu).
 struct RawFrames {
@@ -325,7 +335,7 @@ struct RawFrames {
 };
 
 int run_encode(gitb200_ctx* c, const float* frames, int n_clips, int n_frames, cudaStream_t s, int clip_offset = 0, int total_clips = 0,
-               bf16* frame_out = nullptr, bool temporal = true, const RawFrames* raw = nullptr) {
+               bf16* frame_out = nullptr, bool temporal = true, const RawFrames* raw = nullptr, const int* out_rows = nullptr) {
   const gitb200_config& k = c->cfg;
   const int W = k.vit_width, T = c->T, G = k.resolution / k.patch;
   // zip() truncation of model.py:380: frames beyond the temporal-embedding list are dropped
@@ -451,7 +461,10 @@ int run_encode(gitb200_ctx* c, const float* frames, int n_clips, int n_frames, c
   }
   // ln_post on all tokens + temporal embedding of the frame (frame index = (row / T) % F)
   if (frame_out != nullptr) {
-    TRY(ln(c, c->x.p, rows, W, c->ln_post_g, c->ln_post_b, k.vit_ln_eps, frame_out, s));
+    LayerNormArgs a;
+    a.x = c->x.p; a.ldx = W; a.rows = rows; a.cols = W; a.gamma = c->ln_post_g; a.beta = c->ln_post_b; a.eps = k.vit_ln_eps;
+    a.out = frame_out; a.ldo = W; a.out_row_base = out_rows; a.out_group = T;
+    CUDA_OK(c, layernorm_bf16(a, s));
     return 0;
   }
   TRY(ln(c, c->x.p, rows, W, c->ln_post_g, c->ln_post_b, k.vit_ln_eps, c->vf.p + (size_t)clip_offset * F * T * W, s,
@@ -933,6 +946,7 @@ void free_workspaces(gitb200_ctx* c) {
   fr(c->tx); fr(c->tq); fr(c->ta); fr(c->tb); fr(c->tc); fr(c->tf); fr(c->logits); fr(c->partial); fr(c->vf_in_f32);
   fr(c->ibuf); fr(c->dbuf); fr(c->fbuf); fr(c->pos_arr); fr(c->ntext_arr); fr(c->tok_arr); fr(c->stage[0]); fr(c->stage[1]); fr(c->stage_u8[0]); fr(c->stage_u8[1]);
   fr(c->out_tok); fr(c->out_lp); fr(c->stats_a); fr(c->stats_b); fr(c->ring);
+  fr(c->pool); fr(c->pool_rows); fr(c->pool_oldest);
 }
 
 // second workspace set that shares this context's (read-only) weights
@@ -1359,16 +1373,21 @@ int gitb200_reserve(gitb200_ctx* c, int max_clips, int max_frames, int max_rows_
 }
 
 // run_encode over `n_clips` clips in sub-batches of ~sweep_rows token rows (see gitb200_ctx::sweep_rows); every sub-batch
-// writes its slice of the visual features, so the result is the one sweep's, bit for bit.
-static int run_encode_sweeps(gitb200_ctx* c, const float* frames, int n_clips, int n_frames, cudaStream_t s, bool temporal = true) {
+// writes its slice of the visual features (or, with frame_out / out_rows, its frames' rows), so the result is the one
+// sweep's, bit for bit.  raw != nullptr: raw uint8 frames instead of `frames` (see run_encode).
+static int run_encode_sweeps(gitb200_ctx* c, const float* frames, int n_clips, int n_frames, cudaStream_t s, bool temporal = true,
+                             bf16* frame_out = nullptr, const int* out_rows = nullptr, const RawFrames* raw = nullptr) {
   const gitb200_config& k = c->cfg;
   const int F = (temporal && k.num_image_with_embedding > 0 && n_frames > k.num_image_with_embedding) ? k.num_image_with_embedding : n_frames;
   const int sub = sweep_clips(c->sweep_rows, F * c->T, n_clips);
-  if (sub >= n_clips) return run_encode(c, frames, n_clips, n_frames, s, 0, 0, nullptr, temporal);
+  if (sub >= n_clips) return run_encode(c, frames, n_clips, n_frames, s, 0, 0, frame_out, temporal, raw, out_rows);
   const size_t clip_elems = (size_t)n_frames * 3 * k.resolution * k.resolution;
   for (int done = 0; done < n_clips; done += sub) {
     const int nc = (n_clips - done) < sub ? (n_clips - done) : sub;
-    TRY(run_encode(c, frames + (size_t)done * clip_elems, nc, n_frames, s, done, n_clips, nullptr, temporal));
+    RawFrames part{};
+    if (raw) part = RawFrames{raw->p + (size_t)done * n_frames * raw->height * raw->width * 3, raw->height, raw->width};
+    TRY(run_encode(c, frames ? frames + (size_t)done * clip_elems : nullptr, nc, n_frames, s, done, n_clips, frame_out, temporal,
+                   raw ? &part : nullptr, out_rows ? out_rows + (size_t)done * F : nullptr));
   }
   return 0;
 }
@@ -1580,6 +1599,187 @@ int gitb200_stream_caption(gitb200_ctx* c, const gitb200_search_params* sp, int3
     return GITB200_OK;
   }
   return r;
+}
+
+// ---- multi-stream pool: one window per camera stream, pushes and captions batched over streams
+// Host-side checks of a stream-id list, before anything is enqueued: the pool exists, k >= 1, every id is known and distinct.
+static int pool_check_ids(gitb200_ctx* c, const char* what, const int32_t* ids, int k) {
+  if (c->pool_streams < 1) return fail(c, GITB200_ERR_STATE, "%s: no stream pool: call gitb200_streams_configure first", what);
+  if (k < 1 || ids == nullptr) return fail(c, GITB200_ERR_INVALID, "%s: need k >= 1 stream ids (k = %d)", what, k);
+  std::vector<char> seen((size_t)c->pool_streams, 0);
+  for (int j = 0; j < k; ++j) {
+    const int id = ids[j];
+    if (id < 0 || id >= c->pool_streams)
+      return fail(c, GITB200_ERR_INVALID, "%s: unknown stream id %d (the pool has ids 0..%d)", what, id, c->pool_streams - 1);
+    if (seen[id]) return fail(c, GITB200_ERR_INVALID, "%s: stream id %d appears twice in one call", what, id);
+    seen[id] = 1;
+  }
+  return 0;
+}
+
+// The per-call tables sit at fixed device addresses: a call on another stream than this context's previous call first waits
+// for that stream, so that a table (or a window) is not rewritten while the previous call still reads it.
+static int pool_order_after_last_stream(gitb200_ctx* c, cudaStream_t s) {
+  if (!c->last_stream_valid || c->last_stream == s) return 0;
+  if (!c->ev_user) CUDA_OK(c, cudaEventCreateWithFlags(&c->ev_user, cudaEventDisableTiming));
+  if (cudaEventRecord(c->ev_user, c->last_stream) != cudaSuccess) {
+    cudaGetLastError();  // that stream no longer exists: everything it was given has to be complete
+    CUDA_OK(c, cudaDeviceSynchronize());
+  } else {
+    CUDA_OK(c, cudaStreamWaitEvent(s, c->ev_user, 0));
+  }
+  return 0;
+}
+
+int gitb200_streams_configure(gitb200_ctx* c, int n_streams) {
+  if (!c) return GITB200_ERR_INVALID;
+  if (n_streams < 1) return fail(c, GITB200_ERR_INVALID, "gitb200_streams_configure: n_streams must be >= 1 (got %d)", n_streams);
+  const int cap = c->cfg.num_image_with_embedding;
+  if (cap < 1) return fail(c, GITB200_ERR_STATE, "streaming needs num_image_with_embedding >= 1 (the window length)");
+  CUDA_OK(c, cudaSetDevice(c->device));
+  if (n_streams != c->pool_streams) {
+    for (void* p : {(void*)c->pool.p, (void*)c->pool_rows.p, (void*)c->pool_oldest.p})
+      if (p) {
+        CUDA_OK(c, cudaFree(p));
+        c->ws_gen++;  // captured graphs hold the freed pointers
+      }
+    c->pool = Buf<bf16>{}; c->pool_rows = Buf<int>{}; c->pool_oldest = Buf<int>{};
+    c->pool_streams = 0;
+    c->pool_head.clear(); c->pool_count.clear();
+    ENSURE(c, c->pool, (size_t)n_streams * cap * c->T * c->cfg.vit_width);
+    ENSURE(c, c->pool_rows, (size_t)n_streams);
+    ENSURE(c, c->pool_oldest, (size_t)n_streams);
+    c->pool_streams = n_streams;
+  }
+  c->pool_head.assign((size_t)n_streams, 0);
+  c->pool_count.assign((size_t)n_streams, 0);
+  return GITB200_OK;
+}
+
+static int streams_push_any(gitb200_ctx* c, const int32_t* ids, int k, const float* frames, const uint8_t* raw, int height, int width,
+                            void* stream) {
+  const char* what = raw ? "gitb200_streams_push_u8" : "gitb200_streams_push";
+  if (!c) return GITB200_ERR_INVALID;
+  if (!c->finalized) return fail(c, GITB200_ERR_STATE, "call gitb200_finalize_weights first");
+  TRY(pool_check_ids(c, what, ids, k));
+  if ((raw == nullptr && frames == nullptr) || (raw != nullptr && (height < 1 || width < 1)))
+    return fail(c, GITB200_ERR_INVALID, "%s: bad frame buffer / size", what);
+  CUDA_OK(c, cudaSetDevice(c->device));
+  const cudaStream_t s = (cudaStream_t)stream;
+  TRY(pool_order_after_last_stream(c, s));
+  caller_stream(c, stream);
+  const int cap = c->cfg.num_image_with_embedding, T = c->T;
+  std::vector<int> rows((size_t)k);
+  for (int j = 0; j < k; ++j) rows[j] = (ids[j] * cap + c->pool_head[ids[j]]) * T;
+  CUDA_OK(c, cudaMemcpyAsync(c->pool_rows.p, rows.data(), (size_t)k * sizeof(int), cudaMemcpyHostToDevice, s));
+  // the launch sequence of gitb200_encode_images on the same k frames, except that ln_post writes through the row table
+  gitb200_ctx::GraphKey key;
+  key.kind = raw ? 11 : 10; key.p0 = raw ? (const void*)raw : (const void*)frames; key.i0 = k; key.i1 = height; key.i2 = width;
+  const RawFrames rf{raw, height, width};
+  const int r = run_graphed(c, key, s, k <= c->graph_max_clips || c->graph_segments, [&]() {
+    return run_encode_sweeps(c, frames, k, 1, s, /*temporal=*/false, c->pool.p, c->pool_rows.p, raw ? &rf : nullptr);
+  });
+  if (r != 0 && r != 1) return r;
+  for (int j = 0; j < k; ++j) {
+    const int id = ids[j];
+    c->pool_head[id] = (c->pool_head[id] + 1) % cap;
+    if (c->pool_count[id] < cap) c->pool_count[id]++;
+  }
+  return GITB200_OK;
+}
+
+int gitb200_streams_push(gitb200_ctx* c, const int32_t* ids, int k, const float* frames, void* stream) {
+  return streams_push_any(c, ids, k, frames, nullptr, 0, 0, stream);
+}
+
+int gitb200_streams_push_u8(gitb200_ctx* c, const int32_t* ids, int k, const uint8_t* frames, int height, int width, void* stream) {
+  if (!frames) return fail(c, GITB200_ERR_INVALID, "gitb200_streams_push_u8: null frame buffer");
+  return streams_push_any(c, ids, k, nullptr, frames, height, width, stream);
+}
+
+int gitb200_streams_caption(gitb200_ctx* c, const int32_t* ids, int k, const gitb200_search_params* sp, int32_t* tokens,
+                            float* logprobs, void* stream) {
+  if (!c || !sp || !tokens || !logprobs) return fail(c, GITB200_ERR_INVALID, "bad streams_caption argument");
+  if (!c->finalized) return fail(c, GITB200_ERR_STATE, "call gitb200_finalize_weights first");
+  TRY(pool_check_ids(c, "gitb200_streams_caption", ids, k));
+  const int n = c->pool_count[ids[0]];
+  for (int j = 0; j < k; ++j) {
+    if (c->pool_count[ids[j]] < 1)
+      return fail(c, GITB200_ERR_STATE, "gitb200_streams_caption: stream id %d holds no frames: push first", ids[j]);
+    if (c->pool_count[ids[j]] != n)
+      return fail(c, GITB200_ERR_INVALID, "gitb200_streams_caption: stream id %d holds %d frames but stream id %d holds %d: "
+                  "windows of different lengths go in separate calls", ids[j], c->pool_count[ids[j]], ids[0], n);
+  }
+  CUDA_OK(c, cudaSetDevice(c->device));
+  const cudaStream_t s = (cudaStream_t)stream;
+  TRY(pool_order_after_last_stream(c, s));
+  caller_stream(c, stream);
+  const int cap = c->cfg.num_image_with_embedding, T = c->T, W = c->cfg.vit_width;
+  ENSURE(c, c->vf, (size_t)k * n * T * W);
+  std::vector<int> oldest((size_t)k);
+  for (int j = 0; j < k; ++j) oldest[j] = ids[j] * cap + (c->pool_head[ids[j]] - n + cap) % cap;  // temporal position 0
+  CUDA_OK(c, cudaMemcpyAsync(c->pool_oldest.p, oldest.data(), (size_t)k * sizeof(int), cudaMemcpyHostToDevice, s));
+  auto assemble = [&]() -> int {
+    CUDA_OK(c, assemble_windows(c->pool.p, c->pool_oldest.p, 0, k, n, cap, T, W, c->temporal, c->vf.p, nullptr, s));
+    c->cur_clips = k; c->cur_nv = n * T; c->visual_pass_done = false; c->step_rows_per_clip = 0;
+    return 0;
+  };
+  gitb200_ctx::GraphKey key;
+  key.i0 = k; key.i1 = n;
+  if (k <= c->graph_max_clips) {  // latency mode: the whole call as one graph (k == 1, beam <= 4: the persistent decode kernel)
+    key.kind = 12; key.p0 = tokens; key.p1 = logprobs; key.sp = *sp;
+    const int r = run_graphed(c, key, s, true, [&]() -> int {
+      TRY(assemble());
+      return run_decode(c, *sp, tokens, logprobs, nullptr, s);
+    });
+    if (r == 1) {  // replayed: host-side state the eager run would have left
+      c->cur_clips = k; c->cur_nv = n * T; c->visual_pass_done = true; c->visual_pass_full = 0; c->step_rows_per_clip = 0;
+      c->last_decode_steps = sp->max_steps - 1;
+      return GITB200_OK;
+    }
+    return r;
+  }
+  // throughput-sized: window assembly + the decoder's visual pass as one graph, then the graphed decode segments of run_decode
+  key.kind = 13;
+  const int r = run_graphed(c, key, s, c->graph_segments, [&]() -> int {
+    TRY(assemble());
+    return run_visual_pass(c, false, nullptr, 0, s);
+  });
+  if (r == 1) {
+    c->cur_clips = k; c->cur_nv = n * T; c->visual_pass_done = true; c->visual_pass_full = 0; c->step_rows_per_clip = 0;
+  } else if (r != 0) {
+    return r;
+  }
+  return run_decode(c, *sp, tokens, logprobs, nullptr, s);
+}
+
+int gitb200_streams_reset(gitb200_ctx* c, const int32_t* ids, int k) {
+  if (!c) return GITB200_ERR_INVALID;
+  TRY(pool_check_ids(c, "gitb200_streams_reset", ids, k));
+  for (int j = 0; j < k; ++j) c->pool_head[ids[j]] = c->pool_count[ids[j]] = 0;
+  return GITB200_OK;
+}
+
+int gitb200_streams_frames(const gitb200_ctx* c, int id) {
+  if (!c || id < 0 || id >= c->pool_streams) return GITB200_ERR_INVALID;
+  return c->pool_count[id];
+}
+
+int gitb200_streams_window(gitb200_ctx* c, int id, float* out, void* stream) {
+  if (!c || !out) return fail(c, GITB200_ERR_INVALID, "bad streams_window argument");
+  if (c->pool_streams < 1) return fail(c, GITB200_ERR_STATE, "gitb200_streams_window: no stream pool: call gitb200_streams_configure first");
+  if (id < 0 || id >= c->pool_streams)
+    return fail(c, GITB200_ERR_INVALID, "gitb200_streams_window: unknown stream id %d (the pool has ids 0..%d)", id, c->pool_streams - 1);
+  const int n = c->pool_count[id];
+  if (n < 1) return fail(c, GITB200_ERR_STATE, "gitb200_streams_window: stream id %d holds no frames", id);
+  CUDA_OK(c, cudaSetDevice(c->device));
+  const cudaStream_t s = (cudaStream_t)stream;
+  TRY(pool_order_after_last_stream(c, s));
+  caller_stream(c, stream);
+  const int cap = c->cfg.num_image_with_embedding;
+  CUDA_OK(c, assemble_windows(c->pool.p, nullptr, id * cap + (c->pool_head[id] - n + cap) % cap, 1, n, cap, c->T, c->cfg.vit_width,
+                              c->temporal, nullptr, out, s));
+  return GITB200_OK;
 }
 
 int gitb200_set_fold_layernorm(gitb200_ctx* c, int enable) {

@@ -10,7 +10,8 @@ namespace {
 // Persistent: the grid is sized to the machine and every warp walks rows with a grid stride, the next row's 16-byte loads
 // are issued before the current row is reduced, and gamma / beta sit in shared memory (loaded once per CTA; the first
 // version re-read 6 KB of them from L1 for every 1.5 KB row and started one 8-row CTA per 12 KB of traffic).
-template <int VECS>  // 16-byte vectors per lane: cols = 32 * 8 * VECS  (768 -> 3, 1024 -> 4)
+// REMAP: output rows go through LayerNormArgs::out_row_base (a separate instantiation, so the plain kernel is untouched).
+template <int VECS, bool REMAP>  // 16-byte vectors per lane: cols = 32 * 8 * VECS  (768 -> 3, 1024 -> 4)
 __global__ void __launch_bounds__(256, 3) layernorm_kernel(LayerNormArgs a) {
   __shared__ float4 sg[VECS * 64], sb[VECS * 64];  // gamma / beta as float4: index (i * 32 + lane) * 2 + {0, 1}
   for (int i = threadIdx.x; i < VECS * 64; i += blockDim.x) {
@@ -51,6 +52,7 @@ __global__ void __launch_bounds__(256, 3) layernorm_kernel(LayerNormArgs a) {
   }
   const float rstd = rsqrtf(warp_sum(q) / (float)a.cols + a.eps);
   const float* add = a.addend ? a.addend + (size_t)((warp / a.add_group) % a.add_period) * a.cols : nullptr;
+  const size_t orow = REMAP ? (size_t)a.out_row_base[warp / a.out_group] + warp % a.out_group : (size_t)warp;
   float st1 = 0.f, st2 = 0.f;
 #pragma unroll
   for (int i = 0; i < VECS; ++i) {
@@ -75,7 +77,7 @@ __global__ void __launch_bounds__(256, 3) layernorm_kernel(LayerNormArgs a) {
     if (a.out) {
       uint4 u;
       u.x = pack_bf16(o[0], o[1]); u.y = pack_bf16(o[2], o[3]); u.z = pack_bf16(o[4], o[5]); u.w = pack_bf16(o[6], o[7]);
-      *reinterpret_cast<uint4*>(a.out + (size_t)warp * a.ldo + c) = u;
+      *reinterpret_cast<uint4*>(a.out + orow * a.ldo + c) = u;
       if (a.stats_out) {
         const float2 r0 = unpack_bf16(u.x), r1 = unpack_bf16(u.y), r2 = unpack_bf16(u.z), r3 = unpack_bf16(u.w);
         st1 += (r0.x + r0.y) + (r1.x + r1.y) + (r2.x + r2.y) + (r3.x + r3.y);
@@ -83,7 +85,7 @@ __global__ void __launch_bounds__(256, 3) layernorm_kernel(LayerNormArgs a) {
       }
     }
     if (a.out_f32) {
-      float4* p = reinterpret_cast<float4*>(a.out_f32 + (size_t)warp * a.ldo32 + c);
+      float4* p = reinterpret_cast<float4*>(a.out_f32 + orow * a.ldo32 + c);
       p[0] = make_float4(o[0], o[1], o[2], o[3]);
       p[1] = make_float4(o[4], o[5], o[6], o[7]);
     }
@@ -275,6 +277,42 @@ __global__ void assemble_window_kernel(const bf16* __restrict__ ring, int first,
   }
 }
 
+// The windows of k streams of the multi-stream pool, n frames each: window w, frame i (0 = oldest), token t is
+//   vf[(w * n + i) * T + t, :] = bf16(ring[(base + (first + i) % cap) * T + t, :] + temporal[i, :])
+// with oldest[w] = base + first (base = the stream's first ring slot, a multiple of cap); oldest == nullptr: oldest_const.
+// The arithmetic of assemble_window_kernel; vf32 != nullptr writes the bf16-rounded values as fp32 instead of vf.
+__global__ void assemble_windows_kernel(const bf16* __restrict__ ring, const int* __restrict__ oldest, int oldest_const, int k,
+                                        int n, int cap, int T, int W, const float* __restrict__ temporal, bf16* __restrict__ vf,
+                                        float* __restrict__ vf32) {
+  const size_t chunks_per_row = W / 8;
+  const size_t total = (size_t)k * n * T * chunks_per_row;
+  for (size_t idx = blockIdx.x * (size_t)blockDim.x + threadIdx.x; idx < total; idx += (size_t)gridDim.x * blockDim.x) {
+    const int c = (int)(idx % chunks_per_row) * 8;
+    const size_t row = idx / chunks_per_row;
+    const int w = (int)(row / ((size_t)n * T));
+    const int r = (int)(row % ((size_t)n * T));
+    const int i = r / T, t = r % T;
+    const int o = oldest ? oldest[w] : oldest_const;
+    const int first = o % cap;
+    const int slot = o - first + (first + i) % cap;
+    const uint4 u = *reinterpret_cast<const uint4*>(ring + ((size_t)slot * T + t) * W + c);
+    float2 a = unpack_bf16(u.x), b = unpack_bf16(u.y), d = unpack_bf16(u.z), e = unpack_bf16(u.w);
+    const float4 t0 = __ldg(reinterpret_cast<const float4*>(temporal + (size_t)i * W + c));
+    const float4 t1 = __ldg(reinterpret_cast<const float4*>(temporal + (size_t)i * W + c + 4));
+    a.x += t0.x; a.y += t0.y; b.x += t0.z; b.y += t0.w; d.x += t1.x; d.y += t1.y; e.x += t1.z; e.y += t1.w;
+    uint4 q;
+    q.x = pack_bf16(a.x, a.y); q.y = pack_bf16(b.x, b.y); q.z = pack_bf16(d.x, d.y); q.w = pack_bf16(e.x, e.y);
+    if (vf32) {
+      const float2 r0 = unpack_bf16(q.x), r1 = unpack_bf16(q.y), r2 = unpack_bf16(q.z), r3 = unpack_bf16(q.w);
+      float4* p = reinterpret_cast<float4*>(vf32 + row * W + c);
+      p[0] = make_float4(r0.x, r0.y, r1.x, r1.y);
+      p[1] = make_float4(r2.x, r2.y, r3.x, r3.y);
+    } else {
+      *reinterpret_cast<uint4*>(vf + row * W + c) = q;
+    }
+  }
+}
+
 __global__ void fill_positions_kernel(int* pos, int* n_text, int rows, int L) {
   const int r = blockIdx.x * blockDim.x + threadIdx.x;
   if (r < rows) {
@@ -290,6 +328,17 @@ cudaError_t assemble_window(const bf16* ring, int first, int cap, int n, int T, 
   const size_t total = (size_t)n * T * (W / 8);
   if (total == 0) return cudaSuccess;
   assemble_window_kernel<<<(int)((total + 255) / 256), 256, 0, stream>>>(ring, first, cap, n, T, W, temporal, vf);
+  note_launch();
+  return cudaGetLastError();
+}
+
+cudaError_t assemble_windows(const bf16* ring, const int* oldest, int oldest_const, int k, int n, int cap, int T, int W,
+                             const float* temporal, bf16* vf, float* vf32, cudaStream_t stream) {
+  const size_t total = (size_t)k * n * T * (W / 8);
+  if (total == 0) return cudaSuccess;
+  const size_t blocks = (total + 255) / 256;
+  assemble_windows_kernel<<<(int)(blocks > 148 * 32 ? 148 * 32 : blocks), 256, 0, stream>>>(ring, oldest, oldest_const, k, n, cap, T, W,
+                                                                                          temporal, vf, vf32);
   note_launch();
   return cudaGetLastError();
 }
@@ -314,10 +363,16 @@ cudaError_t layernorm_bf16(const LayerNormArgs& a, cudaStream_t stream) {
   int blocks = (a.rows * 32 + 255) / 256;
   const int max_blocks = 148 * 3;  // three 256-thread CTAs per SM (two rows in flight per warp), grid-stride over the rows
   if (blocks > max_blocks) blocks = max_blocks;
-  if (a.cols == 768)
-    layernorm_kernel<3><<<blocks, 256, 0, stream>>>(a);
+  const bool remap = a.out_row_base != nullptr;
+  if (remap && a.out_group < 1) return cudaErrorInvalidValue;
+  if (a.cols == 768 && !remap)
+    layernorm_kernel<3, false><<<blocks, 256, 0, stream>>>(a);
+  else if (a.cols == 1024 && !remap)
+    layernorm_kernel<4, false><<<blocks, 256, 0, stream>>>(a);
+  else if (a.cols == 768)
+    layernorm_kernel<3, true><<<blocks, 256, 0, stream>>>(a);
   else if (a.cols == 1024)
-    layernorm_kernel<4><<<blocks, 256, 0, stream>>>(a);
+    layernorm_kernel<4, true><<<blocks, 256, 0, stream>>>(a);
   else
     return cudaErrorInvalidValue;
   note_launch();

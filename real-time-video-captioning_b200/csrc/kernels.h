@@ -89,6 +89,10 @@ struct LayerNormArgs {
   int ldo32 = 0;
   float* stats_out = nullptr;  // optional [rows, stats_slots, 2]: (sum, sum of squares) of the bf16-rounded output row in slot 0, zeros elsewhere
   int stats_slots = 1;
+  // optional device table: input rows [g * out_group, (g + 1) * out_group) are written to output rows out_row_base[g] + 0,
+  // 1, ... (ln_post of a multi-stream push straight into each frame's ring slot); null = output row r for input row r
+  const int* out_row_base = nullptr;
+  int out_group = 0;
 };
 cudaError_t layernorm_bf16(const LayerNormArgs& a, cudaStream_t stream);
 
@@ -229,3 +233,8 @@ cudaError_t ln_fold_weight(const float* w, int N, int K, const float* gamma, con
 // Streaming window: vf[i*T + t, :] = ring[((first + i) % cap)*T + t, :] + temporal[i, :]  for i < n  (bf16, fp32 temporal)
 cudaError_t assemble_window(const bf16* ring, int first, int cap, int n, int T, int W, const float* temporal, bf16* vf,
                             cudaStream_t stream);
+// Multi-stream pool: the k windows of n frames each, vf[(w*n + i)*T + t, :] = ring[slot(w, i)*T + t, :] + temporal[i, :] with
+// slot(w, i) = base + (first + i) % cap and oldest[w] = base + first (device table; nullptr: oldest_const for the one window).
+// Writes bf16 vf, or, if vf32 != nullptr, the same bf16-rounded values as fp32 to vf32 instead.
+cudaError_t assemble_windows(const bf16* ring, const int* oldest, int oldest_const, int k, int n, int cap, int T, int W,
+                             const float* temporal, bf16* vf, float* vf32, cudaStream_t stream);

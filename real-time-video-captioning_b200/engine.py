@@ -314,6 +314,69 @@ class Engine:
         self._cur_clips, self._cur_nv, self._step_rows = 1, int(self.lib.gitb200_stream_frames(self.h)) * self.T, 0
         return tokens.clone(), logprobs.clone()
 
+    # ---- multi-stream pool: one window per camera, pushes and captions batched over cameras
+    @staticmethod
+    def _ids(ids):
+        ids = [int(i) for i in ids]
+        return (ctypes.c_int32 * max(1, len(ids)))(*ids), len(ids)
+
+    def streams_configure(self, n_streams: int) -> None:
+        """A pool of ``n_streams`` windows (ids 0 .. n_streams-1), all empty."""
+        check(self.lib.gitb200_streams_configure(self.h, n_streams), self.h, "gitb200_streams_configure")
+
+    def streams_push(self, ids, frames: torch.Tensor) -> None:
+        """One preprocessed frame per stream: frames fp32 [k, 3, R, R], frame j into the window of stream ids[j]; one ViT batch."""
+        R = self.cfg.resolution
+        assert frames.is_cuda and frames.dtype == torch.float32 and frames.shape == (len(ids), 3, R, R)
+        frames = frames.contiguous()
+        arr, k = self._ids(ids)
+        check(self.lib.gitb200_streams_push(self.h, arr, k, _ptr(frames), self._stream()), self.h, "gitb200_streams_push")
+
+    def streams_push_u8(self, ids, frames_u8: torch.Tensor) -> None:
+        """One RAW frame per stream: uint8 [k, H, W, 3] (OpenCV BGR, on this device), image_transform() fused into the
+        patch-embed loader.  Keep pushing from the same buffer and the library replays a CUDA graph."""
+        assert frames_u8.is_cuda and frames_u8.dtype == torch.uint8 and frames_u8.dim() == 4 and frames_u8.shape[-1] == 3
+        assert frames_u8.is_contiguous() and frames_u8.shape[0] == len(ids)
+        h, w = frames_u8.shape[1:3]
+        arr, k = self._ids(ids)
+        check(self.lib.gitb200_streams_push_u8(self.h, arr, k, _ptr(frames_u8), h, w, self._stream()), self.h,
+              "gitb200_streams_push_u8")
+
+    def streams_caption(self, ids, sp: SearchConfig):
+        """Caption the windows of the streams ``ids`` (all holding the same number of frames) as one decode batch:
+        (tokens int32 [k, keep, max_steps], logprobs [k, keep]), row j = stream ids[j]."""
+        arr, k = self._ids(ids)
+        # persistent output buffers: identical call signatures let the library replay its captured CUDA graph
+        key = (k, sp.num_keep_best, sp.max_steps)
+        if not hasattr(self, "_streams_out"):
+            self._streams_out = {}
+        if key not in self._streams_out:
+            self._streams_out[key] = (torch.empty(k, sp.num_keep_best, sp.max_steps, dtype=torch.int32, device=self.device),
+                                      torch.empty(k, sp.num_keep_best, dtype=torch.float32, device=self.device))
+        tokens, logprobs = self._streams_out[key]
+        c = sp.to_c()
+        check(self.lib.gitb200_streams_caption(self.h, arr, k, ctypes.byref(c), _ptr(tokens), _ptr(logprobs), self._stream()),
+              self.h, "gitb200_streams_caption")
+        self._cur_clips, self._cur_nv, self._step_rows = k, self.streams_frames(int(ids[0])) * self.T, 0
+        return tokens.clone(), logprobs.clone()
+
+    def streams_reset(self, ids) -> None:
+        arr, k = self._ids(ids)
+        check(self.lib.gitb200_streams_reset(self.h, arr, k), self.h, "gitb200_streams_reset")
+
+    def streams_frames(self, stream_id: int) -> int:
+        n = int(self.lib.gitb200_streams_frames(self.h, stream_id))
+        if n < 0:
+            raise GitB200Error(f"gitb200_streams_frames: unknown stream id {stream_id}")
+        return n
+
+    def streams_window(self, stream_id: int) -> torch.Tensor:
+        """The window of one stream as the decoder sees it (temporal embeddings added, bf16 values): fp32 [n*T, Dv]."""
+        n = self.streams_frames(stream_id)
+        out = torch.empty(max(1, n) * self.T, self.cfg.vit_width, dtype=torch.float32, device=self.device)
+        check(self.lib.gitb200_streams_window(self.h, stream_id, _ptr(out), self._stream()), self.h, "gitb200_streams_window")
+        return out
+
     def set_fold_layernorm(self, enable: bool) -> None:
         """Opt-in (default off, DESIGN.md dead ends): ViT ln_1/ln_2 folded into the QKV/fc1 GEMM epilogues instead of separate LayerNorm kernels."""
         check(self.lib.gitb200_set_fold_layernorm(self.h, 1 if enable else 0), self.h, "gitb200_set_fold_layernorm")

@@ -19,7 +19,7 @@ Differences from the reference, all deliberate (DESIGN.md):
 from __future__ import annotations
 
 import functools
-from typing import Callable, List, Optional, Sequence
+from typing import Callable, Dict, List, Optional, Sequence
 
 import numpy as np
 import torch
@@ -771,3 +771,77 @@ class StreamingCaptioner:
         if not self.sliding:
             self.engine.stream_reset()
         return self.latest_caption
+
+
+class MultiStreamCaptioner:
+    """The webcam loop of src/real_time_inference.py:38-61 for many cameras on ONE engine: every camera (stream id
+    0 .. n_streams-1) has its own stride counter and its own window of per-frame ViT features in the engine's stream pool.
+    ``push({id: frame})`` takes the frames that arrived this tick; the frames due (every `stride`-th of each camera) are
+    encoded as one ViT batch per frame size, and the windows that completed are captioned as one decode batch per
+    held-frame count.  ``sliding=False`` reproduces the reference (``frames.clear()`` after each caption, :61);
+    ``sliding=True`` re-captions a camera on every frame it pushes, reusing the other frames' features.
+    The constructor (re)configures the engine's pool: one captioner per engine."""
+
+    def __init__(self, teacher: GenerativeImageTextTeacher, n_streams: int, stride: int = 3, max_len: int = 25, beam_size: int = 1,
+                 sliding: bool = False):
+        if n_streams < 1 or stride < 1:
+            raise ValueError("n_streams and stride must be >= 1")
+        self.teacher, self.n_streams, self.stride, self.sliding = teacher, n_streams, stride, sliding
+        self.engine = teacher.model.engine()
+        self.window = teacher.model.num_image_with_embedding or 6
+        d = teacher.model.decoder
+        self.search = SearchConfig(beam_size=beam_size, max_steps=max_len + 1, length_penalty=d.length_penalty,
+                                   per_node_beam_size=d.per_node_beam_size, num_keep_best=1)
+        self._counter = [0] * n_streams
+        self._raw = {}  # (k, H, W) -> persistent device buffer: repeated shapes replay the library's CUDA graphs
+        self.latest_caption = [""] * n_streams
+        self.engine.streams_configure(n_streams)
+
+    def reset(self, stream_ids) -> None:
+        """Empty the windows (and stride counters) of these cameras, e.g. after a scene cut or a reconnect."""
+        ids = list(stream_ids)
+        for sid in ids:
+            self._counter[sid] = 0
+        self.engine.streams_reset(ids)
+
+    @torch.no_grad()
+    def push(self, frames: Dict[int, torch.Tensor]) -> Dict[int, str]:
+        """frames: {stream id: uint8 [H, W, 3] BGR frame} for the cameras that delivered one this tick (host or device).
+        Returns {stream id: new caption} for the cameras whose window produced a caption."""
+        due = []
+        for sid, frame in frames.items():
+            if not 0 <= sid < self.n_streams:
+                raise KeyError(f"unknown stream id {sid} (this captioner has ids 0..{self.n_streams - 1})")
+            self._counter[sid] += 1
+            if self._counter[sid] < self.stride:
+                continue
+            self._counter[sid] = 0
+            due.append((sid, frame))
+        if not due:
+            return {}
+        self.teacher.model._vf_token = None  # the pool's windows replace whatever an earlier infer() left resident
+        for (h, w), group in _group_by(due, lambda it: tuple(it[1].shape[:2])).items():
+            ids = [sid for sid, _ in group]
+            key = (len(ids), h, w)
+            if key not in self._raw:
+                self._raw[key] = torch.empty(len(ids), h, w, 3, dtype=torch.uint8, device=self.engine.device)
+            buf = self._raw[key]
+            torch.stack([f.to(buf.device, non_blocking=True) for _, f in group], out=buf)
+            self.engine.streams_push_u8(ids, buf)
+        ready = [sid for sid, _ in due if self.engine.streams_frames(sid) >= self.window]
+        out = {}
+        for _, ids in _group_by(ready, self.engine.streams_frames).items():
+            tokens, _ = self.engine.streams_caption(ids, self.search)
+            for sid, row in zip(ids, tokens[:, 0].tolist()):
+                out[sid] = self.latest_caption[sid] = self.teacher.tokenizer.decode(row, skip_special_tokens=True)
+            if not self.sliding:
+                self.engine.streams_reset(ids)
+        return out
+
+
+def _group_by(items, key):
+    """Stable grouping: {key: [items in their original order]} with the keys in order of first appearance."""
+    groups = {}
+    for it in items:
+        groups.setdefault(key(it), []).append(it)
+    return groups
