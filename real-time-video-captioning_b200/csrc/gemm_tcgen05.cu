@@ -451,7 +451,8 @@ cudaError_t gemm_bf16(const GemmArgs& a, cudaStream_t stream, int force_bn) {
     g_err = "gemm_bf16: unsupported shape/stride (need N%128==0, K%8==0, 16-byte aligned rows)";
     return cudaErrorInvalidValue;
   }
-  if ((a.lnl_gamma != nullptr || a.sc_kv != nullptr) && !(force_bn == 1 || (force_bn == 0 && a.M <= 8))) {
+  // checked here, not in gemv_skinny: a shape the skinny kernel declines would otherwise run on a tensor-core kernel WITHOUT the fusion
+  if ((a.lnl_gamma != nullptr || a.sc_kv != nullptr) && (a.M > 8 || (force_bn != 0 && force_bn != 1) || a.gin > 0 || a.res_periodic)) {
     g_err = "gemm_bf16: LayerNorm-on-load / K-V scatter exist only in the skinny kernel (M <= 8)";
     return cudaErrorInvalidValue;
   }

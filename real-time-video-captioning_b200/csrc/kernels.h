@@ -77,7 +77,7 @@ void gemm_profile_read(double* ms, double* flops, long long* launches);
 struct LayerNormArgs {
   const bf16* x = nullptr;
   int ldx = 0;
-  int rows = 0, cols = 0;  // cols % 256 == 0 or cols == 768/1024; handled generically for cols % 8 == 0, cols <= 4096
+  int rows = 0, cols = 0;  // cols == 768 or 1024 (layernorm_bf16 returns cudaErrorInvalidValue for any other width)
   const float* gamma = nullptr;
   const float* beta = nullptr;
   float eps = 1e-5f;

@@ -204,6 +204,20 @@ def test_library_exports_every_declared_symbol_and_binding_covers_them():
     assert b"sm_100a" in lib.gitb200_version()
 
 
+def test_op_modes_shim_builds_and_links_against_the_library():
+    """tests/cuda/op_modes.cpp (the operator-mode tests' entry points over kernels.h) must keep compiling and resolving its
+    launchers when an argument struct changes, also where no GPU runs the tests that use it."""
+    import op_modes_shim
+    lib_mod = importlib.import_module("real-time-video-captioning_b200._lib")
+    if not os.path.exists(lib_mod.LIB_PATH):
+        pytest.skip("libgitb200.so is not built")
+    if op_modes_shim.compiler() is None:
+        pytest.skip("no C++ compiler")
+    lib_mod.load()
+    shim = op_modes_shim.load()
+    assert shim.opm_text_attention_workspace_floats(4, 12, 3) == 4 * 12 * 3 * (64 + 2)
+
+
 @pytest.mark.skipif(torch.cuda.is_available(), reason="checks the no-GPU failure mode")
 def test_no_gpu_means_loud_failure_not_fallback():
     lib_mod = importlib.import_module("real-time-video-captioning_b200._lib")

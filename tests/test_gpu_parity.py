@@ -269,26 +269,30 @@ def test_op_attention_growing_scores(g, n_groups, group_len, heads, gain):
 
 @pytest.mark.parametrize("nb,keep,max_steps,eos_boost", [(1, 1, 6, 0.0), (1, 1, 15, 3.0), (4, 1, 15, 2.0), (4, 3, 10, 4.0), (3, 2, 8, 6.0)])
 def test_op_search_exact(g, nb, keep, max_steps, eos_boost):
-    """Device search == restated reference loop (model.py:479-678) on identical score sequences."""
+    """Device search == restated reference loop (model.py:479-678) on identical score sequences.  Two row geometries: V = 1000
+    in rows of 1024, and the GIT vocabulary (30522, not a multiple of 8: the tail path) in rows of 30720 whose padding columns
+    hold +1e4 -- a search that read a padding column would pick it (the engine's padding logits are exact zeros)."""
     from importlib import import_module
     eng = import_module("real-time-video-captioning_b200.engine")
-    V, ld, n_clips, sos, eos = 1000, 1024, 5, 101, 102
-    gen = torch.Generator().manual_seed(nb * 100 + max_steps)
-    logits = torch.randn(max_steps - 1, n_clips * nb, ld, generator=gen) * 2
-    logits[:, :, eos] += eos_boost * torch.rand(max_steps - 1, n_clips * nb, generator=gen) * 2
-    sp = g.SearchConfig(beam_size=nb, max_steps=max_steps, length_penalty=0.6, per_node_beam_size=2, num_keep_best=keep)
-    tok, lp = eng.op_search(logits.cuda(), V, n_clips, sos, eos, sp)
-    t = {"i": 0}
+    n_clips, sos, eos = 5, 101, 102
+    for V, ld in ((1000, 1024), (30522, 30720)):
+        gen = torch.Generator().manual_seed(nb * 100 + max_steps)
+        logits = torch.randn(max_steps - 1, n_clips * nb, ld, generator=gen) * 2
+        logits[:, :, eos] += eos_boost * torch.rand(max_steps - 1, n_clips * nb, generator=gen) * 2
+        logits[:, :, V:] = 1e4
+        sp = g.SearchConfig(beam_size=nb, max_steps=max_steps, length_penalty=0.6, per_node_beam_size=2, num_keep_best=keep)
+        tok, lp = eng.op_search(logits.cuda(), V, n_clips, sos, eos, sp)
+        t = {"i": 0}
 
-    def step(ids):
-        s = logits[t["i"], :, :V]
-        t["i"] += 1
-        return s.clone()
-    dec, olp, _ = so.search(torch.full((n_clips, 1), sos, dtype=torch.long), step, eos_index=eos, max_steps=max_steps,
-                            beam_size=nb, length_penalty=0.6, per_node_beam_size=2, num_keep_best=keep, save_logits=False)
-    dec = dec.view(n_clips, keep, max_steps)
-    assert torch.equal(tok.cpu().long(), dec), (tok.cpu()[0], dec[0])
-    assert torch.allclose(lp.cpu(), olp, atol=2e-5, rtol=1e-5), (lp.cpu() - olp).abs().max()
+        def step(ids):
+            s = logits[t["i"], :, :V]
+            t["i"] += 1
+            return s.clone()
+        dec, olp, _ = so.search(torch.full((n_clips, 1), sos, dtype=torch.long), step, eos_index=eos, max_steps=max_steps,
+                                beam_size=nb, length_penalty=0.6, per_node_beam_size=2, num_keep_best=keep, save_logits=False)
+        dec = dec.view(n_clips, keep, max_steps)
+        assert torch.equal(tok.cpu().long(), dec), (V, tok.cpu()[0], dec[0])
+        assert torch.allclose(lp.cpu(), olp, atol=2e-5, rtol=1e-5), (V, (lp.cpu() - olp).abs().max())
 
 
 # ------------------------------------------------------------------------------------------ model level
