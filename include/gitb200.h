@@ -53,6 +53,23 @@ typedef struct {
                              re-order (model.py:623-634 is commented out); 1 = re-index by parent beam */
 } gitb200_search_params;
 
+/* The search's sampling / penalty arguments (model.py:479-480, :524-554).  top_k = 0 and top_p = 1 disable the filters;
+ * temperature, top_k and top_p act only with do_sample.  seed is the Philox4x32-10 key of the draws: a clip's sample depends
+ * only on (seed, its index in the call, its scores).  All-default values (do_sample 0, repetition_penalty 1,
+ * num_return_sequences 1) select exactly the calls without this struct. */
+typedef struct {
+  int do_sample;              /* 0: beam / greedy; 1: sample per_node_beam_size words per beam row, without replacement */
+  int top_k;                  /* keep the top max(top_k, 2) scores, ties included (0 = off); must keep at least
+                                 per_node_beam_size tokens, as torch.multinomial without replacement needs */
+  float top_p;                /* nucleus: keep the sorted prefix whose mass before the token is <= top_p, >= 3 tokens (1 = off).
+                                 Where it keeps fewer tokens than per_node_beam_size (the reference raises), the missing
+                                 draws are removed tokens in index order with score -inf */
+  float temperature;          /* scores / temperature before filtering (> 0) */
+  float repetition_penalty;   /* every distinct token of a row's history: x * rp if x < 0 else x / rp (> 0; 1 = off) */
+  int num_return_sequences;   /* independent searches per clip (>= 1); output row i * nrs + j = sequence j of clip i */
+  uint64_t seed;
+} gitb200_sample_params;
+
 /* ---- lifetime ------------------------------------------------------------------------------- */
 int gitb200_create(const gitb200_config* cfg, int device, gitb200_ctx** out);
 void gitb200_destroy(gitb200_ctx* ctx);
@@ -111,6 +128,17 @@ int gitb200_caption(gitb200_ctx* ctx, const float* frames_dev, int n_clips, int 
  * it equals n_clips.  Finished clips never change again, so tokens / scores are identical either way; only calls that
  * are being captured into a CUDA graph always run all steps.  gitb200_last_decode_steps: steps the last decode enqueued
  * (= len(saved_logits) of the reference; rows of logits_dev beyond it are not written). */
+/* gitb200_decode / gitb200_caption with the sampling / penalty arguments (sp_ext must not be NULL).  tokens_dev: int32
+ * [n_clips * nrs, num_keep_best, max_steps], logprobs_dev fp32 [n_clips * nrs, num_keep_best], logits_dev (optional) fp32
+ * [max_steps-1, n_clips*nrs*beam_size, logits_ld]: the scores BEFORE penalty and temperature (model.py:521).  The visual
+ * pass and visual K/V are computed once per clip and shared by its nrs * beam_size rows.  Invalid values (temperature <= 0,
+ * top_p outside (0, 1], repetition_penalty <= 0, nrs < 1, more rows per clip than the decoder pass takes, the beam limits)
+ * fail with GITB200_ERR_INVALID before anything is enqueued.  A CUDA graph captured for these calls replays for any seed. */
+int gitb200_decode_ext(gitb200_ctx* ctx, const gitb200_search_params* sp, const gitb200_sample_params* sp_ext,
+                       int32_t* tokens_dev, float* logprobs_dev, float* logits_dev, void* stream);
+int gitb200_caption_ext(gitb200_ctx* ctx, const float* frames_dev, int n_clips, int n_frames, const gitb200_search_params* sp,
+                        const gitb200_sample_params* sp_ext, int32_t* tokens_dev, float* logprobs_dev, float* logits_dev,
+                        void* stream);
 int gitb200_set_early_exit(gitb200_ctx* ctx, int every_steps);
 int gitb200_last_decode_steps(const gitb200_ctx* ctx);
 /* Latency mode of the search loop (default on): the search of ONE clip (gitb200_caption / _decode / _stream_caption with one
@@ -346,6 +374,11 @@ int gitb200_op_text_attention(const void* q_dev, const void* vis_kv_dev, const v
 /* Search on a pre-computed score sequence: logits_dev fp32 [max_steps-1, n_clips*beam, ld]. */
 int gitb200_op_search(const float* logits_dev, int ld, int vocab, int n_clips, int sos, int eos,
                       const gitb200_search_params* sp, int32_t* tokens_dev, float* logprobs_dev, void* stream);
+/* The same with the sampling / penalty arguments: logits_dev [max_steps-1, n_clips*nrs*beam, ld], tokens_dev
+ * [n_clips * nrs, num_keep_best, max_steps]. */
+int gitb200_op_search_ext(const float* logits_dev, int ld, int vocab, int n_clips, int sos, int eos,
+                          const gitb200_search_params* sp, const gitb200_sample_params* sp_ext, int32_t* tokens_dev,
+                          float* logprobs_dev, void* stream);
 
 /* Per-launch timing of the tcgen05 GEMM kernel with CUDA events recorded on the launching stream
  * (enable != 0 resets the counters).  read: summed milliseconds, summed 2*M*N*K flops, launches. */

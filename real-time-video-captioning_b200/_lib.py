@@ -6,7 +6,7 @@ from __future__ import annotations
 
 import ctypes
 import os
-from ctypes import POINTER, Structure, c_char_p, c_float, c_int, c_int32, c_int64, c_longlong, c_void_p
+from ctypes import POINTER, Structure, c_char_p, c_float, c_int, c_int32, c_int64, c_longlong, c_uint64, c_void_p
 
 HERE = os.path.dirname(os.path.abspath(__file__))
 LIB_PATH = os.path.join(HERE, "libgitb200.so")
@@ -38,6 +38,13 @@ class SearchParams(Structure):
     _fields_ = [
         ("beam_size", c_int), ("max_steps", c_int), ("per_node_beam_size", c_int), ("num_keep_best", c_int),
         ("length_penalty", c_float), ("reorder_cache", c_int),
+    ]
+
+
+class SampleParams(Structure):
+    _fields_ = [
+        ("do_sample", c_int), ("top_k", c_int), ("top_p", c_float), ("temperature", c_float),
+        ("repetition_penalty", c_float), ("num_return_sequences", c_int), ("seed", c_uint64),
     ]
 
 
@@ -74,6 +81,9 @@ SIGNATURES = {
     "gitb200_decode": (c_int, [c_void_p, POINTER(SearchParams), c_void_p, c_void_p, c_void_p, c_void_p]),
     "gitb200_caption": (c_int, [c_void_p, c_void_p, c_int, c_int, POINTER(SearchParams), c_void_p, c_void_p, c_void_p,
                                 c_void_p]),
+    "gitb200_decode_ext": (c_int, [c_void_p, POINTER(SearchParams), POINTER(SampleParams), c_void_p, c_void_p, c_void_p, c_void_p]),
+    "gitb200_caption_ext": (c_int, [c_void_p, c_void_p, c_int, c_int, POINTER(SearchParams), POINTER(SampleParams), c_void_p,
+                                    c_void_p, c_void_p, c_void_p]),
     "gitb200_set_fold_layernorm": (c_int, [c_void_p, c_int]),
     "gitb200_set_pipeline": (c_int, [c_void_p, c_int]),
     "gitb200_caption_from_host": (c_int, [c_void_p, c_void_p, c_int, c_int, c_int, POINTER(SearchParams), c_void_p, c_void_p, c_void_p, c_void_p, c_void_p]),
@@ -115,6 +125,8 @@ SIGNATURES = {
     "gitb200_op_attention_groups_mma": (c_int, [c_void_p, c_void_p, c_int, c_int, c_int, c_float, c_void_p]),
     "gitb200_op_search": (c_int, [c_void_p, c_int, c_int, c_int, c_int, c_int, POINTER(SearchParams), c_void_p, c_void_p,
                                   c_void_p]),
+    "gitb200_op_search_ext": (c_int, [c_void_p, c_int, c_int, c_int, c_int, c_int, POINTER(SearchParams), POINTER(SampleParams),
+                                      c_void_p, c_void_p, c_void_p]),
     "gitb200_launch_count": (c_longlong, [c_int]),
     "gitb200_graph_launches": (c_longlong, [c_void_p]),
     "gitb200_profile_gemm": (None, [c_int]),

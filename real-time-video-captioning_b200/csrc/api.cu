@@ -100,6 +100,7 @@ struct gitb200_ctx {
   Buf<uint8_t> stage_u8[2];  // host-path staging of raw uint8 video frames (gitb200_caption_host_u8)
   Buf<int> out_tok;
   Buf<float> out_lp;
+  Buf<unsigned long long> seed_dev;  // Philox key of the sampling search, copied in before any (graphed) launch reads it
   cudaStream_t copy_stream = nullptr, comp_stream = nullptr;
   // The caller's stream that last received work of this context (every entry point with a `stream` argument is asynchronous).
   // The host-frame entry points run on the context's private NON-BLOCKING streams, which nothing orders behind that stream --
@@ -117,9 +118,10 @@ struct gitb200_ctx {
     const void *p0 = nullptr, *p1 = nullptr, *p2 = nullptr;
     int i0 = 0, i1 = 0, i2 = 0, i3 = 0, i4 = 0, i5 = 0;
     gitb200_search_params sp{};
+    gitb200_sample_params smp{};  // seed always 0: the seed is read from seed_dev, so a graph replays for any seed
     bool operator==(const GraphKey& o) const {
       return kind == o.kind && p0 == o.p0 && p1 == o.p1 && p2 == o.p2 && i0 == o.i0 && i1 == o.i1 && i2 == o.i2 && i3 == o.i3 &&
-             i4 == o.i4 && i5 == o.i5 && memcmp(&sp, &o.sp, sizeof(sp)) == 0;
+             i4 == o.i4 && i5 == o.i5 && memcmp(&sp, &o.sp, sizeof(sp)) == 0 && memcmp(&smp, &o.smp, sizeof(smp)) == 0;
     }
   };
   struct GraphEntry {
@@ -833,13 +835,22 @@ int make_search_state(gitb200_ctx* c, int n_clips, int V, int ldl, int sos_unuse
   return 0;
 }
 
+// smp (optional, active sampling / penalty / return-sequence parameters, validated by check_sample): the search runs over
+// B * nrs entries of nb rows each, the rows of one clip (nrs * nb) sharing its visual K/V; the persistent kernel is not used.
 int run_decode(gitb200_ctx* c, const gitb200_search_params& sp, int32_t* tokens_out, float* logprobs_out, float* logits_out,
-               cudaStream_t s) {
+               cudaStream_t s, const gitb200_sample_params* smp = nullptr) {
   const gitb200_config& k = c->cfg;
-  const int B = c->cur_clips, nb = sp.beam_size, rows = B * nb;
+  const int nrs = smp ? smp->num_return_sequences : 1;
+  const int B = c->cur_clips, nb = sp.beam_size, entries = B * nrs, rows = entries * nb;
   if (sp.max_steps > k.max_positions) return fail(c, GITB200_ERR_INVALID, "max_steps %d exceeds the %d text positions", sp.max_steps, k.max_positions);
   SearchState st;
-  TRY(make_search_state(c, B, k.vocab, c->vocab_pad, k.sos, k.eos, sp, &st));
+  TRY(make_search_state(c, entries, k.vocab, c->vocab_pad, k.sos, k.eos, sp, &st));
+  SampleState ss{};
+  const bool ext_step = smp && (smp->do_sample || smp->repetition_penalty != 1.f);
+  if (smp) {
+    ss.do_sample = smp->do_sample; ss.top_k = smp->top_k; ss.nrs = nrs; ss.pnb = sp.per_node_beam_size;
+    ss.top_p = smp->top_p; ss.temperature = smp->temperature; ss.rp = smp->repetition_penalty; ss.seed = c->seed_dev.p;
+  }
   if (!c->visual_pass_done) TRY(run_visual_pass(c, false, nullptr, 0, s));
   TRY(ensure_text(c, rows, rows, sp.max_steps));
   if (!logits_out) ENSURE(c, c->logits, (size_t)rows * c->vocab_pad);
@@ -847,7 +858,7 @@ int run_decode(gitb200_ctx* c, const gitb200_search_params& sp, int32_t* tokens_
   // search step of every step -- runs as one persistent cooperative kernel whose phases are separated by grid barriers
   // instead of kernel boundaries (decode_mega.cu; bit-identical to the launch sequence below, which remains the path for
   // everything else and for devices that cannot keep the grid resident).  It leaves its loop itself once the clip is done.
-  if (c->persistent_decode && B == 1 && rows <= 4 && logits_out == nullptr && k.hidden == 768 && k.dec_layers <= MEGA_MAX_LAYERS &&
+  if (c->persistent_decode && !smp && B == 1 && rows <= 4 && logits_out == nullptr && k.hidden == 768 && k.dec_layers <= MEGA_MAX_LAYERS &&
       !gemm_profile_enabled()) {
     MegaArgs m;
     memset(&m, 0, sizeof(m));
@@ -908,12 +919,16 @@ int run_decode(gitb200_ctx* c, const gitb200_search_params& sp, int32_t* tokens_
     const int n = steps - t0 < seg ? steps - t0 : seg;
     gitb200_ctx::GraphKey key;
     key.kind = 5; key.i0 = B; key.i1 = t0; key.i2 = n; key.i3 = c->cur_nv; key.sp = sp; key.p0 = logits_out;
+    if (smp) {
+      key.smp = *smp;
+      key.smp.seed = 0;
+    }
     const int r = run_graphed(c, key, s, graphable, [&]() -> int {
       if (t0 == 0) CUDA_OK(c, search_init(st, k.sos, s));
       for (int t = t0; t < t0 + n; ++t) {
         const int parity = t & 1;
         TextPass tp;
-        tp.n_clips = B; tp.rows_per_clip = nb; tp.max_len = sp.max_steps;
+        tp.n_clips = B; tp.rows_per_clip = nrs * nb; tp.max_len = sp.max_steps;
         tp.tokens = st.cur_tok; tp.positions = nullptr; tp.pos_const = t;
         tp.n_text = nullptr; tp.n_text_const = t + 1;
         tp.anc = sp.reorder_cache ? (parity ? st.anc_tmp : st.anc) : nullptr;
@@ -921,7 +936,10 @@ int run_decode(gitb200_ctx* c, const gitb200_search_params& sp, int32_t* tokens_
         tp.logits = logits_out ? logits_out + (size_t)t * rows * c->vocab_pad : c->logits.p;
         tp.hidden_out = nullptr;
         TRY(run_text_pass(c, tp, s));
-        CUDA_OK(c, search_step(st, tp.logits, t + 1, parity, s));
+        if (ext_step)
+          CUDA_OK(c, sample_step(st, ss, tp.logits, t + 1, parity, t, s));
+        else
+          CUDA_OK(c, search_step(st, tp.logits, t + 1, parity, s));
       }
       return 0;
     });
@@ -930,7 +948,7 @@ int run_decode(gitb200_ctx* c, const gitb200_search_params& sp, int32_t* tokens_
     if (poll_done && t0 + n < steps) {
       CUDA_OK(c, cudaMemcpyAsync(c->h_done, st.done_count, sizeof(int), cudaMemcpyDeviceToHost, s));
       CUDA_OK(c, cudaStreamSynchronize(s));
-      if (*c->h_done >= B) break;
+      if (*c->h_done >= entries) break;
     }
   }
   CUDA_OK(c, search_finalize(st, tokens_out, logprobs_out, s));
@@ -946,7 +964,7 @@ void free_workspaces(gitb200_ctx* c) {
   fr(c->tx); fr(c->tq); fr(c->ta); fr(c->tb); fr(c->tc); fr(c->tf); fr(c->logits); fr(c->partial); fr(c->vf_in_f32);
   fr(c->ibuf); fr(c->dbuf); fr(c->fbuf); fr(c->pos_arr); fr(c->ntext_arr); fr(c->tok_arr); fr(c->stage[0]); fr(c->stage[1]); fr(c->stage_u8[0]); fr(c->stage_u8[1]);
   fr(c->out_tok); fr(c->out_lp); fr(c->stats_a); fr(c->stats_b); fr(c->ring);
-  fr(c->pool); fr(c->pool_rows); fr(c->pool_oldest);
+  fr(c->pool); fr(c->pool_rows); fr(c->pool_oldest); fr(c->seed_dev);
 }
 
 // second workspace set that shares this context's (read-only) weights
@@ -1455,15 +1473,16 @@ int gitb200_decode(gitb200_ctx* c, const gitb200_search_params* sp, int32_t* tok
 }
 
 static int caption_eager(gitb200_ctx* c, const float* frames, int n_clips, int n_frames, const gitb200_search_params* sp,
-                         int32_t* tokens, float* logprobs, float* logits, void* stream) {
+                         int32_t* tokens, float* logprobs, float* logits, void* stream, const gitb200_sample_params* smp) {
   int r = gitb200_encode(c, frames, n_clips, n_frames, nullptr, stream);
   if (r) return r;
+  if (smp) return run_decode(c, *sp, tokens, logprobs, logits, caller_stream(c, stream), smp);
   return gitb200_decode(c, sp, tokens, logprobs, logits, stream);
 }
 
-int gitb200_caption(gitb200_ctx* c, const float* frames, int n_clips, int n_frames, const gitb200_search_params* sp,
-                    int32_t* tokens, float* logprobs, float* logits, void* stream) {
-  if (!c || !sp) return fail(c, GITB200_ERR_INVALID, "bad caption argument");
+// gitb200_caption (smp == nullptr) and gitb200_caption_ext with active sampling parameters (the seed already in seed_dev)
+static int caption_impl(gitb200_ctx* c, const float* frames, int n_clips, int n_frames, const gitb200_search_params* sp,
+                        const gitb200_sample_params* smp, int32_t* tokens, float* logprobs, float* logits, void* stream) {
   // Latency mode: a small batch is launch-bound (~850 kernels per caption), so the second call with the same
   // buffers / shapes on a capturable stream is recorded into a CUDA graph and later calls replay it.
   cudaStream_t s = caller_stream(c, stream);
@@ -1471,8 +1490,12 @@ int gitb200_caption(gitb200_ctx* c, const float* frames, int n_clips, int n_fram
     gitb200_ctx::GraphKey key;
     key.kind = 0; key.p0 = frames; key.p1 = tokens; key.p2 = logprobs; key.i0 = n_clips; key.i1 = n_frames;
     key.i2 = logits != nullptr; key.sp = *sp;
+    if (smp) {
+      key.smp = *smp;
+      key.smp.seed = 0;
+    }
     CUDA_OK(c, cudaSetDevice(c->device));
-    const int r = run_graphed(c, key, s, logits == nullptr, [&]() { return caption_eager(c, frames, n_clips, n_frames, sp, tokens, logprobs, logits, stream); });
+    const int r = run_graphed(c, key, s, logits == nullptr, [&]() { return caption_eager(c, frames, n_clips, n_frames, sp, tokens, logprobs, logits, stream, smp); });
     if (r == 1) {  // replayed: host-side state the eager path would have left behind
       const int F = (c->cfg.num_image_with_embedding > 0 && n_frames > c->cfg.num_image_with_embedding) ? c->cfg.num_image_with_embedding : n_frames;
       c->cur_clips = n_clips; c->cur_nv = F * c->T; c->visual_pass_done = true; c->visual_pass_full = 0; c->step_rows_per_clip = 0;
@@ -1482,7 +1505,7 @@ int gitb200_caption(gitb200_ctx* c, const float* frames, int n_clips, int n_fram
     return r;
   }
   if (logits == nullptr && frames && tokens && logprobs && c->finalized && n_clips > 0 && n_frames > 0) {
-    const int chunk = pipeline_chunk_for(c, n_clips);
+    const int chunk = smp ? 0 : pipeline_chunk_for(c, n_clips);
     if (chunk > 0) {
       CUDA_OK(c, cudaSetDevice(c->device));
       return caption_pipelined(c, frames, n_clips, n_frames, *sp, tokens, logprobs, s, chunk);
@@ -1512,7 +1535,7 @@ int gitb200_caption(gitb200_ctx* c, const float* frames, int n_clips, int n_fram
       } else if (r != 0) {
         return r;
       }
-      TRY(run_decode(c, *sp, tokens, logprobs, nullptr, gs));
+      TRY(run_decode(c, *sp, tokens, logprobs, nullptr, gs, smp));
       if (forked) {
         CUDA_OK(c, cudaEventRecord(c->ev_gjoin, gs));
         CUDA_OK(c, cudaStreamWaitEvent(s, c->ev_gjoin, 0));
@@ -1520,7 +1543,85 @@ int gitb200_caption(gitb200_ctx* c, const float* frames, int n_clips, int n_fram
       return GITB200_OK;
     }
   }
-  return caption_eager(c, frames, n_clips, n_frames, sp, tokens, logprobs, logits, stream);
+  return caption_eager(c, frames, n_clips, n_frames, sp, tokens, logprobs, logits, stream, smp);
+}
+
+int gitb200_caption(gitb200_ctx* c, const float* frames, int n_clips, int n_frames, const gitb200_search_params* sp,
+                    int32_t* tokens, float* logprobs, float* logits, void* stream) {
+  if (!c || !sp) return fail(c, GITB200_ERR_INVALID, "bad caption argument");
+  return caption_impl(c, frames, n_clips, n_frames, sp, nullptr, tokens, logprobs, logits, stream);
+}
+
+namespace {
+
+bool sample_active(const gitb200_sample_params& p) {
+  return p.do_sample != 0 || p.repetition_penalty != 1.f || p.num_return_sequences != 1;
+}
+
+// Every rejection of the *_ext entry points, before anything is enqueued.  n_clips = clips of the call (0: not known yet);
+// text_rows: whether the rows run through the decoder pass (text_attention's grid takes at most 65535 clip x row-chunk
+// blocks; a chunk is 4 rows, 2 rows for 2-3 rows per clip, 1 row for 1).
+int check_sample(gitb200_ctx* c, const gitb200_search_params& sp, const gitb200_sample_params& p, int V, int n_clips,
+                 int max_positions, bool text_rows) {
+  if (!(p.temperature > 0.f)) return fail(c, GITB200_ERR_INVALID, "temperature must be > 0 (got %g)", (double)p.temperature);
+  if (!(p.top_p > 0.f && p.top_p <= 1.f)) return fail(c, GITB200_ERR_INVALID, "top_p must lie in (0, 1] (got %g)", (double)p.top_p);
+  if (!(p.repetition_penalty > 0.f))
+    return fail(c, GITB200_ERR_INVALID, "repetition_penalty must be > 0 (got %g)", (double)p.repetition_penalty);
+  if (p.num_return_sequences < 1) return fail(c, GITB200_ERR_INVALID, "num_return_sequences must be >= 1 (got %d)", p.num_return_sequences);
+  const int nb = sp.beam_size, ml = sp.max_steps, nk = sp.num_keep_best;
+  if (nb < 1 || nb > 8 || sp.per_node_beam_size < 1 || nb * sp.per_node_beam_size > 16 || nk < 1 || nk > 15 || ml < 2)
+    return fail(c, GITB200_ERR_INVALID, "unsupported search parameters (beam %d, per-node %d, keep %d, max_steps %d)", nb,
+                sp.per_node_beam_size, nk, ml);
+  if (max_positions > 0 && ml > max_positions) return fail(c, GITB200_ERR_INVALID, "max_steps %d exceeds the %d text positions", ml, max_positions);
+  const long long rpc = (long long)p.num_return_sequences * nb, entries = (long long)n_clips * p.num_return_sequences;
+  const long long chunk = rpc >= 4 ? 4 : (rpc >= 2 ? 2 : 1);
+  if (entries > 65535 || (text_rows && (long long)n_clips * ((rpc + chunk - 1) / chunk) > 65535))
+    return fail(c, GITB200_ERR_INVALID, "%lld rows per clip (num_return_sequences %d x beam %d) for %d clips exceed the decoder pass's "
+                "65535 clip x row-chunk blocks / the search's 65535 entries", rpc, p.num_return_sequences, nb, n_clips);
+  // torch.multinomial(..., replacement=False) raises when fewer tokens survive the filters than it draws; top-k alone
+  // decides that before any score is seen
+  if (p.do_sample && p.top_k > 0 && (p.top_k < 2 ? 2 : p.top_k) < sp.per_node_beam_size && (p.top_k < 2 ? 2 : p.top_k) < V)
+    return fail(c, GITB200_ERR_INVALID, "top_k %d keeps fewer tokens than the %d draws per beam (per_node_beam_size)", p.top_k,
+                sp.per_node_beam_size);
+  if ((p.do_sample || p.repetition_penalty != 1.f) && sample_step_smem(V) > 200 * 1024)
+    return fail(c, GITB200_ERR_INVALID, "vocabulary %d too large for a shared-memory row (at most %d)", V, 200 * 1024 / 4);
+  return 0;
+}
+
+int upload_seed(gitb200_ctx* c, uint64_t seed, cudaStream_t s) {
+  ENSURE(c, c->seed_dev, 1);
+  // (a pageable source: the copy is staged before cudaMemcpyAsync returns, so the local may go out of scope)
+  const unsigned long long v = seed;
+  CUDA_OK(c, cudaMemcpyAsync(c->seed_dev.p, &v, sizeof(v), cudaMemcpyHostToDevice, s));
+  return 0;
+}
+
+}  // namespace
+
+int gitb200_decode_ext(gitb200_ctx* c, const gitb200_search_params* sp, const gitb200_sample_params* smp, int32_t* tokens,
+                       float* logprobs, float* logits, void* stream) {
+  if (!c || !sp || !smp) return fail(c, GITB200_ERR_INVALID, "bad decode_ext argument");
+  TRY(check_sample(c, *sp, *smp, c->cfg.vocab, c->cur_clips, c->cfg.max_positions, true));
+  if (!tokens || !logprobs) return fail(c, GITB200_ERR_INVALID, "bad decode_ext argument");
+  if (!c->finalized) return fail(c, GITB200_ERR_STATE, "call gitb200_finalize_weights first");
+  if (c->cur_clips <= 0) return fail(c, GITB200_ERR_STATE, "no visual features: call gitb200_encode or gitb200_set_visual_features first");
+  if (!sample_active(*smp)) return gitb200_decode(c, sp, tokens, logprobs, logits, stream);
+  CUDA_OK(c, cudaSetDevice(c->device));
+  cudaStream_t s = caller_stream(c, stream);
+  TRY(upload_seed(c, smp->seed, s));
+  return run_decode(c, *sp, tokens, logprobs, logits, s, smp);
+}
+
+int gitb200_caption_ext(gitb200_ctx* c, const float* frames, int n_clips, int n_frames, const gitb200_search_params* sp,
+                        const gitb200_sample_params* smp, int32_t* tokens, float* logprobs, float* logits, void* stream) {
+  if (!c || !sp || !smp) return fail(c, GITB200_ERR_INVALID, "bad caption_ext argument");
+  TRY(check_sample(c, *sp, *smp, c->cfg.vocab, n_clips, c->cfg.max_positions, true));
+  if (!frames || !tokens || !logprobs || n_clips < 1 || n_frames < 1) return fail(c, GITB200_ERR_INVALID, "bad caption_ext argument");
+  if (!c->finalized) return fail(c, GITB200_ERR_STATE, "call gitb200_finalize_weights first");
+  if (!sample_active(*smp)) return gitb200_caption(c, frames, n_clips, n_frames, sp, tokens, logprobs, logits, stream);
+  CUDA_OK(c, cudaSetDevice(c->device));
+  TRY(upload_seed(c, smp->seed, caller_stream(c, stream)));
+  return caption_impl(c, frames, n_clips, n_frames, sp, smp, tokens, logprobs, logits, stream);
 }
 
 int gitb200_stream_reset(gitb200_ctx* c) {
@@ -2130,6 +2231,48 @@ int gitb200_op_search(const float* logits, int ld, int vocab, int n_clips, int s
   if (tmp.ibuf.p) cudaFree(tmp.ibuf.p);
   if (tmp.dbuf.p) cudaFree(tmp.dbuf.p);
   if (tmp.fbuf.p) cudaFree(tmp.fbuf.p);
+  if (r) return fail(nullptr, r, "%s", tmp.err.c_str());
+  if (e != cudaSuccess) return fail(nullptr, GITB200_ERR_CUDA, "search: %s", cudaGetErrorString(e));
+  return GITB200_OK;
+}
+
+int gitb200_op_search_ext(const float* logits, int ld, int vocab, int n_clips, int sos, int eos, const gitb200_search_params* sp,
+                          const gitb200_sample_params* smp, int32_t* tokens, float* logprobs, void* stream) {
+  if (!sp || !smp) return fail(nullptr, GITB200_ERR_INVALID, "bad op_search_ext argument");
+  {
+    const int r = check_sample(nullptr, *sp, *smp, vocab, n_clips, 0, false);
+    if (r) return r;
+  }
+  if (!logits || !tokens || !logprobs || n_clips < 1 || vocab < 1 || ld < vocab)
+    return fail(nullptr, GITB200_ERR_INVALID, "bad op_search_ext argument");
+  if (!sample_active(*smp)) return gitb200_op_search(logits, ld, vocab, n_clips, sos, eos, sp, tokens, logprobs, stream);
+  gitb200_ctx tmp;  // scratch owner for the search buffers
+  cudaGetDevice(&tmp.device);
+  const int nrs = smp->num_return_sequences, entries = n_clips * nrs, rows = entries * sp->beam_size;
+  SearchState st;
+  int r = make_search_state(&tmp, entries, vocab, ld, sos, eos, *sp, &st);
+  cudaStream_t s = (cudaStream_t)stream;
+  cudaError_t e = cudaSuccess;
+  if (!r) r = upload_seed(&tmp, smp->seed, s);
+  if (!r) {
+    SampleState ss{};
+    ss.do_sample = smp->do_sample; ss.top_k = smp->top_k; ss.nrs = nrs; ss.pnb = sp->per_node_beam_size;
+    ss.top_p = smp->top_p; ss.temperature = smp->temperature; ss.rp = smp->repetition_penalty; ss.seed = tmp.seed_dev.p;
+    const bool ext_step = smp->do_sample || smp->repetition_penalty != 1.f;
+    e = search_init(st, sos, s);
+    int parity = 0;
+    for (int t = 0; e == cudaSuccess && t + 1 < sp->max_steps; ++t) {
+      const float* lt = logits + (size_t)t * rows * ld;
+      e = ext_step ? sample_step(st, ss, lt, t + 1, parity, t, s) : search_step(st, lt, t + 1, parity, s);
+      parity ^= 1;
+    }
+    if (e == cudaSuccess) e = search_finalize(st, tokens, logprobs, s);
+    if (e == cudaSuccess) e = cudaStreamSynchronize(s);
+  }
+  if (tmp.ibuf.p) cudaFree(tmp.ibuf.p);
+  if (tmp.dbuf.p) cudaFree(tmp.dbuf.p);
+  if (tmp.fbuf.p) cudaFree(tmp.fbuf.p);
+  if (tmp.seed_dev.p) cudaFree(tmp.seed_dev.p);
   if (r) return fail(nullptr, r, "%s", tmp.err.c_str());
   if (e != cudaSuccess) return fail(nullptr, GITB200_ERR_CUDA, "search: %s", cudaGetErrorString(e));
   return GITB200_OK;

@@ -182,6 +182,19 @@ cudaError_t search_step(const SearchState& s, const float* logits, int cur_len, 
 cudaError_t search_init(const SearchState& s, int sos, cudaStream_t stream);
 // decoded [n_clips, n_keep, max_len] (eos padded), logprobs [n_clips, n_keep]
 cudaError_t search_finalize(const SearchState& s, int* decoded, float* logprobs, cudaStream_t stream);
+// Extended search step (model.py:524-554): repetition penalty, and with do_sample temperature, top-k / top-p filtering
+// (min_tokens_to_keep = 2) and per_node_beam_size draws without replacement per beam row.  The search "clips" of `s` are
+// entries e = clip * nrs + j (return sequence j of clip `clip`), nb rows each.
+struct SampleState {
+  int do_sample, top_k, nrs, pnb;
+  float top_p, temperature, rp;
+  const unsigned long long* seed;  // device word: the Philox key
+};
+// Bytes of dynamic shared memory a row of `V` logits needs (the limit the caller checks before enqueueing anything).
+size_t sample_step_smem(int V);
+// step = t for cur_len = t + 1 (the Philox counter's step word)
+cudaError_t sample_step(const SearchState& s, const SampleState& p, const float* logits, int cur_len, int parity, int step,
+                        cudaStream_t stream);
 
 // ---- persistent single-clip decode kernel (decode_mega.cu): the whole search of ONE clip (rows = beams <= 4) in one launch
 constexpr int MEGA_MAX_LAYERS = 8;

@@ -353,9 +353,11 @@ __device__ __forceinline__ void search_row_staged(const SearchState& st, const f
 
 // Parts 3 + 4 of a search step: the reference's candidate walk over sh.cand_score / sh.cand_idx (the clip's top-C, ordered),
 // then the re-ordering of token rows / the ancestor table.  Same thread / sync contract as above.
+// done_on_max: is_done sees the maximum candidate score (the sampling branch, whose candidates are in sample order); otherwise
+// candidate 0, which is the maximum of a sorted top-C.
 template <class Sync>
 __device__ __forceinline__ void search_walk_reorder(const SearchState& st, int cur_len, int parity, int clip, int tid, Sync sync,
-                                                    SearchSmem& sh) {
+                                                    SearchSmem& sh, bool done_on_max = false) {
   const int nb = st.nb, V = st.V, C = st.cand;
   const int* tok_in = parity ? st.tokens_tmp : st.tokens;
   int* tok_out = parity ? st.tokens : st.tokens_tmp;
@@ -379,7 +381,10 @@ __device__ __forceinline__ void search_walk_reorder(const SearchState& st, int c
     int is_done = st.done[clip];
     if (!is_done) {
       // BeamHypotheses.is_done(best_sum_logprobs) with early_stopping=False
-      if (cnt >= nk) is_done = worst >= (double)cand_score[0] / pow((double)(max_len - 1), (double)st.length_penalty);
+      float best = cand_score[0];
+      if (done_on_max)
+        for (int c = 1; c < C; ++c) best = fmaxf(best, cand_score[c]);
+      if (cnt >= nk) is_done = worst >= (double)best / pow((double)(max_len - 1), (double)st.length_penalty);
     }
     int n_next = 0;
     if (!is_done) {

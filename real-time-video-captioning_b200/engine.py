@@ -9,7 +9,7 @@ from typing import Dict, Optional
 import torch
 
 from . import _lib
-from ._lib import Config, GitB200Error, SearchParams, check
+from ._lib import Config, GitB200Error, SampleParams, SearchParams, check
 
 VIT_CONFIGS = {
     # get_image_encoder(param['image_encoder_type']) of the reference (model.py:682-685)
@@ -31,6 +31,24 @@ class SearchConfig:
     def to_c(self) -> SearchParams:
         return SearchParams(self.beam_size, self.max_steps, self.per_node_beam_size, self.num_keep_best,
                             float(self.length_penalty), 1 if self.reorder_cache else 0)
+
+
+@dataclass
+class SampleConfig:
+    """search() sampling keyword arguments (model.py:479-480) and the decoder's repetition_penalty / temperature
+    (model.py:524-535), plus the seed of the device's counter-based RNG: a clip's sample depends only on (seed, its index
+    in the call, its scores).  top_k = 0 and top_p = 1.0 disable the filters."""
+    do_sample: bool = False
+    top_k: int = 0
+    top_p: float = 1.0
+    temperature: float = 1.0
+    repetition_penalty: float = 1.0
+    num_return_sequences: int = 1
+    seed: int = 0
+
+    def to_c(self) -> SampleParams:
+        return SampleParams(1 if self.do_sample else 0, int(self.top_k), float(self.top_p), float(self.temperature),
+                            float(self.repetition_penalty), int(self.num_return_sequences), int(self.seed) & (2 ** 64 - 1))
 
 
 def make_config(param: dict, sos: int, eos: int, *, vocab: int = 30522, hidden: int = 768, layers: int = 6,
@@ -142,31 +160,44 @@ class Engine:
               "gitb200_set_visual_features")
         self._cur_nv, self._cur_clips, self._step_rows = vf.shape[1], vf.shape[0], 0
 
-    def decode(self, n_clips: int, sp: SearchConfig, save_logits: bool = False):
-        """Search on the current visual features: (tokens int32 [B, keep, max_steps], logprobs [B, keep],
-        logits fp32 [max_steps-1, B*beam, ld] or None)."""
-        tokens = torch.empty(n_clips, sp.num_keep_best, sp.max_steps, dtype=torch.int32, device=self.device)
-        logprobs = torch.empty(n_clips, sp.num_keep_best, dtype=torch.float32, device=self.device)
-        logits = torch.empty(sp.max_steps - 1, n_clips * sp.beam_size, self.ld, dtype=torch.float32,
+    def _search_outputs(self, n_clips: int, sp: SearchConfig, sample: Optional[SampleConfig], save_logits: bool):
+        n = n_clips * (sample.num_return_sequences if sample is not None else 1)
+        tokens = torch.empty(n, sp.num_keep_best, sp.max_steps, dtype=torch.int32, device=self.device)
+        logprobs = torch.empty(n, sp.num_keep_best, dtype=torch.float32, device=self.device)
+        logits = torch.empty(sp.max_steps - 1, n * sp.beam_size, self.ld, dtype=torch.float32,
                              device=self.device) if save_logits else None
+        return tokens, logprobs, logits
+
+    def decode(self, n_clips: int, sp: SearchConfig, save_logits: bool = False, sample: Optional[SampleConfig] = None):
+        """Search on the current visual features: (tokens int32 [B, keep, max_steps], logprobs [B, keep],
+        logits fp32 [max_steps-1, B*beam, ld] or None).  With ``sample``, B becomes B * num_return_sequences (row
+        i * nrs + j = sequence j of clip i) and the logits are the scores before penalty and temperature."""
+        tokens, logprobs, logits = self._search_outputs(n_clips, sp, sample, save_logits)
         c = sp.to_c()
-        check(self.lib.gitb200_decode(self.h, ctypes.byref(c), _ptr(tokens), _ptr(logprobs), _ptr(logits), self._stream()),
-              self.h, "gitb200_decode")
+        if sample is None:
+            check(self.lib.gitb200_decode(self.h, ctypes.byref(c), _ptr(tokens), _ptr(logprobs), _ptr(logits), self._stream()),
+                  self.h, "gitb200_decode")
+        else:
+            x = sample.to_c()
+            check(self.lib.gitb200_decode_ext(self.h, ctypes.byref(c), ctypes.byref(x), _ptr(tokens), _ptr(logprobs), _ptr(logits),
+                                              self._stream()), self.h, "gitb200_decode_ext")
         if logits is not None:  # the step loop may have stopped early (`if all(done): break`, model.py:640)
             logits = logits[: self.last_decode_steps()]
         return tokens, logprobs, logits
 
-    def caption(self, frames: torch.Tensor, sp: SearchConfig, save_logits: bool = False):
+    def caption(self, frames: torch.Tensor, sp: SearchConfig, save_logits: bool = False, sample: Optional[SampleConfig] = None):
         assert frames.is_cuda and frames.dtype == torch.float32 and frames.dim() == 5
         frames = frames.contiguous()
         B, F = frames.shape[:2]
-        tokens = torch.empty(B, sp.num_keep_best, sp.max_steps, dtype=torch.int32, device=self.device)
-        logprobs = torch.empty(B, sp.num_keep_best, dtype=torch.float32, device=self.device)
-        logits = torch.empty(sp.max_steps - 1, B * sp.beam_size, self.ld, dtype=torch.float32,
-                             device=self.device) if save_logits else None
+        tokens, logprobs, logits = self._search_outputs(B, sp, sample, save_logits)
         c = sp.to_c()
-        check(self.lib.gitb200_caption(self.h, _ptr(frames), B, F, ctypes.byref(c), _ptr(tokens), _ptr(logprobs),
-                                       _ptr(logits), self._stream()), self.h, "gitb200_caption")
+        if sample is None:
+            check(self.lib.gitb200_caption(self.h, _ptr(frames), B, F, ctypes.byref(c), _ptr(tokens), _ptr(logprobs),
+                                           _ptr(logits), self._stream()), self.h, "gitb200_caption")
+        else:
+            x = sample.to_c()
+            check(self.lib.gitb200_caption_ext(self.h, _ptr(frames), B, F, ctypes.byref(c), ctypes.byref(x), _ptr(tokens),
+                                               _ptr(logprobs), _ptr(logits), self._stream()), self.h, "gitb200_caption_ext")
         n = self.cfg.num_image_with_embedding
         self._cur_nv, self._cur_clips, self._step_rows = (min(F, n) if n > 0 else F) * self.T, B, 0
         if logits is not None:
@@ -487,16 +518,24 @@ def op_text_attention(q: torch.Tensor, vis_kv: torch.Tensor, txt_kv, anc, n_clip
     return out
 
 
-def op_search(logits: torch.Tensor, vocab: int, n_clips: int, sos: int, eos: int, sp: SearchConfig):
-    """logits fp32 [max_steps-1, n_clips*beam, ld] (device) -> tokens [n_clips, keep, max_steps], logprobs."""
+def op_search(logits: torch.Tensor, vocab: int, n_clips: int, sos: int, eos: int, sp: SearchConfig,
+              sample: Optional[SampleConfig] = None):
+    """logits fp32 [max_steps-1, n_clips*beam, ld] (device) -> tokens [n_clips, keep, max_steps], logprobs.
+    With ``sample``: logits [max_steps-1, n_clips*nrs*beam, ld] -> tokens [n_clips*nrs, keep, max_steps]."""
     lib = _lib.load()
     logits = logits.contiguous()
-    tokens = torch.empty(n_clips, sp.num_keep_best, sp.max_steps, dtype=torch.int32, device=logits.device)
-    logprobs = torch.empty(n_clips, sp.num_keep_best, dtype=torch.float32, device=logits.device)
+    n = n_clips * (sample.num_return_sequences if sample is not None else 1)
+    tokens = torch.empty(n, sp.num_keep_best, sp.max_steps, dtype=torch.int32, device=logits.device)
+    logprobs = torch.empty(n, sp.num_keep_best, dtype=torch.float32, device=logits.device)
     c = sp.to_c()
     s = ctypes.c_void_p(torch.cuda.current_stream(logits.device).cuda_stream)
-    check(lib.gitb200_op_search(_ptr(logits), logits.shape[-1], vocab, n_clips, sos, eos, ctypes.byref(c), _ptr(tokens),
-                                _ptr(logprobs), s), None, "gitb200_op_search")
+    if sample is None:
+        check(lib.gitb200_op_search(_ptr(logits), logits.shape[-1], vocab, n_clips, sos, eos, ctypes.byref(c), _ptr(tokens),
+                                    _ptr(logprobs), s), None, "gitb200_op_search")
+    else:
+        x = sample.to_c()
+        check(lib.gitb200_op_search_ext(_ptr(logits), logits.shape[-1], vocab, n_clips, sos, eos, ctypes.byref(c),
+                                        ctypes.byref(x), _ptr(tokens), _ptr(logprobs), s), None, "gitb200_op_search_ext")
     return tokens, logprobs
 
 

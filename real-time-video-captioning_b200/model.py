@@ -25,7 +25,7 @@ import numpy as np
 import torch
 import torch.nn as nn
 
-from .engine import VIT_CONFIGS, Engine, SearchConfig, make_config
+from .engine import VIT_CONFIGS, Engine, SampleConfig, SearchConfig, make_config
 
 VOCAB_SIZE = 30522  # model.py:689
 
@@ -531,21 +531,38 @@ class GenerativeImageTextModel(nn.Module):
         return eng.decode_step(partial_captions[:, pos], pos).float()
 
     def infer(self, batch, visual_features, visual_features_valid, search_param=None):
-        """model.py:426-462."""
+        """model.py:426-462.
+
+        ``search_param['seed']`` (not a reference key) opts into the device's counter-based RNG: sampling, repetition
+        penalty and num_return_sequences then run in the fused device search, reproducible for a given seed but not
+        token-identical to torch's RNG.  Without it those settings take the generic host loop, as the reference does."""
         batch_size = visual_features.size(0)
         search_param = dict(search_param or {})
+        seed = search_param.pop("seed", None)
         eng = self.engine()
-        fast = (isinstance(self.decoder, GeneratorWithBeamSearchV2) and "prefix" not in batch
-                and not search_param.get("do_sample", False) and search_param.get("num_return_sequences", 1) == 1
-                and self.decoder.repetition_penalty == 1.0 and visual_features_valid is None
-                and not self._force_host_search)
+        fused = (isinstance(self.decoder, GeneratorWithBeamSearchV2) and "prefix" not in batch
+                 and visual_features_valid is None and not self._force_host_search)
+        fast = (fused and not search_param.get("do_sample", False) and search_param.get("num_return_sequences", 1) == 1
+                and self.decoder.repetition_penalty == 1.0)
+        sample = None
+        if fused and seed is not None:
+            do_sample = bool(search_param.get("do_sample", False))
+            top_k, top_p = search_param.get("top_k"), search_param.get("top_p")
+            if do_sample and (top_k is None or top_p is None):  # upstream top_k_top_p_filtering compares them with numbers
+                raise TypeError(f"sampling needs top_k and top_p (got top_k={top_k!r}, top_p={top_p!r})")
+            sample = SampleConfig(do_sample, int(top_k or 0), 1.0 if top_p is None else float(top_p), self.decoder.temperature,
+                                  self.decoder.repetition_penalty, search_param.get("num_return_sequences", 1), int(seed))
+            fast = True
         self.prev_encoded_layers = None
         if fast:
             if self._vf_token is not visual_features:
                 eng.set_visual_features(visual_features.to(eng.device))
                 self._vf_token = visual_features
             sc = self.decoder.search_config(search_param.get("num_keep_best", 1), self.cache_reorder == "correct")
-            tokens, logprobs, logits = eng.decode(batch_size, sc, save_logits=True)
+            if sample is None:
+                tokens, logprobs, logits = eng.decode(batch_size, sc, save_logits=True)
+            else:
+                tokens, logprobs, logits = eng.decode(batch_size, sc, save_logits=True, sample=sample)
             predicted = tokens.long()
             if sc.num_keep_best == 1:
                 predicted = predicted.squeeze(1)
