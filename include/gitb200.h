@@ -139,6 +139,21 @@ int gitb200_decode_ext(gitb200_ctx* ctx, const gitb200_search_params* sp, const 
 int gitb200_caption_ext(gitb200_ctx* ctx, const float* frames_dev, int n_clips, int n_frames, const gitb200_search_params* sp,
                         const gitb200_sample_params* sp_ext, int32_t* tokens_dev, float* logprobs_dev, float* logits_dev,
                         void* stream);
+/* Prompted search, batch['prefix'] (model.py:432-437): prefix_host int32 [prefix_rows, P] on the HOST, prefix_rows = 1 (one
+ * prompt for every clip) or n_clips; the prompt starts with the caller's first token (usually [CLS]), no SOS is added.  The
+ * first P - 1 prompt tokens of every clip run through ONE teacher-forced decoder pass (each clip's visual K/V read once),
+ * and the search starts at cur_len = P with the prompt as every row's history: max_steps - P steps (none for P >= max_steps:
+ * eos rows, log-prob -1e5).  tokens_dev [n_clips*nrs, keep, max_steps] WITH the prompt (the search's output; the reference's
+ * infer strips it with predicted[:, P:]); logits_dev (optional) [max_steps-P, n_clips*nrs*beam, ld].  sp_ext may be NULL.
+ * Rejected before anything is enqueued: P < 1, a NULL prompt, prefix_rows neither 1 nor n_clips, a token outside [0, vocab),
+ * P > max_positions, and every rejection of the *_ext entry points.  A CUDA graph is keyed by P, not by the tokens.
+ * P = 1 with the SOS token gives exactly what gitb200_decode / _caption (/ _ext) give. */
+int gitb200_decode_prefix(gitb200_ctx* ctx, const gitb200_search_params* sp, const gitb200_sample_params* sp_ext,
+                          const int32_t* prefix_host, int prefix_rows, int P, int32_t* tokens_dev, float* logprobs_dev,
+                          float* logits_dev, void* stream);
+int gitb200_caption_prefix(gitb200_ctx* ctx, const float* frames_dev, int n_clips, int n_frames, const gitb200_search_params* sp,
+                           const gitb200_sample_params* sp_ext, const int32_t* prefix_host, int prefix_rows, int P,
+                           int32_t* tokens_dev, float* logprobs_dev, float* logits_dev, void* stream);
 int gitb200_set_early_exit(gitb200_ctx* ctx, int every_steps);
 int gitb200_last_decode_steps(const gitb200_ctx* ctx);
 /* Latency mode of the search loop (default on): the search of ONE clip (gitb200_caption / _decode / _stream_caption with one
@@ -379,6 +394,10 @@ int gitb200_op_search(const float* logits_dev, int ld, int vocab, int n_clips, i
 int gitb200_op_search_ext(const float* logits_dev, int ld, int vocab, int n_clips, int sos, int eos,
                           const gitb200_search_params* sp, const gitb200_sample_params* sp_ext, int32_t* tokens_dev,
                           float* logprobs_dev, void* stream);
+/* The same search with a prompt (see gitb200_decode_prefix) over pre-computed scores [max_steps-P, rows, ld]; sp_ext may be NULL. */
+int gitb200_op_search_prefix(const float* logits_dev, int ld, int vocab, int n_clips, int eos, const gitb200_search_params* sp,
+                             const gitb200_sample_params* sp_ext, const int32_t* prefix_host, int prefix_rows, int P,
+                             int32_t* tokens_dev, float* logprobs_dev, void* stream);
 
 /* Per-launch timing of the tcgen05 GEMM kernel with CUDA events recorded on the launching stream
  * (enable != 0 resets the counters).  read: summed milliseconds, summed 2*M*N*K flops, launches. */

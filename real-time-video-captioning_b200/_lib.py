@@ -84,6 +84,10 @@ SIGNATURES = {
     "gitb200_decode_ext": (c_int, [c_void_p, POINTER(SearchParams), POINTER(SampleParams), c_void_p, c_void_p, c_void_p, c_void_p]),
     "gitb200_caption_ext": (c_int, [c_void_p, c_void_p, c_int, c_int, POINTER(SearchParams), POINTER(SampleParams), c_void_p,
                                     c_void_p, c_void_p, c_void_p]),
+    "gitb200_decode_prefix": (c_int, [c_void_p, POINTER(SearchParams), POINTER(SampleParams), c_void_p, c_int, c_int, c_void_p,
+                                      c_void_p, c_void_p, c_void_p]),
+    "gitb200_caption_prefix": (c_int, [c_void_p, c_void_p, c_int, c_int, POINTER(SearchParams), POINTER(SampleParams), c_void_p,
+                                       c_int, c_int, c_void_p, c_void_p, c_void_p, c_void_p]),
     "gitb200_set_fold_layernorm": (c_int, [c_void_p, c_int]),
     "gitb200_set_pipeline": (c_int, [c_void_p, c_int]),
     "gitb200_caption_from_host": (c_int, [c_void_p, c_void_p, c_int, c_int, c_int, POINTER(SearchParams), c_void_p, c_void_p, c_void_p, c_void_p, c_void_p]),
@@ -127,6 +131,8 @@ SIGNATURES = {
                                   c_void_p]),
     "gitb200_op_search_ext": (c_int, [c_void_p, c_int, c_int, c_int, c_int, c_int, POINTER(SearchParams), POINTER(SampleParams),
                                       c_void_p, c_void_p, c_void_p]),
+    "gitb200_op_search_prefix": (c_int, [c_void_p, c_int, c_int, c_int, c_int, POINTER(SearchParams), POINTER(SampleParams),
+                                         c_void_p, c_int, c_int, c_void_p, c_void_p, c_void_p]),
     "gitb200_launch_count": (c_longlong, [c_int]),
     "gitb200_graph_launches": (c_longlong, [c_void_p]),
     "gitb200_profile_gemm": (None, [c_int]),

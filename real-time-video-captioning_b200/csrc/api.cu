@@ -101,6 +101,10 @@ struct gitb200_ctx {
   Buf<int> out_tok;
   Buf<float> out_lp;
   Buf<unsigned long long> seed_dev;  // Philox key of the sampling search, copied in before any (graphed) launch reads it
+  // batch['prefix'] of a prompted decode, copied in before any (graphed) launch reads it: [clips][P] every clip's prompt,
+  // then [clips][P - 1] the prefill's token rows; prefix_kv: the prefill's K/V planes, [layers][P - 1][clips][2H]
+  Buf<int> prefix_dev;
+  Buf<bf16> prefix_kv;
   cudaStream_t copy_stream = nullptr, comp_stream = nullptr;
   // The caller's stream that last received work of this context (every entry point with a `stream` argument is asynchronous).
   // The host-frame entry points run on the context's private NON-BLOCKING streams, which nothing orders behind that stream --
@@ -575,8 +579,10 @@ struct TextPass {
   int n_text_const;
   const int* anc;        // ancestor table or nullptr
   int slot_div, n_slots, slot_is_clip;
-  float* logits;         // [rows, vocab_pad]
+  float* logits;         // [rows, vocab_pad]; nullptr: K/V only -- the pass ends after the last layer's K/V store
   float* hidden_out;     // optional fp32 [B, layers+1, Nv+L, H] (text rows written)
+  bf16* kv_plane = nullptr;    // optional: layer l's text K/V plane is kv_plane + l * kv_plane_stride instead of txt_kv[l]
+  size_t kv_plane_stride = 0;
 };
 
 int ensure_text(gitb200_ctx* c, int rows, int n_slots, int max_len) {
@@ -657,6 +663,7 @@ int run_text_pass(gitb200_ctx* c, const TextPass& t, cudaStream_t s) {
     return 0;
   };
 
+  auto plane = [&](int l) { return t.kv_plane ? t.kv_plane + (size_t)l * t.kv_plane_stride : c->txt_kv[l].p; };
   CUDA_OK(c, embed_text(t.tokens, t.positions, t.pos_const, rows, c->words_f32, c->pos_f32, c->lne_g, c->lne_b,
                         k.embed_ln_eps, H, c->tx.p, s));
   TRY(emit_hidden(0));
@@ -675,18 +682,19 @@ int run_text_pass(gitb200_ctx* c, const TextPass& t, cudaStream_t s) {
         if (l > 0) {
           g.lnl_gamma = c->dec[l - 1].lno_g; g.lnl_beta = c->dec[l - 1].lno_b; g.lnl_eps = k.bert_ln_eps; g.lnl_out = c->tx.p; g.lnl_ldo = H;
         }
-        g.sc_kv = c->txt_kv[l].p; g.sc_q_width = H; g.sc_kv_width = 2 * H; g.sc_pos = t.positions; g.sc_pos_const = t.pos_const;
+        g.sc_kv = plane(l); g.sc_q_width = H; g.sc_kv_width = 2 * H; g.sc_pos = t.positions; g.sc_pos_const = t.pos_const;
         g.sc_slot_div = t.slot_div; g.sc_n_slots = t.n_slots;
       }
       TRY(gemm(c, g, s));
     }
     if (!fused)
-      CUDA_OK(c, store_text_kv(c->tq.p, 3 * H, rows, 2 * H, H, t.positions, t.pos_const, t.slot_div, t.n_slots,
-                               c->txt_kv[l].p, s));
+      CUDA_OK(c, store_text_kv(c->tq.p, 3 * H, rows, 2 * H, H, t.positions, t.pos_const, t.slot_div, t.n_slots, plane(l), s));
+    // K/V only (the prompt prefill): nothing reads the last layer's attention, MLP or the vocabulary head
+    if (t.logits == nullptr && l + 1 == k.dec_layers) return 0;
     TextAttnArgs a;
     a.q = c->tq.p; a.ldq = 3 * H; a.n_clips = t.n_clips; a.rows_per_clip = t.rows_per_clip; a.heads = k.dec_heads;
     a.vis_kv = c->kv[l].p; a.ld_vis = 3 * H; a.k_off = H; a.v_off = 2 * H; a.Nv = Nv;
-    a.txt_kv = c->txt_kv[l].p; a.txt_slots = t.n_slots; a.text_slot_is_clip = t.slot_is_clip;
+    a.txt_kv = plane(l); a.txt_slots = t.n_slots; a.text_slot_is_clip = t.slot_is_clip;
     a.anc = t.anc; a.anc_ld = t.max_len; a.n_text = t.n_text; a.n_text_const = t.n_text_const; a.max_text = t.max_len;
     a.scale = scale; a.out = c->ta.p; a.ldo = H; a.partial = c->partial.p; a.splits = splits;
     const int pslot = dap_begin(s);
@@ -837,8 +845,12 @@ int make_search_state(gitb200_ctx* c, int n_clips, int V, int ldl, int sos_unuse
 
 // smp (optional, active sampling / penalty / return-sequence parameters, validated by check_sample): the search runs over
 // B * nrs entries of nb rows each, the rows of one clip (nrs * nb) sharing its visual K/V; the persistent kernel is not used.
+// P > 0: batch['prefix'] (model.py:432-437), P prompt tokens per clip already in prefix_dev (upload_prefix).  One teacher-
+// forced pass writes the K/V of the first P - 1 of them (every clip's visual K/V read once for the whole prompt), the K/V are
+// copied into the decode slots of all the clip's rows, and the search starts at t0 = P - 1 with the prompt as its history:
+// max_steps - P steps, saved logits [max_steps - P][rows][ld].  P = 0: no prompt (the search starts from SOS at t = 0).
 int run_decode(gitb200_ctx* c, const gitb200_search_params& sp, int32_t* tokens_out, float* logprobs_out, float* logits_out,
-               cudaStream_t s, const gitb200_sample_params* smp = nullptr) {
+               cudaStream_t s, const gitb200_sample_params* smp = nullptr, int P = 0) {
   const gitb200_config& k = c->cfg;
   const int nrs = smp ? smp->num_return_sequences : 1;
   const int B = c->cur_clips, nb = sp.beam_size, entries = B * nrs, rows = entries * nb;
@@ -852,19 +864,51 @@ int run_decode(gitb200_ctx* c, const gitb200_search_params& sp, int32_t* tokens_
     ss.top_p = smp->top_p; ss.temperature = smp->temperature; ss.rp = smp->repetition_penalty; ss.seed = c->seed_dev.p;
   }
   if (!c->visual_pass_done) TRY(run_visual_pass(c, false, nullptr, 0, s));
-  TRY(ensure_text(c, rows, rows, sp.max_steps));
+  const int steps = sp.max_steps - 1;        // model.py:518: while cur_len < max_length, cur_len = t + 1
+  const int t0 = P > 0 ? P - 1 : 0;          // first step: cur_len = len(input_ids)
+  const int Lp = t0 < steps ? t0 : 0;        // prompt tokens through the prefill (none when no step runs)
+  const int H = k.hidden;
+  const size_t kv_stride = (size_t)Lp * B * 2 * H;
+  TRY(ensure_text(c, rows > B * Lp ? rows : B * Lp, rows, sp.max_steps));
   if (!logits_out) ENSURE(c, c->logits, (size_t)rows * c->vocab_pad);
+  if (Lp > 0) {
+    ENSURE(c, c->pos_arr, (size_t)B * Lp);
+    ENSURE(c, c->ntext_arr, (size_t)B * Lp);
+    ENSURE(c, c->prefix_kv, kv_stride * k.dec_layers);
+  }
+  // search state init; with a prompt also its prefill and the fan-out of its K/V
+  auto start = [&]() -> int {
+    if (P == 0) {
+      CUDA_OK(c, search_init(st, k.sos, s));
+      return 0;
+    }
+    if (Lp > 0) {
+      CUDA_OK(c, fill_positions(c->pos_arr.p, c->ntext_arr.p, B * Lp, Lp, s));
+      TextPass tp;
+      tp.n_clips = B; tp.rows_per_clip = Lp; tp.max_len = Lp;
+      tp.tokens = c->prefix_dev.p + (size_t)B * P; tp.positions = c->pos_arr.p; tp.pos_const = 0;
+      tp.n_text = c->ntext_arr.p; tp.n_text_const = 0; tp.anc = nullptr;
+      tp.slot_div = Lp; tp.n_slots = B; tp.slot_is_clip = 1;
+      tp.logits = nullptr; tp.hidden_out = nullptr;
+      tp.kv_plane = c->prefix_kv.p; tp.kv_plane_stride = kv_stride;
+      TRY(run_text_pass(c, tp, s));
+      for (int l = 0; l < k.dec_layers; ++l)
+        CUDA_OK(c, fanout_prefix_kv(c->prefix_kv.p + (size_t)l * kv_stride, c->txt_kv[l].p, Lp, B, nrs * nb, 2 * H, s));
+    }
+    CUDA_OK(c, search_init_prefix(st, c->prefix_dev.p, P, nrs * nb, s));
+    return 0;
+  };
   // Latency mode: ONE clip (rows = its beams <= 4).  The whole step loop -- embedding, decoder layers, vocabulary head and
   // search step of every step -- runs as one persistent cooperative kernel whose phases are separated by grid barriers
   // instead of kernel boundaries (decode_mega.cu; bit-identical to the launch sequence below, which remains the path for
   // everything else and for devices that cannot keep the grid resident).  It leaves its loop itself once the clip is done.
   if (c->persistent_decode && !smp && B == 1 && rows <= 4 && logits_out == nullptr && k.hidden == 768 && k.dec_layers <= MEGA_MAX_LAYERS &&
-      !gemm_profile_enabled()) {
+      t0 < steps && !gemm_profile_enabled()) {
     MegaArgs m;
     memset(&m, 0, sizeof(m));
     m.n_layers = k.dec_layers; m.rows = rows; m.hidden = k.hidden; m.heads = k.dec_heads; m.ffn = k.ffn; m.Nv = c->cur_nv;
     decode_mega_attention_geometry(rows, k.dec_heads, c->cur_nv, sp.max_steps, &m.splits, &m.kcap);
-    m.vocab_pad = c->vocab_pad; m.steps = sp.max_steps - 1;
+    m.vocab_pad = c->vocab_pad; m.steps = steps; m.first_step = t0;
     m.words = c->words_f32; m.pos_table = c->pos_f32; m.lne_g = c->lne_g; m.lne_b = c->lne_b;
     m.embed_eps = k.embed_ln_eps; m.ln_eps = k.bert_ln_eps;
     m.scale_log2 = (1.0f / sqrtf((float)(k.hidden / k.dec_heads))) * 1.4426950408889634f;
@@ -872,6 +916,7 @@ int run_decode(gitb200_ctx* c, const gitb200_search_params& sp, int32_t* tokens_
     m.logits = c->logits.p; m.logits_step_stride = 0;
     m.st = st;
     if (decode_mega_supported(m)) {
+      TRY(start());  // first: the prompt's prefill may grow the workspaces whose addresses m takes below
       if (m.splits > 1) ENSURE(c, c->partial, text_attention_workspace_floats(rows, k.dec_heads, m.splits));
       ENSURE(c, c->mega_bar, 32 + 2 * 128);  // [0]: barrier counter; [32, 160): candidate scores; [160, 288): candidate ids
       for (int l = 0; l < k.dec_layers; ++l) {
@@ -885,10 +930,9 @@ int run_decode(gitb200_ctx* c, const gitb200_search_params& sp, int32_t* tokens_
       m.trace = c->mega_trace_on ? c->mega_trace.p : nullptr;
       m.tq = c->tq.p; m.ta = c->ta.p; m.tb = c->tb.p; m.tf = c->tf.p; m.partial = c->partial.p; m.barrier = c->mega_bar.p; m.attn_cnt = reinterpret_cast<int*>(c->mega_bar.p + 8);
       m.cand_score = reinterpret_cast<float*>(c->mega_bar.p + 32); m.cand_idx = reinterpret_cast<int*>(c->mega_bar.p + 160);
-      CUDA_OK(c, search_init(st, k.sos, s));
       const cudaError_t e = decode_mega(m, s);
       if (e == cudaSuccess) {
-        c->last_decode_steps = sp.max_steps - 1;
+        c->last_decode_steps = steps - t0;
         CUDA_OK(c, search_finalize(st, tokens_out, logprobs_out, s));
         return 0;
       }
@@ -907,25 +951,29 @@ int run_decode(gitb200_ctx* c, const gitb200_search_params& sp, int32_t* tokens_
     if (poll_done && !c->h_done) CUDA_OK(c, cudaMallocHost(&c->h_done, sizeof(int)));
   }
   c->last_decode_steps = 0;
-  const int steps = sp.max_steps - 1;  // model.py:518: while cur_len < max_length, cur_len = t + 1
+  if (t0 >= steps) {  // a prompt of max_steps tokens or more: the reference's loop body never runs
+    TRY(start());
+    CUDA_OK(c, search_finalize(st, tokens_out, logprobs_out, s));
+    return 0;
+  }
   // The loop runs in segments of `early_exit_every` steps (all steps when polling is off).  A segment touches only
   // context-owned buffers, so it is captured into a CUDA graph on its second occurrence and replayed from then on; the
   // poll of the finished-clip count sits between segments.  Saved logits go to a caller buffer: its address is part of the
   // graph key (a caller that hands in the same buffer again -- torch's caching allocator does -- replays; another buffer is
   // another graph, and the cache is bounded).
-  const int seg = (poll_done && c->early_exit_every < steps) ? c->early_exit_every : steps;
+  const int seg = (poll_done && c->early_exit_every < steps - t0) ? c->early_exit_every : steps - t0;
   const bool graphable = c->graph_segments && B > c->graph_max_clips;
-  for (int t0 = 0; t0 < steps; t0 += seg) {
-    const int n = steps - t0 < seg ? steps - t0 : seg;
+  for (int ts = t0; ts < steps; ts += seg) {
+    const int n = steps - ts < seg ? steps - ts : seg;
     gitb200_ctx::GraphKey key;
-    key.kind = 5; key.i0 = B; key.i1 = t0; key.i2 = n; key.i3 = c->cur_nv; key.sp = sp; key.p0 = logits_out;
+    key.kind = 5; key.i0 = B; key.i1 = ts; key.i2 = n; key.i3 = c->cur_nv; key.i4 = P; key.sp = sp; key.p0 = logits_out;
     if (smp) {
       key.smp = *smp;
       key.smp.seed = 0;
     }
     const int r = run_graphed(c, key, s, graphable, [&]() -> int {
-      if (t0 == 0) CUDA_OK(c, search_init(st, k.sos, s));
-      for (int t = t0; t < t0 + n; ++t) {
+      if (ts == t0) TRY(start());
+      for (int t = ts; t < ts + n; ++t) {
         const int parity = t & 1;
         TextPass tp;
         tp.n_clips = B; tp.rows_per_clip = nrs * nb; tp.max_len = sp.max_steps;
@@ -933,7 +981,7 @@ int run_decode(gitb200_ctx* c, const gitb200_search_params& sp, int32_t* tokens_
         tp.n_text = nullptr; tp.n_text_const = t + 1;
         tp.anc = sp.reorder_cache ? (parity ? st.anc_tmp : st.anc) : nullptr;
         tp.slot_div = 1; tp.n_slots = rows; tp.slot_is_clip = 0;
-        tp.logits = logits_out ? logits_out + (size_t)t * rows * c->vocab_pad : c->logits.p;
+        tp.logits = logits_out ? logits_out + (size_t)(t - t0) * rows * c->vocab_pad : c->logits.p;
         tp.hidden_out = nullptr;
         TRY(run_text_pass(c, tp, s));
         if (ext_step)
@@ -944,8 +992,8 @@ int run_decode(gitb200_ctx* c, const gitb200_search_params& sp, int32_t* tokens_
       return 0;
     });
     if (r != 0 && r != 1) return r;
-    c->last_decode_steps = t0 + n;
-    if (poll_done && t0 + n < steps) {
+    c->last_decode_steps = ts + n - t0;
+    if (poll_done && ts + n < steps) {
       CUDA_OK(c, cudaMemcpyAsync(c->h_done, st.done_count, sizeof(int), cudaMemcpyDeviceToHost, s));
       CUDA_OK(c, cudaStreamSynchronize(s));
       if (*c->h_done >= entries) break;
@@ -965,6 +1013,7 @@ void free_workspaces(gitb200_ctx* c) {
   fr(c->ibuf); fr(c->dbuf); fr(c->fbuf); fr(c->pos_arr); fr(c->ntext_arr); fr(c->tok_arr); fr(c->stage[0]); fr(c->stage[1]); fr(c->stage_u8[0]); fr(c->stage_u8[1]);
   fr(c->out_tok); fr(c->out_lp); fr(c->stats_a); fr(c->stats_b); fr(c->ring);
   fr(c->pool); fr(c->pool_rows); fr(c->pool_oldest); fr(c->seed_dev);
+  fr(c->prefix_dev); fr(c->prefix_kv);
 }
 
 // second workspace set that shares this context's (read-only) weights
@@ -1473,39 +1522,41 @@ int gitb200_decode(gitb200_ctx* c, const gitb200_search_params* sp, int32_t* tok
 }
 
 static int caption_eager(gitb200_ctx* c, const float* frames, int n_clips, int n_frames, const gitb200_search_params* sp,
-                         int32_t* tokens, float* logprobs, float* logits, void* stream, const gitb200_sample_params* smp) {
+                         int32_t* tokens, float* logprobs, float* logits, void* stream, const gitb200_sample_params* smp, int P) {
   int r = gitb200_encode(c, frames, n_clips, n_frames, nullptr, stream);
   if (r) return r;
-  if (smp) return run_decode(c, *sp, tokens, logprobs, logits, caller_stream(c, stream), smp);
+  if (smp || P > 0) return run_decode(c, *sp, tokens, logprobs, logits, caller_stream(c, stream), smp, P);
   return gitb200_decode(c, sp, tokens, logprobs, logits, stream);
 }
 
-// gitb200_caption (smp == nullptr) and gitb200_caption_ext with active sampling parameters (the seed already in seed_dev)
+// gitb200_caption (smp == nullptr) and gitb200_caption_ext with active sampling parameters (the seed already in seed_dev);
+// P > 0: gitb200_caption_prefix (the prompt already in prefix_dev, see run_decode)
 static int caption_impl(gitb200_ctx* c, const float* frames, int n_clips, int n_frames, const gitb200_search_params* sp,
-                        const gitb200_sample_params* smp, int32_t* tokens, float* logprobs, float* logits, void* stream) {
+                        const gitb200_sample_params* smp, int32_t* tokens, float* logprobs, float* logits, void* stream, int P = 0) {
   // Latency mode: a small batch is launch-bound (~850 kernels per caption), so the second call with the same
   // buffers / shapes on a capturable stream is recorded into a CUDA graph and later calls replay it.
   cudaStream_t s = caller_stream(c, stream);
   if (n_clips > 0 && n_clips <= c->graph_max_clips && frames && tokens && logprobs && c->finalized) {
     gitb200_ctx::GraphKey key;
     key.kind = 0; key.p0 = frames; key.p1 = tokens; key.p2 = logprobs; key.i0 = n_clips; key.i1 = n_frames;
-    key.i2 = logits != nullptr; key.sp = *sp;
+    key.i2 = logits != nullptr; key.i3 = P; key.sp = *sp;
     if (smp) {
       key.smp = *smp;
       key.smp.seed = 0;
     }
     CUDA_OK(c, cudaSetDevice(c->device));
-    const int r = run_graphed(c, key, s, logits == nullptr, [&]() { return caption_eager(c, frames, n_clips, n_frames, sp, tokens, logprobs, logits, stream, smp); });
+    const int r = run_graphed(c, key, s, logits == nullptr, [&]() { return caption_eager(c, frames, n_clips, n_frames, sp, tokens, logprobs, logits, stream, smp, P); });
     if (r == 1) {  // replayed: host-side state the eager path would have left behind
       const int F = (c->cfg.num_image_with_embedding > 0 && n_frames > c->cfg.num_image_with_embedding) ? c->cfg.num_image_with_embedding : n_frames;
       c->cur_clips = n_clips; c->cur_nv = F * c->T; c->visual_pass_done = true; c->visual_pass_full = 0; c->step_rows_per_clip = 0;
-      c->last_decode_steps = sp->max_steps - 1;
+      const int first = P > 0 ? P : 1;  // the search's first cur_len
+      c->last_decode_steps = sp->max_steps > first ? sp->max_steps - first : 0;
       return GITB200_OK;
     }
     return r;
   }
   if (logits == nullptr && frames && tokens && logprobs && c->finalized && n_clips > 0 && n_frames > 0) {
-    const int chunk = smp ? 0 : pipeline_chunk_for(c, n_clips);
+    const int chunk = (smp || P > 0) ? 0 : pipeline_chunk_for(c, n_clips);
     if (chunk > 0) {
       CUDA_OK(c, cudaSetDevice(c->device));
       return caption_pipelined(c, frames, n_clips, n_frames, *sp, tokens, logprobs, s, chunk);
@@ -1535,7 +1586,7 @@ static int caption_impl(gitb200_ctx* c, const float* frames, int n_clips, int n_
       } else if (r != 0) {
         return r;
       }
-      TRY(run_decode(c, *sp, tokens, logprobs, nullptr, gs, smp));
+      TRY(run_decode(c, *sp, tokens, logprobs, nullptr, gs, smp, P));
       if (forked) {
         CUDA_OK(c, cudaEventRecord(c->ev_gjoin, gs));
         CUDA_OK(c, cudaStreamWaitEvent(s, c->ev_gjoin, 0));
@@ -1543,7 +1594,7 @@ static int caption_impl(gitb200_ctx* c, const float* frames, int n_clips, int n_
       return GITB200_OK;
     }
   }
-  return caption_eager(c, frames, n_clips, n_frames, sp, tokens, logprobs, logits, stream, smp);
+  return caption_eager(c, frames, n_clips, n_frames, sp, tokens, logprobs, logits, stream, smp, P);
 }
 
 int gitb200_caption(gitb200_ctx* c, const float* frames, int n_clips, int n_frames, const gitb200_search_params* sp,
@@ -1596,6 +1647,36 @@ int upload_seed(gitb200_ctx* c, uint64_t seed, cudaStream_t s) {
   return 0;
 }
 
+// Every rejection of a prompt (batch['prefix']), on the host before anything is enqueued.  max_positions 0: not checked.
+int check_prefix(gitb200_ctx* c, const int32_t* prefix, int prefix_rows, int P, int n_clips, int vocab, int max_positions) {
+  if (P < 1) return fail(c, GITB200_ERR_INVALID, "prefix length P must be >= 1 (got %d)", P);
+  if (!prefix) return fail(c, GITB200_ERR_INVALID, "prefix is NULL");
+  if (prefix_rows != 1 && prefix_rows != n_clips)
+    return fail(c, GITB200_ERR_INVALID, "prefix_rows must be 1 or the %d clips (got %d)", n_clips, prefix_rows);
+  if (max_positions > 0 && P > max_positions)
+    return fail(c, GITB200_ERR_INVALID, "prefix length P %d exceeds the %d text positions", P, max_positions);
+  for (long long i = 0; i < (long long)prefix_rows * P; ++i)
+    if (prefix[i] < 0 || prefix[i] >= vocab)
+      return fail(c, GITB200_ERR_INVALID, "prefix token %d at [%lld, %lld] lies outside the vocabulary [0, %d)", prefix[i], i / P,
+                  i % P, vocab);
+  return 0;
+}
+
+// prefix_dev = [n_clips][P] every clip's prompt (a shared prompt repeated), then [n_clips][P - 1] the prefill's token rows.  The
+// prompt sits at a fixed device address, so a captured graph replays for any prompt of the same length.
+int upload_prefix(gitb200_ctx* c, const int32_t* prefix, int prefix_rows, int P, int n_clips, cudaStream_t s) {
+  std::vector<int> h((size_t)n_clips * (2 * P - 1));
+  int* q = h.data();
+  for (int b = 0; b < n_clips; ++b, q += P) memcpy(q, prefix + (size_t)(prefix_rows == 1 ? 0 : b) * P, (size_t)P * sizeof(int));
+  for (int b = 0; b < n_clips; ++b, q += P - 1) memcpy(q, h.data() + (size_t)b * P, (size_t)(P - 1) * sizeof(int));
+  ENSURE(c, c->prefix_dev, h.size());
+  // (a pageable source: the copy is staged before cudaMemcpyAsync returns, so the vector may go out of scope)
+  CUDA_OK(c, cudaMemcpyAsync(c->prefix_dev.p, h.data(), h.size() * sizeof(int), cudaMemcpyHostToDevice, s));
+  return 0;
+}
+
+const gitb200_sample_params kDefaultSample = {0, 0, 1.f, 1.f, 1.f, 1, 0};
+
 }  // namespace
 
 int gitb200_decode_ext(gitb200_ctx* c, const gitb200_search_params* sp, const gitb200_sample_params* smp, int32_t* tokens,
@@ -1622,6 +1703,41 @@ int gitb200_caption_ext(gitb200_ctx* c, const float* frames, int n_clips, int n_
   CUDA_OK(c, cudaSetDevice(c->device));
   TRY(upload_seed(c, smp->seed, caller_stream(c, stream)));
   return caption_impl(c, frames, n_clips, n_frames, sp, smp, tokens, logprobs, logits, stream);
+}
+
+int gitb200_decode_prefix(gitb200_ctx* c, const gitb200_search_params* sp, const gitb200_sample_params* smp,
+                          const int32_t* prefix_host, int prefix_rows, int P, int32_t* tokens, float* logprobs, float* logits,
+                          void* stream) {
+  if (!c || !sp) return fail(c, GITB200_ERR_INVALID, "bad decode_prefix argument");
+  const gitb200_sample_params& x = smp ? *smp : kDefaultSample;
+  TRY(check_sample(c, *sp, x, c->cfg.vocab, c->cur_clips, c->cfg.max_positions, true));
+  if (!tokens || !logprobs) return fail(c, GITB200_ERR_INVALID, "bad decode_prefix argument");
+  if (!c->finalized) return fail(c, GITB200_ERR_STATE, "call gitb200_finalize_weights first");
+  if (c->cur_clips <= 0) return fail(c, GITB200_ERR_STATE, "no visual features: call gitb200_encode or gitb200_set_visual_features first");
+  TRY(check_prefix(c, prefix_host, prefix_rows, P, c->cur_clips, c->cfg.vocab, c->cfg.max_positions));
+  CUDA_OK(c, cudaSetDevice(c->device));
+  cudaStream_t s = caller_stream(c, stream);
+  const bool active = sample_active(x);
+  if (active) TRY(upload_seed(c, x.seed, s));
+  TRY(upload_prefix(c, prefix_host, prefix_rows, P, c->cur_clips, s));
+  return run_decode(c, *sp, tokens, logprobs, logits, s, active ? &x : nullptr, P);
+}
+
+int gitb200_caption_prefix(gitb200_ctx* c, const float* frames, int n_clips, int n_frames, const gitb200_search_params* sp,
+                           const gitb200_sample_params* smp, const int32_t* prefix_host, int prefix_rows, int P, int32_t* tokens,
+                           float* logprobs, float* logits, void* stream) {
+  if (!c || !sp) return fail(c, GITB200_ERR_INVALID, "bad caption_prefix argument");
+  const gitb200_sample_params& x = smp ? *smp : kDefaultSample;
+  TRY(check_sample(c, *sp, x, c->cfg.vocab, n_clips, c->cfg.max_positions, true));
+  if (!frames || !tokens || !logprobs || n_clips < 1 || n_frames < 1) return fail(c, GITB200_ERR_INVALID, "bad caption_prefix argument");
+  if (!c->finalized) return fail(c, GITB200_ERR_STATE, "call gitb200_finalize_weights first");
+  TRY(check_prefix(c, prefix_host, prefix_rows, P, n_clips, c->cfg.vocab, c->cfg.max_positions));
+  CUDA_OK(c, cudaSetDevice(c->device));
+  cudaStream_t s = caller_stream(c, stream);
+  const bool active = sample_active(x);
+  if (active) TRY(upload_seed(c, x.seed, s));
+  TRY(upload_prefix(c, prefix_host, prefix_rows, P, n_clips, s));
+  return caption_impl(c, frames, n_clips, n_frames, sp, active ? &x : nullptr, tokens, logprobs, logits, stream, P);
 }
 
 int gitb200_stream_reset(gitb200_ctx* c) {
@@ -2273,6 +2389,55 @@ int gitb200_op_search_ext(const float* logits, int ld, int vocab, int n_clips, i
   if (tmp.dbuf.p) cudaFree(tmp.dbuf.p);
   if (tmp.fbuf.p) cudaFree(tmp.fbuf.p);
   if (tmp.seed_dev.p) cudaFree(tmp.seed_dev.p);
+  if (r) return fail(nullptr, r, "%s", tmp.err.c_str());
+  if (e != cudaSuccess) return fail(nullptr, GITB200_ERR_CUDA, "search: %s", cudaGetErrorString(e));
+  return GITB200_OK;
+}
+
+int gitb200_op_search_prefix(const float* logits, int ld, int vocab, int n_clips, int eos, const gitb200_search_params* sp,
+                             const gitb200_sample_params* smp, const int32_t* prefix_host, int prefix_rows, int P, int32_t* tokens,
+                             float* logprobs, void* stream) {
+  if (!sp) return fail(nullptr, GITB200_ERR_INVALID, "bad op_search_prefix argument");
+  const gitb200_sample_params& x = smp ? *smp : kDefaultSample;
+  {
+    const int r = check_sample(nullptr, *sp, x, vocab, n_clips, 0, false);
+    if (r) return r;
+  }
+  const int steps = sp->max_steps - (P > 1 ? P : 1);  // search steps: scores [steps, rows, ld]
+  if ((!logits && steps > 0) || !tokens || !logprobs || n_clips < 1 || vocab < 1 || ld < vocab)
+    return fail(nullptr, GITB200_ERR_INVALID, "bad op_search_prefix argument");
+  {
+    const int r = check_prefix(nullptr, prefix_host, prefix_rows, P, n_clips, vocab, 0);
+    if (r) return r;
+  }
+  gitb200_ctx tmp;  // scratch owner for the search buffers
+  cudaGetDevice(&tmp.device);
+  const int nrs = x.num_return_sequences, entries = n_clips * nrs, rows = entries * sp->beam_size;
+  SearchState st;
+  int r = make_search_state(&tmp, entries, vocab, ld, 0, eos, *sp, &st);
+  cudaStream_t s = (cudaStream_t)stream;
+  cudaError_t e = cudaSuccess;
+  const bool active = sample_active(x);
+  if (!r && active) r = upload_seed(&tmp, x.seed, s);
+  if (!r) r = upload_prefix(&tmp, prefix_host, prefix_rows, P, n_clips, s);
+  if (!r) {
+    SampleState ss{};
+    ss.do_sample = x.do_sample; ss.top_k = x.top_k; ss.nrs = nrs; ss.pnb = sp->per_node_beam_size;
+    ss.top_p = x.top_p; ss.temperature = x.temperature; ss.rp = x.repetition_penalty; ss.seed = tmp.seed_dev.p;
+    const bool ext_step = x.do_sample || x.repetition_penalty != 1.f;
+    e = search_init_prefix(st, tmp.prefix_dev.p, P, nrs * sp->beam_size, s);
+    for (int t = P - 1; e == cudaSuccess && t + 1 < sp->max_steps; ++t) {
+      const float* lt = logits + (size_t)(t - (P - 1)) * rows * ld;
+      e = ext_step ? sample_step(st, ss, lt, t + 1, t & 1, t, s) : search_step(st, lt, t + 1, t & 1, s);
+    }
+    if (e == cudaSuccess) e = search_finalize(st, tokens, logprobs, s);
+    if (e == cudaSuccess) e = cudaStreamSynchronize(s);
+  }
+  if (tmp.ibuf.p) cudaFree(tmp.ibuf.p);
+  if (tmp.dbuf.p) cudaFree(tmp.dbuf.p);
+  if (tmp.fbuf.p) cudaFree(tmp.fbuf.p);
+  if (tmp.seed_dev.p) cudaFree(tmp.seed_dev.p);
+  if (tmp.prefix_dev.p) cudaFree(tmp.prefix_dev.p);
   if (r) return fail(nullptr, r, "%s", tmp.err.c_str());
   if (e != cudaSuccess) return fail(nullptr, GITB200_ERR_CUDA, "search: %s", cudaGetErrorString(e));
   return GITB200_OK;

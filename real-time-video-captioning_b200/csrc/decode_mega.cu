@@ -350,7 +350,7 @@ __device__ __forceinline__ void mega_body(const MegaArgs& a, const Smem& sm, int
   const int vw = wid & 7, cg = wid >> 3;                                             // fc2: K-slice warp, column group
   preload_qkv(a, 0, gw, lane, wA, bA);
 
-  for (int t = 0; t < a.steps; ++t) {
+  for (int t = a.first_step; t < a.steps; ++t) {
     const int parity = t & 1;
     // ------------------------------------------------------------------ embedding (every CTA, its own copy)
     if (wid < M) {
@@ -629,7 +629,8 @@ void decode_mega_attention_geometry(int rows, int heads, int Nv, int max_text, i
 bool decode_mega_supported(const MegaArgs& a) {
   int af = 0;
   if (a.rows < 1 || a.rows > 4 || a.hidden != H || a.heads * text_attn_dev::HD != H || a.ffn % 256 != 0 || a.ffn < 2048 || a.ffn > 4096 ||
-      a.n_layers < 1 || a.n_layers > MEGA_MAX_LAYERS || a.vocab_pad % 4 != 0 || a.st.n_clips != 1 || a.st.nb != a.rows)
+      a.n_layers < 1 || a.n_layers > MEGA_MAX_LAYERS || a.vocab_pad % 4 != 0 || a.st.n_clips != 1 || a.st.nb != a.rows ||
+      a.first_step < 0 || a.first_step >= a.steps)
     return false;
   return mega_smem_bytes(a, &af) <= 200 * 1024;
 }

@@ -321,7 +321,32 @@ __global__ void fill_positions_kernel(int* pos, int* n_text, int rows, int L) {
   }
 }
 
+// Prompt K/V fan-out: dst[(p * rows + r) * width + c] = src[(p * n_clips + r / rows_per_clip) * width + c] for text positions
+// p < n_pos; 16-byte chunks (width % 8 == 0).  Every decode row gets its clip's prompt K/V in its OWN slot, so that both ways
+// of following the beams (ancestor table or not) read the prompt wherever they look.
+__global__ void fanout_prefix_kv_kernel(const bf16* __restrict__ src, bf16* __restrict__ dst, int n_pos, int n_clips,
+                                        int rows_per_clip, int width) {
+  const int w8 = width / 8, rows = n_clips * rows_per_clip;
+  const size_t total = (size_t)n_pos * rows * w8;
+  for (size_t i = blockIdx.x * (size_t)blockDim.x + threadIdx.x; i < total; i += (size_t)gridDim.x * blockDim.x) {
+    const int c = (int)(i % w8);
+    const size_t pr = i / w8;
+    const int r = (int)(pr % rows), p = (int)(pr / rows);
+    reinterpret_cast<uint4*>(dst)[i] = __ldg(reinterpret_cast<const uint4*>(src) + ((size_t)p * n_clips + r / rows_per_clip) * w8 + c);
+  }
+}
+
 }  // namespace
+
+cudaError_t fanout_prefix_kv(const bf16* src, bf16* dst, int n_pos, int n_clips, int rows_per_clip, int width, cudaStream_t stream) {
+  if (width % 8 != 0 || n_clips < 0 || rows_per_clip < 1) return cudaErrorInvalidValue;
+  const size_t total = (size_t)n_pos * n_clips * rows_per_clip * (width / 8);
+  if (n_pos <= 0 || total == 0) return cudaSuccess;
+  const size_t want = (total + 255) / 256;
+  fanout_prefix_kv_kernel<<<(int)(want < 148 * 16 ? want : 148 * 16), 256, 0, stream>>>(src, dst, n_pos, n_clips, rows_per_clip, width);
+  note_launch();
+  return cudaGetLastError();
+}
 
 cudaError_t assemble_window(const bf16* ring, int first, int cap, int n, int T, int W, const float* temporal, bf16* vf,
                             cudaStream_t stream) {

@@ -180,6 +180,11 @@ struct SearchState {
 // (0: tokens/anc are read and *_tmp written; 1: the reverse).  The caller flips it after every step.
 cudaError_t search_step(const SearchState& s, const float* logits, int cur_len, int parity, cudaStream_t stream);
 cudaError_t search_init(const SearchState& s, int sos, cudaStream_t stream);
+// search_init with a prompt of P tokens (model.py:432-437, batch['prefix']): prompt is device int [clips][P] and row r belongs
+// to clip r / rows_per_clip; its history is that clip's P tokens and it feeds the last of them to the first step.
+// The history goes to the token buffer that the first step (t0 = P - 1) reads: tokens for even t0, tokens_tmp for odd.
+// P >= max_len: no step runs and the prompt (which does not fit) is not written.
+cudaError_t search_init_prefix(const SearchState& s, const int* prompt, int P, int rows_per_clip, cudaStream_t stream);
 // decoded [n_clips, n_keep, max_len] (eos padded), logprobs [n_clips, n_keep]
 cudaError_t search_finalize(const SearchState& s, int* decoded, float* logprobs, cudaStream_t stream);
 // Extended search step (model.py:524-554): repetition penalty, and with do_sample temperature, top-k / top-p filtering
@@ -207,11 +212,12 @@ struct MegaLayer {
 struct MegaArgs {
   MegaLayer layer[MEGA_MAX_LAYERS];
   int n_layers, rows, hidden, heads, ffn, Nv, splits, kcap, vocab_pad, steps;
+  int first_step;                                  // the loop runs t = first_step .. steps - 1 (a prompt of P tokens: P - 1)
   const float *words, *pos_table, *lne_g, *lne_b;  // fp32 embedding tables, embedding LayerNorm
   float embed_eps, ln_eps, scale_log2;
   const bf16* w_vocab;   // [vocab_pad, H]
   const float* b_vocab;  // [vocab_pad]
-  float* logits;         // [steps or 1][rows, vocab_pad]
+  float* logits;         // [steps or 1][rows, vocab_pad] (step t's logits at logits + t * logits_step_stride)
   long long logits_step_stride;  // floats between the logits of consecutive steps (0: one buffer reused)
   bf16 *tq, *ta, *tb, *tf;  // scratch rows: [rows, 3H], [rows, H], [rows, H], [rows, ffn]
   float* partial;           // key-split partials of the attention
@@ -226,6 +232,9 @@ bool decode_mega_supported(const MegaArgs& a);
 void decode_mega_attention_geometry(int rows, int heads, int Nv, int max_text, int* splits, int* kcap);
 cudaError_t decode_mega(const MegaArgs& a, cudaStream_t stream);
 
+// Prompt K/V into the decode plane: dst[(p * n_clips * rows_per_clip + r) * width + c] = src[(p * n_clips + r / rows_per_clip) *
+// width + c] for p < n_pos (src: the teacher-forced plane [n_pos][n_clips][width]; width % 8 == 0)
+cudaError_t fanout_prefix_kv(const bf16* src, bf16* dst, int n_pos, int n_clips, int rows_per_clip, int width, cudaStream_t stream);
 // pos[r] = r % L, n_text[r] = r % L + 1 (teacher-forced text rows)
 cudaError_t fill_positions(int* pos, int* n_text, int rows, int L, cudaStream_t stream);
 // Step-wise decoding cache re-index: out[r][s] = in ? in[beam_idx[r]][s] : beam_idx[r] for s < pos; out[r][pos] = beam_idx[r].

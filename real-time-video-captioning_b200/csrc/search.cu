@@ -397,6 +397,31 @@ __global__ void search_init_kernel(SearchState st, int sos) {
   }
 }
 
+// search_init_kernel with the prompt as every row's history (model.py:432-437, :481-495); see search_init_prefix
+__global__ void search_init_prefix_kernel(SearchState st, const int* __restrict__ prompt, int P, int rows_per_clip) {
+  const int row = blockIdx.x * blockDim.x + threadIdx.x;
+  const int n_rows = st.n_clips * st.nb;
+  if (row < n_rows) {
+    const int* src = prompt + (size_t)(row / rows_per_clip) * P;
+    if (P < st.max_len) {
+      int* dst = (((P - 1) & 1) ? st.tokens_tmp : st.tokens) + (size_t)row * st.max_len;
+      for (int t = 0; t < P; ++t) dst[t] = src[t];
+    }
+    st.cur_tok[row] = src[P - 1];
+    st.beam_scores[row] = (row % st.nb == 0) ? 0.f : -1e9f;  // model.py:508-510
+    for (int t = 0; t < st.max_len; ++t) {
+      st.anc[(size_t)row * st.max_len + t] = row;
+      st.anc_tmp[(size_t)row * st.max_len + t] = row;
+    }
+  }
+  if (row == 0) *st.done_count = 0;
+  if (row < st.n_clips) {
+    st.done[row] = 0;
+    st.hyp_count[row] = 0;
+    st.worst[row] = 1e9;
+  }
+}
+
 // model.py:653-677: best n_keep hypotheses per clip, eos padded, + one eos appended
 __global__ void search_finalize_kernel(SearchState st, int* decoded, float* logprobs) {
   const int clip = blockIdx.x * blockDim.x + threadIdx.x;
@@ -445,6 +470,16 @@ cudaError_t search_init(const SearchState& s, int sos, cudaStream_t stream) {
   if (n <= 0) return cudaSuccess;
   if (s.nb > MAX_NB || s.cand > MAX_CAND || s.n_keep + 1 > MAX_CAND) return cudaErrorInvalidValue;
   search_init_kernel<<<(n + 127) / 128, 128, 0, stream>>>(s, sos);
+  note_launch();
+  return cudaGetLastError();
+}
+
+cudaError_t search_init_prefix(const SearchState& s, const int* prompt, int P, int rows_per_clip, cudaStream_t stream) {
+  const int n = s.n_clips * s.nb;
+  if (n <= 0) return cudaSuccess;
+  if (s.nb > MAX_NB || s.cand > MAX_CAND || s.n_keep + 1 > MAX_CAND || prompt == nullptr || P < 1 || rows_per_clip < 1)
+    return cudaErrorInvalidValue;
+  search_init_prefix_kernel<<<(n + 127) / 128, 128, 0, stream>>>(s, prompt, P, rows_per_clip);
   note_launch();
   return cudaGetLastError();
 }

@@ -68,6 +68,16 @@ def _ptr(t: Optional[torch.Tensor]):
     return None if t is None else ctypes.c_void_p(t.data_ptr())
 
 
+def _prefix_host(prefix) -> torch.Tensor:
+    """batch['prefix'] (model.py:432-437) as the C side takes it: int32 [1 or B, P] on the host, contiguous.  The token values
+    are checked by the library (before anything is enqueued)."""
+    if not isinstance(prefix, torch.Tensor) or prefix.dim() != 2 or prefix.shape[1] < 1:
+        raise GitB200Error(f"prefix must be an int tensor [1 or B, P] with P >= 1 (got {getattr(prefix, 'shape', type(prefix))})")
+    if prefix.dtype.is_floating_point or prefix.dtype.is_complex or prefix.dtype == torch.bool:
+        raise GitB200Error(f"prefix must hold integer token ids (got {prefix.dtype})")
+    return prefix.detach().to(device="cpu", dtype=torch.int32).contiguous()
+
+
 class Engine:
     """One C context bound to one CUDA device."""
 
@@ -160,18 +170,31 @@ class Engine:
               "gitb200_set_visual_features")
         self._cur_nv, self._cur_clips, self._step_rows = vf.shape[1], vf.shape[0], 0
 
-    def _search_outputs(self, n_clips: int, sp: SearchConfig, sample: Optional[SampleConfig], save_logits: bool):
+    def _search_outputs(self, n_clips: int, sp: SearchConfig, sample: Optional[SampleConfig], save_logits: bool, P: int = 1):
         n = n_clips * (sample.num_return_sequences if sample is not None else 1)
         tokens = torch.empty(n, sp.num_keep_best, sp.max_steps, dtype=torch.int32, device=self.device)
         logprobs = torch.empty(n, sp.num_keep_best, dtype=torch.float32, device=self.device)
-        logits = torch.empty(sp.max_steps - 1, n * sp.beam_size, self.ld, dtype=torch.float32,
+        logits = torch.empty(max(0, sp.max_steps - P), n * sp.beam_size, self.ld, dtype=torch.float32,
                              device=self.device) if save_logits else None
         return tokens, logprobs, logits
 
-    def decode(self, n_clips: int, sp: SearchConfig, save_logits: bool = False, sample: Optional[SampleConfig] = None):
+    def decode(self, n_clips: int, sp: SearchConfig, save_logits: bool = False, sample: Optional[SampleConfig] = None,
+               prefix: Optional[torch.Tensor] = None):
         """Search on the current visual features: (tokens int32 [B, keep, max_steps], logprobs [B, keep],
         logits fp32 [max_steps-1, B*beam, ld] or None).  With ``sample``, B becomes B * num_return_sequences (row
-        i * nrs + j = sequence j of clip i) and the logits are the scores before penalty and temperature."""
+        i * nrs + j = sequence j of clip i) and the logits are the scores before penalty and temperature.
+        ``prefix`` (batch['prefix'], int [1 or B, P], host or device): the search starts from that prompt; the tokens then
+        include it (the reference's infer strips it) and the logits hold max_steps - P steps."""
+        if prefix is not None:
+            pre = _prefix_host(prefix)
+            tokens, logprobs, logits = self._search_outputs(n_clips, sp, sample, save_logits, pre.shape[1])
+            c, x = sp.to_c(), sample.to_c() if sample is not None else None
+            check(self.lib.gitb200_decode_prefix(self.h, ctypes.byref(c), ctypes.byref(x) if x is not None else None, _ptr(pre),
+                                                 pre.shape[0], pre.shape[1], _ptr(tokens), _ptr(logprobs), _ptr(logits),
+                                                 self._stream()), self.h, "gitb200_decode_prefix")
+            if logits is not None:
+                logits = logits[: self.last_decode_steps()]
+            return tokens, logprobs, logits
         tokens, logprobs, logits = self._search_outputs(n_clips, sp, sample, save_logits)
         c = sp.to_c()
         if sample is None:
@@ -185,13 +208,21 @@ class Engine:
             logits = logits[: self.last_decode_steps()]
         return tokens, logprobs, logits
 
-    def caption(self, frames: torch.Tensor, sp: SearchConfig, save_logits: bool = False, sample: Optional[SampleConfig] = None):
+    def caption(self, frames: torch.Tensor, sp: SearchConfig, save_logits: bool = False, sample: Optional[SampleConfig] = None,
+                prefix: Optional[torch.Tensor] = None):
+        """encode + decode of frames fp32 [B, F, 3, R, R]; ``sample`` and ``prefix`` as in ``decode``."""
         assert frames.is_cuda and frames.dtype == torch.float32 and frames.dim() == 5
         frames = frames.contiguous()
         B, F = frames.shape[:2]
-        tokens, logprobs, logits = self._search_outputs(B, sp, sample, save_logits)
+        pre = _prefix_host(prefix) if prefix is not None else None
+        tokens, logprobs, logits = self._search_outputs(B, sp, sample, save_logits, pre.shape[1] if pre is not None else 1)
         c = sp.to_c()
-        if sample is None:
+        if pre is not None:
+            x = sample.to_c() if sample is not None else None
+            check(self.lib.gitb200_caption_prefix(self.h, _ptr(frames), B, F, ctypes.byref(c), ctypes.byref(x) if x is not None else None,
+                                                  _ptr(pre), pre.shape[0], pre.shape[1], _ptr(tokens), _ptr(logprobs), _ptr(logits),
+                                                  self._stream()), self.h, "gitb200_caption_prefix")
+        elif sample is None:
             check(self.lib.gitb200_caption(self.h, _ptr(frames), B, F, ctypes.byref(c), _ptr(tokens), _ptr(logprobs),
                                            _ptr(logits), self._stream()), self.h, "gitb200_caption")
         else:
@@ -519,9 +550,10 @@ def op_text_attention(q: torch.Tensor, vis_kv: torch.Tensor, txt_kv, anc, n_clip
 
 
 def op_search(logits: torch.Tensor, vocab: int, n_clips: int, sos: int, eos: int, sp: SearchConfig,
-              sample: Optional[SampleConfig] = None):
+              sample: Optional[SampleConfig] = None, prefix: Optional[torch.Tensor] = None):
     """logits fp32 [max_steps-1, n_clips*beam, ld] (device) -> tokens [n_clips, keep, max_steps], logprobs.
-    With ``sample``: logits [max_steps-1, n_clips*nrs*beam, ld] -> tokens [n_clips*nrs, keep, max_steps]."""
+    With ``sample``: logits [max_steps-1, n_clips*nrs*beam, ld] -> tokens [n_clips*nrs, keep, max_steps].
+    With ``prefix`` (int [1 or n_clips, P]): the search starts from that prompt (``sos`` unused), logits [max_steps-P, ...]."""
     lib = _lib.load()
     logits = logits.contiguous()
     n = n_clips * (sample.num_return_sequences if sample is not None else 1)
@@ -529,7 +561,13 @@ def op_search(logits: torch.Tensor, vocab: int, n_clips: int, sos: int, eos: int
     logprobs = torch.empty(n, sp.num_keep_best, dtype=torch.float32, device=logits.device)
     c = sp.to_c()
     s = ctypes.c_void_p(torch.cuda.current_stream(logits.device).cuda_stream)
-    if sample is None:
+    if prefix is not None:
+        pre = _prefix_host(prefix)
+        x = sample.to_c() if sample is not None else None
+        check(lib.gitb200_op_search_prefix(_ptr(logits) if logits.numel() else None, logits.shape[-1], vocab, n_clips, eos,
+                                           ctypes.byref(c), ctypes.byref(x) if x is not None else None, _ptr(pre), pre.shape[0],
+                                           pre.shape[1], _ptr(tokens), _ptr(logprobs), s), None, "gitb200_op_search_prefix")
+    elif sample is None:
         check(lib.gitb200_op_search(_ptr(logits), logits.shape[-1], vocab, n_clips, sos, eos, ctypes.byref(c), _ptr(tokens),
                                     _ptr(logprobs), s), None, "gitb200_op_search")
     else:

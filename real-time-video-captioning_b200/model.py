@@ -535,12 +535,18 @@ class GenerativeImageTextModel(nn.Module):
 
         ``search_param['seed']`` (not a reference key) opts into the device's counter-based RNG: sampling, repetition
         penalty and num_return_sequences then run in the fused device search, reproducible for a given seed but not
-        token-identical to torch's RNG.  Without it those settings take the generic host loop, as the reference does."""
+        token-identical to torch's RNG.  Without it those settings take the generic host loop, as the reference does.
+
+        ``search_param['device_prefix'] = True`` (not a reference key) lets ``batch['prefix']`` (int [1 or B, P]) take the
+        fused device search too: one decoder pass over the prompt, then the search from cur_len = P.  The prompt's K/V come
+        from a differently shaped GEMM than the host loop's per-token steps, so results agree with it within the parity
+        tolerances, not bit for bit.  Without it a prefix takes the host loop, as before."""
         batch_size = visual_features.size(0)
         search_param = dict(search_param or {})
         seed = search_param.pop("seed", None)
+        device_prefix = bool(search_param.pop("device_prefix", False))
         eng = self.engine()
-        fused = (isinstance(self.decoder, GeneratorWithBeamSearchV2) and "prefix" not in batch
+        fused = (isinstance(self.decoder, GeneratorWithBeamSearchV2) and ("prefix" not in batch or device_prefix)
                  and visual_features_valid is None and not self._force_host_search)
         fast = (fused and not search_param.get("do_sample", False) and search_param.get("num_return_sequences", 1) == 1
                 and self.decoder.repetition_penalty == 1.0)
@@ -559,13 +565,17 @@ class GenerativeImageTextModel(nn.Module):
                 eng.set_visual_features(visual_features.to(eng.device))
                 self._vf_token = visual_features
             sc = self.decoder.search_config(search_param.get("num_keep_best", 1), self.cache_reorder == "correct")
-            if sample is None:
+            if "prefix" in batch:
+                tokens, logprobs, logits = eng.decode(batch_size, sc, save_logits=True, sample=sample, prefix=batch["prefix"])
+            elif sample is None:
                 tokens, logprobs, logits = eng.decode(batch_size, sc, save_logits=True)
             else:
                 tokens, logprobs, logits = eng.decode(batch_size, sc, save_logits=True, sample=sample)
             predicted = tokens.long()
             if sc.num_keep_best == 1:
                 predicted = predicted.squeeze(1)
+            if "prefix" in batch:  # the reference's strip, on whatever shape the search returned (keep > 1: the keep dimension)
+                predicted = predicted[:, batch["prefix"].shape[1]:]
             logits_dict = LazyLogits(logits, eng.cfg.vocab)
         else:
             if "prefix" not in batch:
