@@ -15,7 +15,7 @@ ROOT = os.path.dirname(HERE)
 OBJ_DIR = os.path.join(ROOT, "build", "obj")
 LIB_PATH = os.path.join(HERE, "libgitb200.so")
 SOURCES = ["gemm_tcgen05.cu", "gemm2_tcgen05.cu", "gemv_skinny.cu", "elementwise.cu", "attention.cu", "attention_tc.cu", "search.cu", "decode_mega.cu", "preprocess.cu", "student.cu", "student_train.cu", "api.cu"]
-HEADERS = ["common.cuh", "kernels.h", "student_internal.cuh", "search_step.cuh", "philox.cuh", "text_attention_dev.cuh", os.path.join("..", "..", "include", "gitb200.h")]
+HEADERS = ["common.cuh", "kernels.h", "student_ops.h", "student_internal.cuh", "search_step.cuh", "philox.cuh", "text_attention_dev.cuh", os.path.join("..", "..", "include", "gitb200.h")]
 NVCC_FLAGS = ["-gencode", "arch=compute_100a,code=sm_100a", "-lineinfo", "-O3", "-std=c++17", "-Xcompiler", "-fPIC",
               "-DGITB200_BUILD"]
 

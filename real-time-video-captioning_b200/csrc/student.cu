@@ -195,18 +195,19 @@ int s_ln(gitb200_student* c, const bf16* x, int ldx, int rows, const float* g, c
   S_CUDA_OK(c, cudaGetLastError());
   return 0;
 }
-// teacher-forced embedding of all L positions of every sequence (pos0 = 0)
-int s_embed(gitb200_student* c, const int* tokens, int tok_ld, int L, int rows, bf16* out, cudaStream_t s) {
-  student_embed_kernel<<<rows, 128, 0, s>>>(tokens, tok_ld, 0, L, 0, rows, c->embed, c->pe, c->cfg.d_model, c->cfg.vocab,
+// embedding of positions pos0 .. pos0 + L - 1 of every sequence (teacher forcing: pos0 = 0; cached decoding: L = 1)
+int s_embed(gitb200_student* c, const int* tokens, int tok_ld, int L, int pos0, int rows, bf16* out, cudaStream_t s) {
+  student_embed_kernel<<<rows, 128, 0, s>>>(tokens, tok_ld, pos0, L, pos0, rows, c->embed, c->pe, c->cfg.d_model, c->cfg.vocab,
                                             1.0f / sqrtf((float)c->cfg.d_model), out, c->dp);
   note_launch();
   S_CUDA_OK(c, cudaGetLastError());
   return 0;
 }
-int s_attn(gitb200_student* c, const bf16* q, int ldq, int Lq, const bf16* kv, int kv_rows, int ldkv, int k_off, int v_off, int n_keys,
-           int causal, const int* tokens, int tok_ld, int rows, bf16* out, int ldo, cudaStream_t s) {
-  student_attn_kernel<<<dim3(rows, c->cfg.n_head), 32, 0, s>>>(q, ldq, Lq, 0, kv, kv_rows, ldkv, k_off, v_off, n_keys, causal, tokens, tok_ld,
-                                                               c->cfg.pad, c->hd, 1.0f / sqrtf((float)c->hd), out, ldo);
+int s_attn(gitb200_student* c, const bf16* q, int ldq, int Lq, int pos0, const bf16* kv, int kv_rows, int ldkv, int k_off, int v_off,
+           int n_keys, int causal, const int* tokens, int tok_ld, int rows, bf16* out, int ldo, cudaStream_t s) {
+  if (n_keys < 1 || n_keys > S_MAX_KEYS) return sfail(c, GITB200_ERR_INVALID, "student attention over %d keys (1 .. %d)", n_keys, S_MAX_KEYS);
+  student_attn_kernel<<<dim3(rows, c->cfg.n_head), 32, 0, s>>>(q, ldq, Lq, pos0, kv, kv_rows, ldkv, k_off, v_off, n_keys, causal, tokens,
+                                                               tok_ld, c->cfg.pad, c->hd, 1.0f / sqrtf((float)c->hd), out, ldo);
   note_launch();
   S_CUDA_OK(c, cudaGetLastError());
   return 0;
@@ -248,18 +249,14 @@ int s_alloc(gitb200_student* c, T** p, size_t n) {
 // tokens: int [B, tok_ld] (the ids at every position up to pos0 + L - 1; used for the embedding and the padding mask).
 int run_layers(gitb200_student* c, int B, int L, int pos0, int Lmax, const int* tokens, int tok_ld, int M, float* logits, cudaStream_t s) {
   const gitb200_student_config& k = c->cfg;
-  const int d = k.d_model, dp = c->dp, fp = c->fp, rows = B * L, hd = c->hd;
-  const float scale = 1.0f / sqrtf((float)hd);
+  const int d = k.d_model, dp = c->dp, fp = c->fp, rows = B * L;
   if (pos0 + L > Lmax || Lmax > S_MAX_KEYS || M > S_MAX_KEYS) return sfail(c, GITB200_ERR_INVALID, "sequence / memory longer than %d", S_MAX_KEYS);
   S_TRY(sensure(c, c->x, (size_t)rows * dp));
   S_TRY(sensure(c, c->y, (size_t)rows * dp));
   S_TRY(sensure(c, c->a, (size_t)rows * dp));
   S_TRY(sensure(c, c->q2, (size_t)rows * dp));
   S_TRY(sensure(c, c->h, (size_t)rows * fp));
-  student_embed_kernel<<<rows, 128, 0, s>>>(tokens, tok_ld, pos0, L, pos0, rows, c->embed, c->pe, d, k.vocab, 1.0f / sqrtf((float)d),
-                                            c->x.p, dp);
-  note_launch();
-  S_CUDA_OK(c, cudaGetLastError());
+  S_TRY(s_embed(c, tokens, tok_ld, L, pos0, rows, c->x.p, s));
   for (int l = 0; l < k.n_layers; ++l) {
     const SLayer& W = c->layers[l];
     bf16* cache = c->cache[l].p;
@@ -274,19 +271,13 @@ int run_layers(gitb200_student* c, int B, int L, int pos0, int Lmax, const int* 
     {
       const bf16* qp = (L == Lmax && pos0 == 0) ? cache : cache + (size_t)pos0 * 3 * dp;
       const int ldq = (L == Lmax && pos0 == 0) ? 3 * dp : Lmax * 3 * dp;
-      student_attn_kernel<<<dim3(rows, k.n_head), 32, 0, s>>>(qp, ldq, L, pos0, cache, Lmax, 3 * dp, dp, 2 * dp, pos0 + L, 1, tokens, tok_ld,
-                                                             k.pad, hd, scale, c->a.p, dp);
-      note_launch();
-      S_CUDA_OK(c, cudaGetLastError());
+      S_TRY(s_attn(c, qp, ldq, L, pos0, cache, Lmax, 3 * dp, dp, 2 * dp, pos0 + L, 1, tokens, tok_ld, rows, c->a.p, dp, s));
     }
     S_TRY(s_gemm(c, c->a.p, dp, W.w_sa_out, d, rows, dp, W.b_sa_out, c->x.p, dp, ACT_NONE, c->y.p, dp, nullptr, 0, s));
     S_TRY(s_ln(c, c->y.p, dp, rows, W.n1_g, W.n1_b, c->x.p, dp, s));
     // cross-attention block: x = norm2(x + out_proj(attn(q(x), kv(memory))))
     S_TRY(s_gemm(c, c->x.p, dp, W.w_ca_q, d, rows, dp, W.b_ca_q, nullptr, 0, ACT_NONE, c->q2.p, dp, nullptr, 0, s));
-    student_attn_kernel<<<dim3(rows, k.n_head), 32, 0, s>>>(c->q2.p, dp, L, 0, c->memkv[l].p, M, 2 * dp, 0, dp, M, 0, nullptr, 0, 0, hd, scale,
-                                                           c->a.p, dp);
-    note_launch();
-    S_CUDA_OK(c, cudaGetLastError());
+    S_TRY(s_attn(c, c->q2.p, dp, L, 0, c->memkv[l].p, M, 2 * dp, 0, dp, M, 0, nullptr, 0, rows, c->a.p, dp, s));
     S_TRY(s_gemm(c, c->a.p, dp, W.w_ca_out, d, rows, dp, W.b_ca_out, c->x.p, dp, ACT_NONE, c->y.p, dp, nullptr, 0, s));
     S_TRY(s_ln(c, c->y.p, dp, rows, W.n2_g, W.n2_b, c->x.p, dp, s));
     // feed-forward block: x = norm3(x + linear2(relu(linear1(x))))

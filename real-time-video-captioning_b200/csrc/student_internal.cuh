@@ -12,6 +12,7 @@
 #include "../../include/gitb200.h"
 #include "common.cuh"
 #include "kernels.h"
+#include "student_ops.h"
 
 namespace sdet {
 
@@ -88,14 +89,7 @@ int sensure(gitb200_student* c, SBuf<T>& b, size_t n) {
 }
 inline int round_up(int v, int m) { return (v + m - 1) / m * m; }
 
-// launchers shared with the training step (defined in student.cu)
-int s_gemm(gitb200_student* c, const bf16* A, int lda, const bf16* W, int K, int M, int N, const float* bias, const bf16* residual,
-           int ldr, int act, bf16* out, int ldo, float* out32, int ldo32, cudaStream_t s);
-int s_ln(gitb200_student* c, const bf16* x, int ldx, int rows, const float* g, const float* b, bf16* out, int ldo, cudaStream_t s);
-int s_embed(gitb200_student* c, const int* tokens, int tok_ld, int L, int rows, bf16* out, cudaStream_t s);
-// softmax(q k^T * scale + mask) v, one warp per (query row, head); see student_attn_kernel
-int s_attn(gitb200_student* c, const bf16* q, int ldq, int Lq, const bf16* kv, int kv_rows, int ldkv, int k_off, int v_off, int n_keys,
-           int causal, const int* tokens, int tok_ld, int rows, bf16* out, int ldo, cudaStream_t s);
+// the kernel launchers (s_*: student.cu, t_*: student_train.cu) are declared in student_ops.h
 void student_train_destroy(gitb200_student* c);
 
 }  // namespace sdet

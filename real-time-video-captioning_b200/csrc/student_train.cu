@@ -116,8 +116,9 @@ __device__ __forceinline__ float block_reduce(float v, float* sh, bool is_max) {
 }
 
 // One CTA per row r = (b, i): KL(batchmean) * T^2 + CE(ignore_index) and d loss / d student-logits (model.py:922-935, :983).
-//   loss[0] += KL_row / B * T^2, loss[1] += CE_row / n_valid;  dlogits[r, v] = T (p_s - p_t) / B + [CE row] (p_s1 - onehot) / n_valid
-// where p_s = softmax(s / T), p_t = softmax(t / T), p_s1 = softmax(s).
+//   loss[r] = KL_row / B * T^2, loss[R + r] = CE_row / n_valid (0 without a CE target);
+//   dlogits[r, v] = T (p_s - p_t) / B + [CE row] (p_s1 - onehot) / n_valid  where p_s = softmax(s / T), p_t = softmax(t / T),
+//   p_s1 = softmax(s).  loss_total_kernel sums the rows' parts in a fixed order.
 __global__ void __launch_bounds__(256) distill_loss_kernel(const float* __restrict__ s_logits, int ld_s, const float* __restrict__ t_logits,
                                                            int ld_t, const int* __restrict__ tokens, int B, int L, int V, int Vp, int ignore,
                                                            float temperature, const int* __restrict__ n_valid, bf16* __restrict__ dlogits,
@@ -162,8 +163,8 @@ __global__ void __launch_bounds__(256) distill_loss_kernel(const float* __restri
   }
   kl = block_reduce(kl, sh, false);
   if (threadIdx.x == 0) {
-    atomicAdd(&loss[0], kl * temperature * temperature / (float)B);
-    if (ce_row && nv > 0) atomicAdd(&loss[1], -(s[tgt] - ms - l1) / (float)nv);
+    loss[r] = kl * temperature * temperature / (float)B;
+    loss[gridDim.x + r] = (ce_row && nv > 0) ? -(s[tgt] - ms - l1) / (float)nv : 0.f;
   }
 }
 
@@ -301,14 +302,45 @@ __global__ void __launch_bounds__(128) attn_bwd_kernel(const bf16* __restrict__ 
   }
 }
 
-// d embed[tok(r), c] += dx0[r, c] / sqrt(d)   (model.py:144-148: the embedding sum is divided by sqrt(d) after adding pe)
-__global__ void embed_bwd_kernel(const int* __restrict__ tokens, int rows, const bf16* __restrict__ dx, int ld, int d, int vocab,
-                                 float inv_sqrt_d, float* __restrict__ dembed) {
-  const int r = blockIdx.x;
+// d embed[tok, c] = sum over the rows r with tok(r) == tok of dx0[r, c] / sqrt(d)   (model.py:144-148: the embedding sum is divided
+// by sqrt(d) after adding pe).  One CTA per row; the CTA of a token's first row sums that token's rows in row order and stores
+// the result (every token repeats: CLS starts each sequence), so the gradient does not depend on block scheduling.  The rows
+// of the token are gathered, in order, 32 * EMB_WARPS at a time into a shared list (ballot compaction); the column loop then
+// reads only those rows.  acc: d floats of dynamic shared memory, one column per thread and pass.
+constexpr int EMB_WARPS = 4;
+__global__ void __launch_bounds__(32 * EMB_WARPS) embed_bwd_kernel(const int* __restrict__ tokens, int rows, const bf16* __restrict__ dx,
+                                                                   int ld, int d, int vocab, float inv_sqrt_d, float* __restrict__ dembed) {
+  extern __shared__ float acc[];
+  __shared__ int list[32 * EMB_WARPS];
+  __shared__ int wcnt[EMB_WARPS];
+  const int r = blockIdx.x, tid = threadIdx.x, lane = tid & 31, warp = tid >> 5;
   if (r >= rows) return;
-  int tok = tokens[r];
-  tok = min(max(tok, 0), vocab - 1);
-  for (int c = threadIdx.x; c < d; c += blockDim.x) atomicAdd(&dembed[(size_t)tok * d + c], __bfloat162float(dx[(size_t)r * ld + c]) * inv_sqrt_d);
+  const int tok = min(max(tokens[r], 0), vocab - 1);
+  bool seen = false;
+  for (int j = tid; j < r && !seen; j += blockDim.x) seen = min(max(tokens[j], 0), vocab - 1) == tok;
+  if (__syncthreads_or(seen)) return;
+  for (int c = tid; c < d; c += blockDim.x) acc[c] = 0.f;
+  for (int base = r; base < rows; base += blockDim.x) {
+    const int j = base + tid;
+    const bool m = j < rows && min(max(tokens[j], 0), vocab - 1) == tok;
+    const unsigned bal = __ballot_sync(0xffffffffu, m);
+    if (lane == 0) wcnt[warp] = __popc(bal);
+    __syncthreads();
+    int off = 0, n = 0;
+    for (int w = 0; w < EMB_WARPS; ++w) {
+      off += w < warp ? wcnt[w] : 0;
+      n += wcnt[w];
+    }
+    if (m) list[off + __popc(bal & ((1u << lane) - 1u))] = j;
+    __syncthreads();
+    for (int c = tid; c < d; c += blockDim.x) {
+      float a = acc[c];
+      for (int k = 0; k < n; ++k) a = __fadd_rn(a, __fmul_rn(__bfloat162float(dx[(size_t)list[k] * ld + c]), inv_sqrt_d));
+      acc[c] = a;
+    }
+    __syncthreads();
+  }
+  for (int c = tid; c < d; c += blockDim.x) dembed[(size_t)tok * d + c] = acc[c];
 }
 
 // torch.optim.Adam (no weight decay, no amsgrad): one element per thread over the flat vectors
@@ -335,13 +367,27 @@ __global__ void repack_kernel(const float* __restrict__ p, int rows_pad, int col
   if (wt) wt[(size_t)c * wt_ld + r] = v;
 }
 
-__global__ void loss_total_kernel(const float* __restrict__ parts, float* __restrict__ out) {
-  out[0] = parts[0] + parts[1];
-  out[1] = parts[0];
-  out[2] = parts[1];
+// out = (KL + CE, KL, CE) from the per-row parts [2][R], summed by one warp in a fixed order (run-to-run identical)
+__global__ void loss_total_kernel(const float* __restrict__ parts, int R, float* __restrict__ out) {
+  float kl = 0.f, ce = 0.f;
+  for (int r = threadIdx.x; r < R; r += 32) {
+    kl += parts[r];
+    ce += parts[R + r];
+  }
+  kl = warp_sum(kl);
+  ce = warp_sum(ce);
+  if (threadIdx.x == 0) {
+    out[0] = kl + ce;
+    out[1] = kl;
+    out[2] = ce;
+  }
 }
 
-// ------------------------------------------------------------------ host helpers
+}  // namespace
+
+// ------------------------------------------------------------------ launchers (student_ops.h)
+namespace sdet {
+
 int t_transpose(gitb200_student* c, const bf16* src, int ld_src, int R, int C, bf16* dst, int R_pad, int C_pad, cudaStream_t s) {
   dim3 grid((C_pad + 31) / 32, (R_pad + 31) / 32), block(32, 8);
   transpose_pad_kernel<<<grid, block, 0, s>>>(src, ld_src, R, C, dst, R_pad, R_pad, C_pad);
@@ -356,29 +402,19 @@ int t_colsum(gitb200_student* c, const bf16* x, int ld, int R, int C, float* out
   return 0;
 }
 
-PEntry* find_entry(STrain* t, const std::string& name, int src_row0 = 0) {
-  for (auto& e : t->entries)
-    if (e.name == name && e.src_row0 == src_row0) return &e;
-  return nullptr;
-}
-float* G_of(STrain* t, float* G, const std::string& name, int src_row0 = 0) { return G + find_entry(t, name, src_row0)->off; }
-
-// dW[Npad, Kpad] (fp32, into the flat gradient vector) = dY^T X : dY bf16 [R, ldy] (N_pad columns), X bf16 [R, ldx] (K_pad columns)
 int t_weight_grad(gitb200_student* c, const bf16* dY, int ldy, int n_pad, const bf16* X, int ldx, int x_cols, int k_pad, int R, float* dW,
-                  cudaStream_t s) {
-  STrain* t = c->train;
+                  bf16* tA, bf16* tB, cudaStream_t s) {
   const int Rp = round_up(R, 64);
-  S_TRY(t_transpose(c, dY, ldy, R, n_pad, t->tA.p, Rp, n_pad, s));
-  S_TRY(t_transpose(c, X, ldx, R, x_cols, t->tB.p, Rp, k_pad, s));
-  return s_gemm(c, t->tA.p, Rp, t->tB.p, Rp, n_pad, k_pad, nullptr, nullptr, 0, ACT_NONE, nullptr, 0, dW, k_pad, s);
+  S_TRY(t_transpose(c, dY, ldy, R, n_pad, tA, Rp, n_pad, s));
+  S_TRY(t_transpose(c, X, ldx, R, x_cols, tB, Rp, k_pad, s));
+  return s_gemm(c, tA, Rp, tB, Rp, n_pad, k_pad, nullptr, nullptr, 0, ACT_NONE, nullptr, 0, dW, k_pad, s);
 }
 
 int t_ln_bwd(gitb200_student* c, const bf16* y, const bf16* dx, int rows, const float* gamma, bf16* dy, float* dgamma, float* dbeta,
-             cudaStream_t s) {
-  STrain* t = c->train;
+             float* stats, cudaStream_t s) {
   const int d = c->cfg.d_model, dp = c->dp;
-  ln_bwd_kernel<<<(rows * 32 + 255) / 256, 256, 0, s>>>(y, dx, dp, rows, d, gamma, c->cfg.ln_eps, dy, t->stats.p);
-  ln_param_grad_kernel<<<(d + 127) / 128, 128, 0, s>>>(y, dx, dp, rows, d, t->stats.p, dgamma, dbeta);
+  ln_bwd_kernel<<<(rows * 32 + 255) / 256, 256, 0, s>>>(y, dx, dp, rows, d, gamma, c->cfg.ln_eps, dy, stats);
+  ln_param_grad_kernel<<<(d + 127) / 128, 128, 0, s>>>(y, dx, dp, rows, d, stats, dgamma, dbeta);
   note_launch(2);
   S_CUDA_OK(c, cudaGetLastError());
   return 0;
@@ -387,9 +423,11 @@ int t_ln_bwd(gitb200_student* c, const bf16* y, const bf16* dx, int rows, const 
 int t_attn_bwd(gitb200_student* c, const bf16* q, int ldq, int Lq, const bf16* kv, int kv_rows, int ldkv, int k_off, int v_off, int n_keys,
                int causal, const int* tokens, int tok_ld, int B, const bf16* dO, bf16* dq, int lddq, bf16* dkv, int lddkv, int dk_off,
                int dv_off, cudaStream_t s) {
+  if (Lq < 1 || Lq > T_MAX_SEQ || n_keys < 1 || n_keys > T_MAX_SEQ)
+    return sfail(c, GITB200_ERR_INVALID, "attention backward over %d queries x %d keys (1 .. %d each)", Lq, n_keys, T_MAX_SEQ);
   const int hd = c->hd;
   const size_t smem = ((size_t)(2 * Lq + 2 * n_keys) * (hd + 1) + (size_t)2 * Lq * (n_keys + 1)) * sizeof(float);
-  static size_t attr = 0;
+  static size_t attr = 0;  // process-wide, not per device: one process trains on one GPU (dist.py)
   if (smem > 48 * 1024 && smem > attr) {
     S_CUDA_OK(c, cudaFuncSetAttribute(attn_bwd_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
     attr = smem;
@@ -401,6 +439,47 @@ int t_attn_bwd(gitb200_student* c, const bf16* q, int ldq, int Lq, const bf16* k
   S_CUDA_OK(c, cudaGetLastError());
   return 0;
 }
+
+int t_distill_loss(gitb200_student* c, const float* s_logits, int ld_s, const float* t_logits, int ld_t, const int* tokens, int B, int L,
+                   float temperature, int* n_valid, bf16* dlogits, float* loss, float* loss_out, cudaStream_t s) {
+  count_valid_kernel<<<1, 256, 0, s>>>(tokens, B, L, 0, n_valid);
+  distill_loss_kernel<<<B * L, 256, 0, s>>>(s_logits, ld_s, t_logits, ld_t, tokens, B, L, c->cfg.vocab, c->vp, 0, temperature, n_valid,
+                                            dlogits, loss);
+  note_launch(2);
+  S_CUDA_OK(c, cudaGetLastError());
+  loss_total_kernel<<<1, 32, 0, s>>>(loss, B * L, loss_out);  // (KL + CE, KL, CE)
+  note_launch();
+  S_CUDA_OK(c, cudaGetLastError());
+  return 0;
+}
+
+int t_relu_bwd(gitb200_student* c, const bf16* h, bf16* dh, size_t n, cudaStream_t s) {
+  relu_bwd_kernel<<<(unsigned)((n + 255) / 256), 256, 0, s>>>(h, dh, n);
+  note_launch();
+  S_CUDA_OK(c, cudaGetLastError());
+  return 0;
+}
+
+int t_embed_bwd(gitb200_student* c, const int* tokens, int rows, const bf16* dx, int ld, float* dembed, cudaStream_t s) {
+  const int d = c->cfg.d_model;
+  const size_t smem = (size_t)d * sizeof(float);  // the accumulators of one token's row of the table
+  if (smem > 48 * 1024) return sfail(c, GITB200_ERR_INVALID, "embedding backward holds at most %d columns, not %d", 48 * 1024 / 4, d);
+  embed_bwd_kernel<<<rows, 32 * EMB_WARPS, smem, s>>>(tokens, rows, dx, ld, d, c->cfg.vocab, 1.0f / sqrtf((float)d), dembed);
+  note_launch();
+  S_CUDA_OK(c, cudaGetLastError());
+  return 0;
+}
+
+}  // namespace sdet
+
+namespace {
+
+PEntry* find_entry(STrain* t, const std::string& name, int src_row0 = 0) {
+  for (auto& e : t->entries)
+    if (e.name == name && e.src_row0 == src_row0) return &e;
+  return nullptr;
+}
+float* G_of(STrain* t, float* G, const std::string& name, int src_row0 = 0) { return G + find_entry(t, name, src_row0)->off; }
 
 int repack_all(gitb200_student* c, cudaStream_t s) {
   STrain* t = c->train;
@@ -628,23 +707,23 @@ int gitb200_student_train_forward(gitb200_student* c, const int32_t* tokens, con
   S_TRY(sensure(c, t->dmemkv, (size_t)Rm * 2 * dp));
   S_TRY(sensure(c, t->dmem, (size_t)Rm * dp));
   S_TRY(sensure(c, t->stats, (size_t)2 * R));
-  S_TRY(sensure(c, t->loss, 4));
+  S_TRY(sensure(c, t->loss, (size_t)2 * R));
   S_TRY(sensure(c, t->nvalid, 1));
   S_TRY(sensure(c, t->toks, (size_t)R));
   S_CUDA_OK(c, cudaMemcpyAsync(t->toks.p, tokens, (size_t)R * sizeof(int), cudaMemcpyDeviceToDevice, s));  // the backward pass reads them again
   S_CUDA_OK(c, cast_f32_to_bf16(memory, Rm, d, d, t->mem.p, d, Rm, d, s));
-  S_TRY(s_embed(c, t->toks.p, L, L, R, t->acts[0].x0.p, s));
+  S_TRY(s_embed(c, t->toks.p, L, L, 0, R, t->acts[0].x0.p, s));
   for (int l = 0; l < k.n_layers; ++l) {
     const SLayer& W = c->layers[l];
     LayerAct& A = t->acts[l];
     bf16* x3 = (l + 1 < k.n_layers) ? t->acts[l + 1].x0.p : t->xo.p;
     S_TRY(s_gemm(c, A.x0.p, dp, W.w_sa_in, d, R, 3 * dp, W.b_sa_in, nullptr, 0, ACT_NONE, A.qkv.p, 3 * dp, nullptr, 0, s));
-    S_TRY(s_attn(c, A.qkv.p, 3 * dp, L, A.qkv.p, L, 3 * dp, dp, 2 * dp, L, 1, t->toks.p, L, R, A.a.p, dp, s));
+    S_TRY(s_attn(c, A.qkv.p, 3 * dp, L, 0, A.qkv.p, L, 3 * dp, dp, 2 * dp, L, 1, t->toks.p, L, R, A.a.p, dp, s));
     S_TRY(s_gemm(c, A.a.p, dp, W.w_sa_out, d, R, dp, W.b_sa_out, A.x0.p, dp, ACT_NONE, A.y1.p, dp, nullptr, 0, s));
     S_TRY(s_ln(c, A.y1.p, dp, R, W.n1_g, W.n1_b, A.x1.p, dp, s));
     S_TRY(s_gemm(c, A.x1.p, dp, W.w_ca_q, d, R, dp, W.b_ca_q, nullptr, 0, ACT_NONE, A.q2.p, dp, nullptr, 0, s));
     S_TRY(s_gemm(c, t->mem.p, d, W.w_ca_kv, d, Rm, 2 * dp, W.b_ca_kv, nullptr, 0, ACT_NONE, A.memkv.p, 2 * dp, nullptr, 0, s));
-    S_TRY(s_attn(c, A.q2.p, dp, L, A.memkv.p, M, 2 * dp, 0, dp, M, 0, nullptr, 0, R, A.a2.p, dp, s));
+    S_TRY(s_attn(c, A.q2.p, dp, L, 0, A.memkv.p, M, 2 * dp, 0, dp, M, 0, nullptr, 0, R, A.a2.p, dp, s));
     S_TRY(s_gemm(c, A.a2.p, dp, W.w_ca_out, d, R, dp, W.b_ca_out, A.x1.p, dp, ACT_NONE, A.y2.p, dp, nullptr, 0, s));
     S_TRY(s_ln(c, A.y2.p, dp, R, W.n2_g, W.n2_b, A.x2.p, dp, s));
     S_TRY(s_gemm(c, A.x2.p, dp, W.w_ff1, d, R, fp, W.b_ff1, nullptr, 0, ACT_RELU, A.h.p, fp, nullptr, 0, s));
@@ -652,15 +731,8 @@ int gitb200_student_train_forward(gitb200_student* c, const int32_t* tokens, con
     S_TRY(s_ln(c, A.y3.p, dp, R, W.n3_g, W.n3_b, x3, dp, s));
   }
   S_TRY(s_gemm(c, t->xo.p, dp, c->w_vocab, d, R, vp, c->b_vocab, nullptr, 0, ACT_NONE, nullptr, 0, t->logits.p, vp, s));
-  S_CUDA_OK(c, cudaMemsetAsync(t->loss.p, 0, 4 * sizeof(float), s));
-  count_valid_kernel<<<1, 256, 0, s>>>(t->toks.p, B, L, 0, t->nvalid.p);
-  distill_loss_kernel<<<R, 256, 0, s>>>(t->logits.p, vp, teacher_logits, ld_teacher, t->toks.p, B, L, k.vocab, vp, 0, temperature, t->nvalid.p,
-                                        t->dlogits.p, t->loss.p);
-  note_launch(2);
-  S_CUDA_OK(c, cudaGetLastError());
-  loss_total_kernel<<<1, 1, 0, s>>>(t->loss.p, loss_out);  // (KL + CE, KL, CE)
-  note_launch();
-  S_CUDA_OK(c, cudaGetLastError());
+  S_TRY(t_distill_loss(c, t->logits.p, vp, teacher_logits, ld_teacher, t->toks.p, B, L, temperature, t->nvalid.p, t->dlogits.p, t->loss.p,
+                       loss_out, s));
   t->B = B; t->L = L; t->M = M;
   t->have_forward = true;
   t->have_head = false;
@@ -680,13 +752,13 @@ int gitb200_student_train_backward(gitb200_student* c, int phase, float* grads, 
   const int d = k.d_model, dp = c->dp, fp = c->fp, vp = c->vp, B = t->B, L = t->L, M = t->M, R = B * L, Rm = B * M;
   if (phase == 0) {
     // logits = xo W_v^T + b_v
-    S_TRY(t_weight_grad(c, t->dlogits.p, vp, vp, t->xo.p, dp, dp, dp, R, G_of(t, grads, "linear.weight"), s));
+    S_TRY(t_weight_grad(c, t->dlogits.p, vp, vp, t->xo.p, dp, dp, dp, R, G_of(t, grads, "linear.weight"), t->tA.p, t->tB.p, s));
     S_TRY(t_colsum(c, t->dlogits.p, vp, R, vp, G_of(t, grads, "linear.bias"), s));
     S_TRY(s_gemm(c, t->dlogits.p, vp, t->wt_vocab, vp, R, dp, nullptr, nullptr, 0, ACT_NONE, t->dx.p, dp, nullptr, 0, s));
     t->have_head = true;
     return GITB200_OK;
   }
-  // the embedding gradient is a scatter-add: start from zero
+  // embed_bwd_kernel stores the rows of the tokens that occur; the rows of the others must read as zero
   {
     PEntry* e = find_entry(t, "embed.weight");
     S_CUDA_OK(c, cudaMemsetAsync(grads + e->off, 0, (size_t)e->rows_pad * e->cols_pad * sizeof(float), s));
@@ -697,44 +769,42 @@ int gitb200_student_train_backward(gitb200_student* c, int phase, float* grads, 
     const LayerT& T = t->lt[l];
     LayerAct& A = t->acts[l];
     // ---- x3 = norm3(y3), y3 = h W2^T + b2 + x2, h = relu(x2 W1^T + b1)              (dx holds d loss / d x3)
-    S_TRY(t_ln_bwd(c, A.y3.p, t->dx.p, R, W.n3_g, t->dy.p, G_of(t, grads, p + "norm3.weight"), G_of(t, grads, p + "norm3.bias"), s));
-    S_TRY(t_weight_grad(c, t->dy.p, dp, dp, A.h.p, fp, fp, fp, R, G_of(t, grads, p + "linear2.weight"), s));
+    S_TRY(t_ln_bwd(c, A.y3.p, t->dx.p, R, W.n3_g, t->dy.p, G_of(t, grads, p + "norm3.weight"), G_of(t, grads, p + "norm3.bias"), t->stats.p, s));
+    S_TRY(t_weight_grad(c, t->dy.p, dp, dp, A.h.p, fp, fp, fp, R, G_of(t, grads, p + "linear2.weight"), t->tA.p, t->tB.p, s));
     S_TRY(t_colsum(c, t->dy.p, dp, R, dp, G_of(t, grads, p + "linear2.bias"), s));
     S_TRY(s_gemm(c, t->dy.p, dp, T.ff2, dp, R, fp, nullptr, nullptr, 0, ACT_NONE, t->dh.p, fp, nullptr, 0, s));
-    relu_bwd_kernel<<<(unsigned)(((size_t)R * fp + 255) / 256), 256, 0, s>>>(A.h.p, t->dh.p, (size_t)R * fp);
-    note_launch();
-    S_TRY(t_weight_grad(c, t->dh.p, fp, fp, A.x2.p, dp, dp, dp, R, G_of(t, grads, p + "linear1.weight"), s));
+    S_TRY(t_relu_bwd(c, A.h.p, t->dh.p, (size_t)R * fp, s));
+    S_TRY(t_weight_grad(c, t->dh.p, fp, fp, A.x2.p, dp, dp, dp, R, G_of(t, grads, p + "linear1.weight"), t->tA.p, t->tB.p, s));
     S_TRY(t_colsum(c, t->dh.p, fp, R, fp, G_of(t, grads, p + "linear1.bias"), s));
     S_TRY(s_gemm(c, t->dh.p, fp, T.ff1, fp, R, dp, nullptr, t->dy.p, dp, ACT_NONE, t->dx.p, dp, nullptr, 0, s));  // d x2 = dh W1 + d y3
     // ---- x2 = norm2(y2), y2 = a2 Wo^T + bo + x1, a2 = attn(q2, memkv), q2 = x1 Wq^T + bq, memkv = mem Wkv^T + bkv
-    S_TRY(t_ln_bwd(c, A.y2.p, t->dx.p, R, W.n2_g, t->dy.p, G_of(t, grads, p + "norm2.weight"), G_of(t, grads, p + "norm2.bias"), s));
-    S_TRY(t_weight_grad(c, t->dy.p, dp, dp, A.a2.p, dp, dp, dp, R, G_of(t, grads, p + "multihead_attn.out_proj.weight"), s));
+    S_TRY(t_ln_bwd(c, A.y2.p, t->dx.p, R, W.n2_g, t->dy.p, G_of(t, grads, p + "norm2.weight"), G_of(t, grads, p + "norm2.bias"), t->stats.p, s));
+    S_TRY(t_weight_grad(c, t->dy.p, dp, dp, A.a2.p, dp, dp, dp, R, G_of(t, grads, p + "multihead_attn.out_proj.weight"), t->tA.p, t->tB.p, s));
     S_TRY(t_colsum(c, t->dy.p, dp, R, dp, G_of(t, grads, p + "multihead_attn.out_proj.bias"), s));
     S_TRY(s_gemm(c, t->dy.p, dp, T.ca_out, dp, R, dp, nullptr, nullptr, 0, ACT_NONE, t->da.p, dp, nullptr, 0, s));
     S_TRY(t_attn_bwd(c, A.q2.p, dp, L, A.memkv.p, M, 2 * dp, 0, dp, M, 0, nullptr, 0, B, t->da.p, t->dqkv.p, dp, t->dmemkv.p, 2 * dp, 0, dp, s));
-    S_TRY(t_weight_grad(c, t->dqkv.p, dp, dp, A.x1.p, dp, dp, dp, R, G_of(t, grads, p + "multihead_attn.in_proj_weight", 0), s));
+    S_TRY(t_weight_grad(c, t->dqkv.p, dp, dp, A.x1.p, dp, dp, dp, R, G_of(t, grads, p + "multihead_attn.in_proj_weight", 0), t->tA.p, t->tB.p, s));
     S_TRY(t_colsum(c, t->dqkv.p, dp, R, dp, G_of(t, grads, p + "multihead_attn.in_proj_bias", 0), s));
     S_TRY(s_gemm(c, t->dqkv.p, dp, T.ca_q, dp, R, dp, nullptr, t->dy.p, dp, ACT_NONE, t->dx.p, dp, nullptr, 0, s));  // d x1 = dq2 Wq + d y2
     // the k | v blocks of in_proj are adjacent in the layout ([2*dp, dp] fp32): one GEMM fills both
-    S_TRY(t_weight_grad(c, t->dmemkv.p, 2 * dp, 2 * dp, t->mem.p, d, d, dp, Rm, G_of(t, grads, p + "multihead_attn.in_proj_weight", d), s));
+    S_TRY(t_weight_grad(c, t->dmemkv.p, 2 * dp, 2 * dp, t->mem.p, d, d, dp, Rm, G_of(t, grads, p + "multihead_attn.in_proj_weight", d), t->tA.p,
+                        t->tB.p, s));
     S_TRY(t_colsum(c, t->dmemkv.p, 2 * dp, Rm, 2 * dp, G_of(t, grads, p + "multihead_attn.in_proj_bias", d), s));
     S_TRY(s_gemm(c, t->dmemkv.p, 2 * dp, T.ca_kv, 2 * dp, Rm, dp, nullptr, l + 1 < k.n_layers ? t->dmem.p : nullptr, dp, ACT_NONE, t->dmem.p, dp,
                  nullptr, 0, s));  // d memory accumulates over the layers
     // ---- x1 = norm1(y1), y1 = a Wo^T + bo + x0, a = self-attn(qkv), qkv = x0 Win^T + bin
-    S_TRY(t_ln_bwd(c, A.y1.p, t->dx.p, R, W.n1_g, t->dy.p, G_of(t, grads, p + "norm1.weight"), G_of(t, grads, p + "norm1.bias"), s));
-    S_TRY(t_weight_grad(c, t->dy.p, dp, dp, A.a.p, dp, dp, dp, R, G_of(t, grads, p + "self_attn.out_proj.weight"), s));
+    S_TRY(t_ln_bwd(c, A.y1.p, t->dx.p, R, W.n1_g, t->dy.p, G_of(t, grads, p + "norm1.weight"), G_of(t, grads, p + "norm1.bias"), t->stats.p, s));
+    S_TRY(t_weight_grad(c, t->dy.p, dp, dp, A.a.p, dp, dp, dp, R, G_of(t, grads, p + "self_attn.out_proj.weight"), t->tA.p, t->tB.p, s));
     S_TRY(t_colsum(c, t->dy.p, dp, R, dp, G_of(t, grads, p + "self_attn.out_proj.bias"), s));
     S_TRY(s_gemm(c, t->dy.p, dp, T.sa_out, dp, R, dp, nullptr, nullptr, 0, ACT_NONE, t->da.p, dp, nullptr, 0, s));
     S_TRY(t_attn_bwd(c, A.qkv.p, 3 * dp, L, A.qkv.p, L, 3 * dp, dp, 2 * dp, L, 1, t->toks.p, L, B, t->da.p, t->dqkv.p, 3 * dp, t->dqkv.p, 3 * dp, dp,
                      2 * dp, s));
     // q | k | v blocks are adjacent in the layout ([3*dp, dp] fp32): one GEMM fills all three
-    S_TRY(t_weight_grad(c, t->dqkv.p, 3 * dp, 3 * dp, A.x0.p, dp, dp, dp, R, G_of(t, grads, p + "self_attn.in_proj_weight", 0), s));
+    S_TRY(t_weight_grad(c, t->dqkv.p, 3 * dp, 3 * dp, A.x0.p, dp, dp, dp, R, G_of(t, grads, p + "self_attn.in_proj_weight", 0), t->tA.p, t->tB.p, s));
     S_TRY(t_colsum(c, t->dqkv.p, 3 * dp, R, 3 * dp, G_of(t, grads, p + "self_attn.in_proj_bias", 0), s));
     S_TRY(s_gemm(c, t->dqkv.p, 3 * dp, T.sa_in, 3 * dp, R, dp, nullptr, t->dy.p, dp, ACT_NONE, t->dx.p, dp, nullptr, 0, s));  // d x0 = dqkv Win + d y1
   }
-  embed_bwd_kernel<<<R, 128, 0, s>>>(t->toks.p, R, t->dx.p, dp, d, k.vocab, 1.0f / sqrtf((float)d), G_of(t, grads, "embed.weight"));
-  note_launch();
-  S_CUDA_OK(c, cudaGetLastError());
+  S_TRY(t_embed_bwd(c, t->toks.p, R, t->dx.p, dp, G_of(t, grads, "embed.weight"), s));
   if (d_memory) S_CUDA_OK(c, cast_bf16_to_f32(t->dmem.p, Rm, d, dp, d_memory, d, s));
   t->have_forward = false;
   return GITB200_OK;

@@ -91,6 +91,7 @@ class StudentCandidateV1(nn.Module):
         self.image_enc_name = image_enc_name
         self.image_encoder = image_encoder            # model.py:72 builds TinyVIT(image_enc_name) through timm
         self.n_head, self.d_model, self.d_ffn, self.dropout = n_head, d_model, d_ffn, dropout
+        self.ln_eps = 1e-5                            # LayerNorm eps: nn.TransformerDecoderLayer's default layer_norm_eps
         self.decoder = _DecoderParams(d_model, d_ffn, num_decoder_layers)
         self.embed = nn.Embedding(vocab_length, d_model)
         self.linear = nn.Linear(d_model, vocab_length)
@@ -128,7 +129,7 @@ class StudentCandidateV1(nn.Module):
         self.close()
         lib = _lib.load()
         cfg = StudentConfig(self.d_model, self.n_head, self.d_ffn, self.decoder.num_layers, self.embed.num_embeddings,
-                            self.pos_enc.pe.shape[1], self.cls_token_id, self.sep_token_id, 0, 1e-5)
+                            self.pos_enc.pe.shape[1], self.cls_token_id, self.sep_token_id, 0, self.ln_eps)
         h = ctypes.c_void_p()
         _check(lib.gitb200_student_create(ctypes.byref(cfg), p.device.index or 0, ctypes.byref(h)), lib, None, "gitb200_student_create")
         if self._train_cfg is not None:

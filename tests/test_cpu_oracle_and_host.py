@@ -218,6 +218,21 @@ def test_op_modes_shim_builds_and_links_against_the_library():
     assert shim.opm_text_attention_workspace_floats(4, 12, 3) == 4 * 12 * 3 * (64 + 2)
 
 
+def test_student_ops_shim_builds_and_links_against_the_library():
+    """tests/cuda/student_ops.cpp (the student operator tests' entry points over csrc/student_ops.h) must keep compiling, and
+    every launcher it calls must resolve in libgitb200.so (ctypes loads with RTLD_NOW, so a launcher whose signature drifted
+    from student_ops.h fails here, with a mangled-name error, instead of in the GPU tests)."""
+    import op_modes_shim
+    lib_mod = importlib.import_module("real-time-video-captioning_b200._lib")
+    if not os.path.exists(lib_mod.LIB_PATH):
+        pytest.skip("libgitb200.so is not built")
+    if op_modes_shim.compiler() is None:
+        pytest.skip("no C++ compiler")
+    lib_mod.load()
+    shim = op_modes_shim.load_student()
+    assert all(hasattr(shim, n) for n in op_modes_shim.STUDENT_SIGNATURES)
+
+
 @pytest.mark.skipif(torch.cuda.is_available(), reason="checks the no-GPU failure mode")
 def test_no_gpu_means_loud_failure_not_fallback():
     lib_mod = importlib.import_module("real-time-video-captioning_b200._lib")

@@ -220,7 +220,8 @@ def test_distillation_step_gradients_match_autograd(B, L, F, temperature):
     parameter gradient of gitb200_student_train_forward / _backward against torch.autograd on the stock nn modules the
     reference instantiates (oracle/student_oracle.py: KLDivLoss(batchmean) * T^2 + CrossEntropyLoss(ignore_index=0),
     model.py:922-935, :983).  bf16 activations / activation gradients, fp32 weight gradients: relative Frobenius error
-    < 3e-2 over all parameters together, < 1e-1 for any single tensor (the 21-row case leaves single tensors at 6-7e-2)."""
+    < 3e-2 over all parameters together, < 8e-2 for any single tensor (the step is bit-reproducible, so these seeded cases
+    measure the same every run: worst tensor linear1.weight of layer 1, 6.6e-2 in the 21-row case, 4.9e-2 at 8 x 20)."""
     cfg = st.StudentConfig()
     m, s = _gpu_student(cfg, seed=21)
     y, mem, teacher = _train_inputs(cfg, B, L, F, seed=B * 10 + L)
@@ -232,18 +233,18 @@ def test_distillation_step_gradients_match_autograd(B, L, F, temperature):
     assert abs(kl - info["kl"]) < 2e-2 * abs(info["kl"]) and abs(ce - info["ce"]) < 2e-2 * abs(info["ce"]), (kl, info["kl"], ce, info["ce"])
     grads = {k: v.cpu() for k, v in s.gradients().items()}
     assert set(grads) == set(ref_grads)
-    worst, num, den = ("", 0.0), 0.0, 0.0
+    worst, num, den, per = ("", 0.0), 0.0, 0.0, {}
     for k, ref in ref_grads.items():
-        e = _rel(grads[k], ref)
+        e = per[k] = _rel(grads[k], ref)
         num += (grads[k].double() - ref.double()).pow(2).sum().item()
         den += ref.double().pow(2).sum().item()
         if e > worst[1]:
             worst = (k, e)
-        assert e < 1e-1, (k, e)
+        assert e < 8e-2, (k, e)
     total = (num / den) ** 0.5
     e_mem = _rel(out["d_memory"].cpu(), ref_dmem)
     record("distillation_step_grads", B=B, L=L, temperature=temperature, loss=loss, ref_loss=info["loss"], all_params_rel_fro=total,
-           worst_tensor=worst[0], worst_rel_fro=worst[1], d_memory_rel_fro=e_mem)
+           worst_tensor=worst[0], worst_rel_fro=worst[1], d_memory_rel_fro=e_mem, per_tensor_rel_fro=per)
     assert total < 3e-2, total
     assert e_mem < 6e-2, e_mem
     # rows of the embedding table that do not occur in y get exactly zero gradient
