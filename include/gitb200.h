@@ -335,7 +335,18 @@ int gitb200_student_logits_ld(const gitb200_student* s); /* vocabulary rounded u
  * y[:, 1:]).  Parameters live in ONE flat fp32 vector (padded to the GEMM tile multiples; the vocabulary head first); the
  * caller supplies a gradient vector of the same length (n = return value of _train_begin) and all-reduces it between
  * _train_backward and _train_apply -- [0, head_floats) may be reduced as soon as phase 0 has been enqueued, while phase 1
- * runs.  Dropout is not applied (parity oracle: torch.autograd on the same modules with dropout off).
+ * runs.
+ * Dropout (opt-in, off after _train_begin): _train_set_dropout(p, seed, step) with 0 < p < 1 applies nn.TransformerDecoderLayer's
+ * six dropout sites of every layer l in its train-mode call order, site = 6 l + k: k = 0 self-attention probabilities [B, H, L, L],
+ * 1 dropout1 on the self-attention output [B*L, d], 2 cross-attention probabilities [B, H, L, M], 3 dropout2 [B*L, d],
+ * 4 the feed-forward's inner dropout after the ReLU [B*L, d_ffn], 5 dropout3 [B*L, d].  Element idx over the LOGICAL tensor
+ * (probabilities: ((b H + h) L + i) n_keys + j; activations: r * cols + c, r = b L + i) is kept iff
+ * u >= p (in double; u = ((w >> 8) + 0.5) 2^-24, w = word idx % 4 of Philox4x32-10 with counter (idx / 4, step mod 2^32, site,
+ * 0x44524F50) and key (seed & 0xffffffff, seed >> 32)); a kept element is scaled by 1 / (1 - p) in fp32.  Masks do not depend
+ * on the rank: pass seed + rank for independent masks per rank.  `step` counts the _train_forward calls that applied dropout
+ * (each uses the current step, then increments it); _train_backward replays the masks of the last forward.  p = 0 turns
+ * dropout off (bit-identical to never setting it); p outside [0, 1) or step < 0 returns GITB200_ERR_INVALID and changes
+ * nothing.  _train_get_dropout reads (p, seed, step); any output pointer may be NULL.  Inference entry points never apply it.
  *   _set_training(1) before the weights are loaded keeps their fp32 values for the master copy;
  *   _train_forward: tokens_dev int32 [B, L], memory_dev fp32 [B, M, d_model], teacher_logits_dev fp32 [B*L, ld_teacher]
  *                   -> loss_dev fp32 [3] = (total, KL, CE); activations are kept for the backward pass;
@@ -345,6 +356,8 @@ int gitb200_student_logits_ld(const gitb200_student* s); /* vocabulary rounded u
 int gitb200_student_set_training(gitb200_student* s, int enable);
 long long gitb200_student_train_begin(gitb200_student* s, float lr, float beta1, float beta2, float eps);
 long long gitb200_student_train_head_floats(const gitb200_student* s);
+int gitb200_student_train_set_dropout(gitb200_student* s, float p, uint64_t seed, long long step);
+int gitb200_student_train_get_dropout(const gitb200_student* s, float* p, uint64_t* seed, long long* step);
 int gitb200_student_train_forward(gitb200_student* s, const int32_t* tokens_dev, const float* memory_dev, const float* teacher_logits_dev,
                                   int ld_teacher, int B, int L, int M, float temperature, float* loss_dev, void* stream);
 int gitb200_student_train_backward(gitb200_student* s, int phase, float* grads_dev, float* d_memory_dev, void* stream);

@@ -68,6 +68,8 @@ SIGNATURES = {
     "gitb200_student_set_training": (c_int, [c_void_p, c_int]),
     "gitb200_student_train_begin": (c_longlong, [c_void_p, c_float, c_float, c_float, c_float]),
     "gitb200_student_train_head_floats": (c_longlong, [c_void_p]),
+    "gitb200_student_train_set_dropout": (c_int, [c_void_p, c_float, c_uint64, c_longlong]),
+    "gitb200_student_train_get_dropout": (c_int, [c_void_p, c_void_p, c_void_p, c_void_p]),
     "gitb200_student_train_forward": (c_int, [c_void_p, c_void_p, c_void_p, c_void_p, c_int, c_int, c_int, c_int, c_float, c_void_p, c_void_p]),
     "gitb200_student_train_backward": (c_int, [c_void_p, c_int, c_void_p, c_void_p, c_void_p]),
     "gitb200_student_train_apply": (c_int, [c_void_p, c_void_p, c_float, c_void_p]),

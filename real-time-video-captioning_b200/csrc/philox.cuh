@@ -44,3 +44,17 @@ PHILOX_HD double philox_uniform(uint32_t x) { return ((double)(x >> 8) + 0.5) * 
 
 // The Gumbel term of the exponential race, -log(-log u), in double: finite for every u above (from -2.85 to 17.33).
 PHILOX_HD float philox_gumbel(uint32_t x) { return (float)-log(-log(philox_uniform(x))); }
+
+// Dropout mask of the student's distillation step (csrc/student_train.cu; restated in tests/student_dropout_ref.py).  Element
+// idx of site `site` at dropout step `step` (mod 2^32) is kept iff philox_uniform(w) >= p in double, w = word idx % 4 of
+// Philox4x32-10(counter (idx / 4, step, site, 0x44524F50 "DROP"), key = (seed low 32 bits, seed high 32 bits)); a kept element
+// is scaled by 1 / (1 - p) in fp32 (inv_keep), a dropped one is 0.
+constexpr uint32_t DROPOUT_TAG = 0x44524F50u;
+PHILOX_HD Philox4 dropout_words(uint64_t seed, uint32_t step, uint32_t site, uint32_t idx) {
+  return philox4x32_10(idx >> 2, step, site, DROPOUT_TAG, (uint32_t)seed, (uint32_t)(seed >> 32));
+}
+PHILOX_HD float dropout_keep(uint32_t word, float p, float inv_keep) { return philox_uniform(word) >= (double)p ? inv_keep : 0.f; }
+// one element: 0 or inv_keep = 1 / (1 - p)
+PHILOX_HD float dropout_scale(uint64_t seed, uint32_t step, uint32_t site, uint32_t idx, float p, float inv_keep) {
+  return dropout_keep(dropout_words(seed, step, site, idx).x[idx & 3], p, inv_keep);
+}

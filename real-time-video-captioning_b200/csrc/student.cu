@@ -71,11 +71,14 @@ __global__ void student_ln_kernel(const bf16* __restrict__ x, int ldx, int rows,
 //   q row r at q[r * ldq + h * hd]; key / value j of batch b at kv[(b * kv_rows + j) * ldkv + {k_off, v_off} + h * hd]
 //   causal != 0: keys 0 .. pos0 + (r % Lq) (the query's own position included); else all n_keys
 //   tokens != nullptr: key j is masked when tokens[b * tok_ld + j] == pad (tgt_key_padding_mask, masking.py:14)
+//   DROP (distillation step only): out = (D o P) v with D the dropout mask of site dr over the element index
+//   ((b * gridDim.y + h) * Lq + i) * n_keys + j; the softmax sum is over the undropped probabilities
 constexpr int S_MAX_KEYS = 128, S_MAX_HD = 128;
+template <bool DROP>
 __global__ void __launch_bounds__(32) student_attn_kernel(const bf16* __restrict__ q, int ldq, int Lq, int pos0,
                                                           const bf16* __restrict__ kv, int kv_rows, int ldkv, int k_off, int v_off,
                                                           int n_keys, int causal, const int* __restrict__ tokens, int tok_ld, int pad,
-                                                          int hd, float scale, bf16* __restrict__ out, int ldo) {
+                                                          int hd, float scale, bf16* __restrict__ out, int ldo, SDrop dr) {
   __shared__ float sq[S_MAX_HD];
   __shared__ float sp[S_MAX_KEYS];
   const int r = blockIdx.x, h = blockIdx.y, lane = threadIdx.x;
@@ -100,8 +103,11 @@ __global__ void __launch_bounds__(32) student_attn_kernel(const bf16* __restrict
   float sum = 0.f;
   for (int j = lane; j < nk; j += 32) {
     const float p = __expf(sp[j] - mx);
-    sp[j] = p;
     sum += p;
+    if constexpr (DROP)
+      sp[j] = p * dropout_scale(dr.seed, dr.step, dr.site, (unsigned)(((b * gridDim.y + h) * Lq + i) * n_keys + j), dr.p, dr.inv_keep);
+    else
+      sp[j] = p;
   }
   sum = warp_sum(sum);
   __syncwarp();
@@ -206,8 +212,18 @@ int s_embed(gitb200_student* c, const int* tokens, int tok_ld, int L, int pos0, 
 int s_attn(gitb200_student* c, const bf16* q, int ldq, int Lq, int pos0, const bf16* kv, int kv_rows, int ldkv, int k_off, int v_off,
            int n_keys, int causal, const int* tokens, int tok_ld, int rows, bf16* out, int ldo, cudaStream_t s) {
   if (n_keys < 1 || n_keys > S_MAX_KEYS) return sfail(c, GITB200_ERR_INVALID, "student attention over %d keys (1 .. %d)", n_keys, S_MAX_KEYS);
-  student_attn_kernel<<<dim3(rows, c->cfg.n_head), 32, 0, s>>>(q, ldq, Lq, pos0, kv, kv_rows, ldkv, k_off, v_off, n_keys, causal, tokens,
-                                                               tok_ld, c->cfg.pad, c->hd, 1.0f / sqrtf((float)c->hd), out, ldo);
+  student_attn_kernel<false><<<dim3(rows, c->cfg.n_head), 32, 0, s>>>(q, ldq, Lq, pos0, kv, kv_rows, ldkv, k_off, v_off, n_keys, causal,
+                                                                      tokens, tok_ld, c->cfg.pad, c->hd, 1.0f / sqrtf((float)c->hd), out, ldo,
+                                                                      SDrop{});
+  note_launch();
+  S_CUDA_OK(c, cudaGetLastError());
+  return 0;
+}
+int s_attn_dropout(gitb200_student* c, const bf16* q, int ldq, int Lq, const bf16* kv, int kv_rows, int ldkv, int k_off, int v_off,
+                   int n_keys, int causal, const int* tokens, int tok_ld, int rows, bf16* out, int ldo, const SDrop& dr, cudaStream_t s) {
+  if (n_keys < 1 || n_keys > S_MAX_KEYS) return sfail(c, GITB200_ERR_INVALID, "student attention over %d keys (1 .. %d)", n_keys, S_MAX_KEYS);
+  student_attn_kernel<true><<<dim3(rows, c->cfg.n_head), 32, 0, s>>>(q, ldq, Lq, 0, kv, kv_rows, ldkv, k_off, v_off, n_keys, causal, tokens,
+                                                                     tok_ld, c->cfg.pad, c->hd, 1.0f / sqrtf((float)c->hd), out, ldo, dr);
   note_launch();
   S_CUDA_OK(c, cudaGetLastError());
   return 0;

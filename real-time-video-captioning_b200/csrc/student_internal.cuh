@@ -12,6 +12,7 @@
 #include "../../include/gitb200.h"
 #include "common.cuh"
 #include "kernels.h"
+#include "philox.cuh"
 #include "student_ops.h"
 
 namespace sdet {

@@ -9,6 +9,15 @@ struct gitb200_student;
 
 namespace sdet {
 
+// One dropout site of the distillation step (mask: philox.cuh, dropout_scale): key `seed`, counter word `step` (the dropout
+// step, mod 2^32) and `site` = 6 * layer + k; p in (0, 1), inv_keep = 1 / (1 - p) in fp32.
+struct SDrop {
+  unsigned long long seed;
+  unsigned step;
+  unsigned site;
+  float p, inv_keep;
+};
+
 // ---- forward (student.cu)
 // out = A W^T + bias (+ residual), act; bf16 out and / or fp32 out32 (gemm_bf16)
 int s_gemm(gitb200_student* c, const bf16* A, int lda, const bf16* W, int K, int M, int N, const float* bias, const bf16* residual,
@@ -22,6 +31,10 @@ int s_embed(gitb200_student* c, const int* tokens, int tok_ld, int L, int pos0, 
 // 0 .. pos0 + r % Lq; tokens != nullptr: key j of sequence b masked when tokens[b * tok_ld + j] == cfg.pad.  n_keys <= 128.
 int s_attn(gitb200_student* c, const bf16* q, int ldq, int Lq, int pos0, const bf16* kv, int kv_rows, int ldkv, int k_off, int v_off,
            int n_keys, int causal, const int* tokens, int tok_ld, int rows, bf16* out, int ldo, cudaStream_t s);
+// s_attn with dropout on the probabilities (distillation step only): out = (D o P) V, D the mask of site dr over the element
+// index ((b * H + h) * Lq + i) * n_keys + j, b = r / Lq, i = r % Lq.  pos0 = 0.
+int s_attn_dropout(gitb200_student* c, const bf16* q, int ldq, int Lq, const bf16* kv, int kv_rows, int ldkv, int k_off, int v_off,
+                   int n_keys, int causal, const int* tokens, int tok_ld, int rows, bf16* out, int ldo, const SDrop& dr, cudaStream_t s);
 
 // ---- distillation backward (student_train.cu)
 // dst[c * R_pad + r] = src[r * ld_src + c] for r < R, c < C; zero for R <= r < R_pad or C <= c < C_pad
@@ -49,6 +62,23 @@ int t_distill_loss(gitb200_student* c, const float* s_logits, int ld_s, const fl
                    float temperature, int* n_valid, bf16* dlogits, float* loss, float* loss_out, cudaStream_t s);
 // dh[i] = 0 where !(h[i] > 0), i < n
 int t_relu_bwd(gitb200_student* c, const bf16* h, bf16* dh, size_t n, cudaStream_t s);
+// ---- dropout sites of the distillation step (student_train.cu); element index r * cols + c over the logical columns
+// y = x + D o z (bf16, kept for the LayerNorm backward) and out = LN(y) * g + b over d_model columns (leading dimension dp),
+// one warp per row; D = mask of site dr
+int t_dropout_add_ln(gitb200_student* c, const bf16* x, const bf16* z, int rows, const float* g, const float* b, bf16* y, bf16* out,
+                     const SDrop& dr, cudaStream_t s);
+// h[r, c] *= D[r, c] in place for r < rows, c < cols (cols % 4 == 0), leading dimension ld
+int t_dropout_inplace(gitb200_student* c, bf16* h, int ld, int rows, int cols, const SDrop& dr, cudaStream_t s);
+// t_ln_bwd with a second output dz = D o dy (bf16 of the rounded dy), D = mask of site dr
+int t_ln_bwd_dropout(gitb200_student* c, const bf16* y, const bf16* dx, int rows, const float* gamma, bf16* dy, bf16* dz, float* dgamma,
+                     float* dbeta, float* stats, const SDrop& dr, cudaStream_t s);
+// t_attn_bwd for out = (D o P) V: dV = (D o P)^T dO, dP = D o (dO V^T), dS = P o (dP - rowsum(P o dP)); D over the element
+// index ((b * H + h) * Lq + i) * n_keys + j
+int t_attn_bwd_dropout(gitb200_student* c, const bf16* q, int ldq, int Lq, const bf16* kv, int kv_rows, int ldkv, int k_off, int v_off,
+                       int n_keys, int causal, const int* tokens, int tok_ld, int B, const bf16* dO, bf16* dq, int lddq, bf16* dkv, int lddkv,
+                       int dk_off, int dv_off, const SDrop& dr, cudaStream_t s);
+// ReLU backward through h' = D o relu(.): dh[i] = h'[i] > 0 ? dh[i] * inv_keep : 0, i < n (exact: where D = 0, h' = 0)
+int t_relu_bwd_dropout(gitb200_student* c, const bf16* h, bf16* dh, size_t n, float inv_keep, cudaStream_t s);
 // dembed[tok, :] = sum over the rows r with tokens[r] == tok (clamped to [0, vocab)), in row order, of dx[r, :d] / sqrt(d);
 // rows of tokens that do not occur are left untouched
 int t_embed_bwd(gitb200_student* c, const int* tokens, int rows, const bf16* dx, int ld, float* dembed, cudaStream_t s);

@@ -16,7 +16,9 @@
 // Every contraction -- forward, dX = dY W and dW = dY^T X -- runs on the tcgen05 GEMM of the inference path (C = A W^T with
 // both operands K-major): dX uses a transposed bf16 copy of W kept next to W, dW uses explicit bf16 transposes of the two
 // (small: B*L = 160 rows) activation matrices.  Activations and activation gradients are bf16, weight gradients fp32.
-// Dropout (0.3 in config.py:83) is not applied: the parity oracle is torch.autograd on the same modules with dropout off.
+// Dropout (nn.TransformerDecoderLayer's six sites per layer, p = 0.3 in config.py:83) is opt-in: gitb200_student_train_set_dropout
+// gives p and a Philox seed.  The masks are regenerated in the backward pass, never stored (mask: philox.cuh, dropout_scale);
+// where dropout is on, the three residual sites' GEMMs write z without the residual and dropout_add_ln_kernel forms x + D o z.
 #include "student_internal.cuh"
 
 using namespace sdet;
@@ -53,6 +55,12 @@ struct STrain {
   bf16* wt_vocab = nullptr;
   std::vector<LayerAct> acts;
   SBuf<bf16> xo, mem, dlogits, tA, tB, dx, dy, da, dqkv, dh, dmemkv, dmem;
+  SBuf<bf16> z, dz;  // dropout only: the residual sites' dropped addend (forward scratch) and its gradient D o dy
+  // dropout (off while drop_p == 0): drop_step counts the forwards that applied it; the backward pass replays fwd_step's masks
+  float drop_p = 0.f;
+  unsigned long long drop_seed = 0;
+  long long drop_step = 0, fwd_step = 0;
+  bool fwd_drop = false;
   SBuf<float> logits, stats, loss;
   SBuf<int> nvalid, toks;
   int B = 0, L = 0, M = 0;
@@ -170,8 +178,11 @@ __global__ void __launch_bounds__(256) distill_loss_kernel(const float* __restri
 
 // LayerNorm backward, one warp per row: y = LN input (pre-norm), dx = gradient of the LN output.
 //   dy = rstd * (g - mean(g) - xhat * mean(g * xhat)),  g = dx * gamma;  stats[r] = (mean, rstd) for the parameter-gradient kernel
+//   DROP: also dz = D o dy (D = dropout mask of `site`, element index warp * cols + c): the gradient of the dropped addend
+template <bool DROP>
 __global__ void ln_bwd_kernel(const bf16* __restrict__ y, const bf16* __restrict__ dx, int ld, int rows, int cols,
-                              const float* __restrict__ gamma, float eps, bf16* __restrict__ dy, float* __restrict__ stats) {
+                              const float* __restrict__ gamma, float eps, bf16* __restrict__ dy, float* __restrict__ stats,
+                              bf16* __restrict__ dz, SDrop site) {
   const int warp = (blockIdx.x * blockDim.x + threadIdx.x) >> 5, lane = threadIdx.x & 31;
   if (warp >= rows) return;
   const bf16* yr = y + (size_t)warp * ld;
@@ -194,7 +205,11 @@ __global__ void ln_bwd_kernel(const bf16* __restrict__ y, const bf16* __restrict
   const float c1 = warp_sum(s1) / (float)cols, c2 = warp_sum(s2) / (float)cols;
   for (int c = lane; c < cols; c += 32) {
     const float xh = (__bfloat162float(yr[c]) - mean) * rstd, g = __bfloat162float(dr[c]) * gamma[c];
-    dy[(size_t)warp * ld + c] = __float2bfloat16(rstd * (g - c1 - xh * c2));
+    const bf16 v = __float2bfloat16(rstd * (g - c1 - xh * c2));
+    dy[(size_t)warp * ld + c] = v;
+    if constexpr (DROP)
+      dz[(size_t)warp * ld + c] =
+          __float2bfloat16(__bfloat162float(v) * dropout_scale(site.seed, site.step, site.site, (unsigned)(warp * cols + c), site.p, site.inv_keep));
   }
   if (lane == 0) {
     stats[2 * warp] = mean;
@@ -221,16 +236,63 @@ __global__ void relu_bwd_kernel(const bf16* __restrict__ h, bf16* __restrict__ d
   const size_t i = (size_t)blockIdx.x * blockDim.x + threadIdx.x;
   if (i < n && !(__bfloat162float(h[i]) > 0.f)) dh[i] = __float2bfloat16(0.f);
 }
+// dh[r, c] = h'[r, c] > 0 ? dh[r, c] * inv_keep : 0   (h' = D o relu(.), the stored post-dropout activation)
+__global__ void relu_bwd_dropout_kernel(const bf16* __restrict__ h, bf16* __restrict__ dh, size_t n, float inv_keep) {
+  const size_t i = (size_t)blockIdx.x * blockDim.x + threadIdx.x;
+  if (i < n) dh[i] = __bfloat162float(h[i]) > 0.f ? __float2bfloat16(__bfloat162float(dh[i]) * inv_keep) : __float2bfloat16(0.f);
+}
+
+// h[r, c] *= D[r, c] for c < cols (cols % 4 == 0): one thread per 4 consecutive elements, one Philox call each
+__global__ void dropout_inplace_kernel(bf16* __restrict__ h, int ld, int rows, int cols, SDrop dr) {
+  const size_t g = (size_t)blockIdx.x * blockDim.x + threadIdx.x, quads = (size_t)rows * (cols >> 2);
+  if (g >= quads) return;
+  const unsigned idx = (unsigned)(g * 4);
+  const int r = (int)(idx / cols), c = (int)(idx % cols);
+  const Philox4 w = dropout_words(dr.seed, dr.step, dr.site, idx);
+  bf16* p = h + (size_t)r * ld + c;
+  for (int k = 0; k < 4; ++k) p[k] = __float2bfloat16(__bfloat162float(p[k]) * dropout_keep(w.x[k], dr.p, dr.inv_keep));
+}
+
+// y = x + D o z (bf16), out = LN(y) * gamma + beta over `cols` columns (cols % 4 == 0); one warp per row, each lane owns
+// groups of 4 consecutive columns (one Philox call each).  The statistics are those of student_ln_kernel on the stored y.
+__global__ void dropout_add_ln_kernel(const bf16* __restrict__ x, const bf16* __restrict__ z, int ld, int rows, int cols,
+                                      const float* __restrict__ gamma, const float* __restrict__ beta, float eps, bf16* __restrict__ y,
+                                      bf16* __restrict__ out, SDrop dr) {
+  const int warp = (blockIdx.x * blockDim.x + threadIdx.x) >> 5, lane = threadIdx.x & 31;
+  if (warp >= rows) return;
+  const size_t row = (size_t)warp * ld;
+  for (int c = 4 * lane; c < cols; c += 128) {
+    const Philox4 w = dropout_words(dr.seed, dr.step, dr.site, (unsigned)(warp * cols + c));
+    for (int k = 0; k < 4; ++k)
+      y[row + c + k] = __float2bfloat16(__bfloat162float(x[row + c + k]) +
+                                        __bfloat162float(z[row + c + k]) * dropout_keep(w.x[k], dr.p, dr.inv_keep));
+  }
+  __syncwarp();
+  const bf16* yr = y + row;
+  float s = 0.f;
+  for (int c = lane; c < cols; c += 32) s += __bfloat162float(yr[c]);
+  const float mean = warp_sum(s) / (float)cols;
+  float q = 0.f;
+  for (int c = lane; c < cols; c += 32) {
+    const float v = __bfloat162float(yr[c]) - mean;
+    q += v * v;
+  }
+  const float rstd = rsqrtf(warp_sum(q) / (float)cols + eps);
+  for (int c = lane; c < cols; c += 32) out[row + c] = __float2bfloat16((__bfloat162float(yr[c]) - mean) * rstd * gamma[c] + beta[c]);
+}
 
 // Attention backward for one (sequence b, head h): recomputes P = softmax(scale Q K^T + mask) and returns dQ, dK, dV.
 //   q row (b * Lq + i) at q[.. * ldq + h * hd]; key / value j at kv[(b * kv_rows + j) * ldkv + {k_off, v_off} + h * hd]
 //   dO like the forward output; dq like q (leading dimension lddq); dk / dv like k / v in dkv (lddkv, dk_off, dv_off)
 //   causal: key j visible to query i iff j <= i; tokens != nullptr: key j masked when tokens[b * tok_ld + j] == pad
+//   DROP: the forward was (D o P) V, D the dropout mask of site dr over ((b * H + h) * Lq + i) * n_keys + j (kept in shared
+//   memory): dV = (D o P)^T dO, dP = D o (dO V^T), dS = P o (dP - rowsum(P o dP)) with P the undropped probabilities
+template <bool DROP>
 __global__ void __launch_bounds__(128) attn_bwd_kernel(const bf16* __restrict__ q, int ldq, int Lq, const bf16* __restrict__ kv, int kv_rows,
                                                        int ldkv, int k_off, int v_off, int n_keys, int causal,
                                                        const int* __restrict__ tokens, int tok_ld, int pad, int hd, float scale,
                                                        const bf16* __restrict__ dO, int lddo, bf16* __restrict__ dq, int lddq,
-                                                       bf16* __restrict__ dkv, int lddkv, int dk_off, int dv_off) {
+                                                       bf16* __restrict__ dkv, int lddkv, int dk_off, int dv_off, SDrop dr) {
   extern __shared__ float sm[];
   const int b = blockIdx.x, h = blockIdx.y, tid = threadIdx.x, nt = blockDim.x;
   const int hs = hd + 1, ps = n_keys + 1;
@@ -240,6 +302,7 @@ __global__ void __launch_bounds__(128) attn_bwd_kernel(const bf16* __restrict__ 
   float* G = Vv + n_keys * hs;      // [Lq][hs]   dO
   float* P = G + Lq * hs;           // [Lq][ps]
   float* S = P + Lq * ps;           // [Lq][ps]   dP, then dS
+  float* D = S + Lq * ps;           // [Lq][ps]   dropout scales (DROP only)
   for (int e = tid; e < Lq * hd; e += nt) {
     const int i = e / hd, c = e % hd;
     Q[i * hs + c] = __bfloat162float(q[(size_t)(b * Lq + i) * ldq + h * hd + c]);
@@ -261,7 +324,13 @@ __global__ void __launch_bounds__(128) attn_bwd_kernel(const bf16* __restrict__ 
     }
     const bool masked = (causal && j > i) || (tokens != nullptr && tokens[(size_t)b * tok_ld + j] == pad);
     P[i * ps + j] = masked ? -INFINITY : s * scale;
-    S[i * ps + j] = g;  // dP
+    if constexpr (DROP) {
+      const float m = dropout_scale(dr.seed, dr.step, dr.site, (unsigned)(((b * gridDim.y + h) * Lq + i) * n_keys + j), dr.p, dr.inv_keep);
+      D[i * ps + j] = m;
+      S[i * ps + j] = g * m;  // dP of the undropped probabilities
+    } else {
+      S[i * ps + j] = g;  // dP
+    }
   }
   __syncthreads();
   for (int i = tid; i < Lq; i += nt) {
@@ -294,7 +363,7 @@ __global__ void __launch_bounds__(128) attn_bwd_kernel(const bf16* __restrict__ 
     float dk = 0.f, dv = 0.f;
     for (int i = 0; i < Lq; ++i) {
       dk = fmaf(S[i * ps + j], Q[i * hs + c], dk);
-      dv = fmaf(P[i * ps + j], G[i * hs + c], dv);
+      dv = fmaf(DROP ? P[i * ps + j] * D[i * ps + j] : P[i * ps + j], G[i * hs + c], dv);
     }
     bf16* row = dkv + (size_t)(b * kv_rows + j) * lddkv + h * hd + c;
     row[dk_off] = __float2bfloat16(dk * scale);
@@ -410,31 +479,72 @@ int t_weight_grad(gitb200_student* c, const bf16* dY, int ldy, int n_pad, const 
   return s_gemm(c, tA, Rp, tB, Rp, n_pad, k_pad, nullptr, nullptr, 0, ACT_NONE, nullptr, 0, dW, k_pad, s);
 }
 
-int t_ln_bwd(gitb200_student* c, const bf16* y, const bf16* dx, int rows, const float* gamma, bf16* dy, float* dgamma, float* dbeta,
-             float* stats, cudaStream_t s) {
+template <bool DROP>
+static int ln_bwd_launch(gitb200_student* c, const bf16* y, const bf16* dx, int rows, const float* gamma, bf16* dy, bf16* dz, float* dgamma,
+                         float* dbeta, float* stats, const SDrop& dr, cudaStream_t s) {
   const int d = c->cfg.d_model, dp = c->dp;
-  ln_bwd_kernel<<<(rows * 32 + 255) / 256, 256, 0, s>>>(y, dx, dp, rows, d, gamma, c->cfg.ln_eps, dy, stats);
+  ln_bwd_kernel<DROP><<<(rows * 32 + 255) / 256, 256, 0, s>>>(y, dx, dp, rows, d, gamma, c->cfg.ln_eps, dy, stats, dz, dr);
   ln_param_grad_kernel<<<(d + 127) / 128, 128, 0, s>>>(y, dx, dp, rows, d, stats, dgamma, dbeta);
   note_launch(2);
   S_CUDA_OK(c, cudaGetLastError());
   return 0;
 }
+int t_ln_bwd(gitb200_student* c, const bf16* y, const bf16* dx, int rows, const float* gamma, bf16* dy, float* dgamma, float* dbeta,
+             float* stats, cudaStream_t s) {
+  return ln_bwd_launch<false>(c, y, dx, rows, gamma, dy, nullptr, dgamma, dbeta, stats, SDrop{}, s);
+}
+int t_ln_bwd_dropout(gitb200_student* c, const bf16* y, const bf16* dx, int rows, const float* gamma, bf16* dy, bf16* dz, float* dgamma,
+                     float* dbeta, float* stats, const SDrop& dr, cudaStream_t s) {
+  return ln_bwd_launch<true>(c, y, dx, rows, gamma, dy, dz, dgamma, dbeta, stats, dr, s);
+}
 
-int t_attn_bwd(gitb200_student* c, const bf16* q, int ldq, int Lq, const bf16* kv, int kv_rows, int ldkv, int k_off, int v_off, int n_keys,
-               int causal, const int* tokens, int tok_ld, int B, const bf16* dO, bf16* dq, int lddq, bf16* dkv, int lddkv, int dk_off,
-               int dv_off, cudaStream_t s) {
+template <bool DROP>
+static int attn_bwd_launch(gitb200_student* c, const bf16* q, int ldq, int Lq, const bf16* kv, int kv_rows, int ldkv, int k_off, int v_off,
+                           int n_keys, int causal, const int* tokens, int tok_ld, int B, const bf16* dO, bf16* dq, int lddq, bf16* dkv,
+                           int lddkv, int dk_off, int dv_off, const SDrop& dr, cudaStream_t s) {
   if (Lq < 1 || Lq > T_MAX_SEQ || n_keys < 1 || n_keys > T_MAX_SEQ)
     return sfail(c, GITB200_ERR_INVALID, "attention backward over %d queries x %d keys (1 .. %d each)", Lq, n_keys, T_MAX_SEQ);
   const int hd = c->hd;
-  const size_t smem = ((size_t)(2 * Lq + 2 * n_keys) * (hd + 1) + (size_t)2 * Lq * (n_keys + 1)) * sizeof(float);
-  static size_t attr = 0;  // process-wide, not per device: one process trains on one GPU (dist.py)
+  const size_t smem = ((size_t)(2 * Lq + 2 * n_keys) * (hd + 1) + (size_t)(DROP ? 3 : 2) * Lq * (n_keys + 1)) * sizeof(float);
+  static size_t attr = 0;  // per instantiation, process-wide, not per device: one process trains on one GPU (dist.py)
   if (smem > 48 * 1024 && smem > attr) {
-    S_CUDA_OK(c, cudaFuncSetAttribute(attn_bwd_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
+    S_CUDA_OK(c, cudaFuncSetAttribute(attn_bwd_kernel<DROP>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
     attr = smem;
   }
-  attn_bwd_kernel<<<dim3(B, c->cfg.n_head), 128, smem, s>>>(q, ldq, Lq, kv, kv_rows, ldkv, k_off, v_off, n_keys, causal, tokens, tok_ld,
-                                                            c->cfg.pad, hd, 1.0f / sqrtf((float)hd), dO, c->dp, dq, lddq, dkv, lddkv, dk_off,
-                                                            dv_off);
+  attn_bwd_kernel<DROP><<<dim3(B, c->cfg.n_head), 128, smem, s>>>(q, ldq, Lq, kv, kv_rows, ldkv, k_off, v_off, n_keys, causal, tokens,
+                                                                  tok_ld, c->cfg.pad, hd, 1.0f / sqrtf((float)hd), dO, c->dp, dq, lddq, dkv,
+                                                                  lddkv, dk_off, dv_off, dr);
+  note_launch();
+  S_CUDA_OK(c, cudaGetLastError());
+  return 0;
+}
+int t_attn_bwd(gitb200_student* c, const bf16* q, int ldq, int Lq, const bf16* kv, int kv_rows, int ldkv, int k_off, int v_off, int n_keys,
+               int causal, const int* tokens, int tok_ld, int B, const bf16* dO, bf16* dq, int lddq, bf16* dkv, int lddkv, int dk_off,
+               int dv_off, cudaStream_t s) {
+  return attn_bwd_launch<false>(c, q, ldq, Lq, kv, kv_rows, ldkv, k_off, v_off, n_keys, causal, tokens, tok_ld, B, dO, dq, lddq, dkv, lddkv,
+                                dk_off, dv_off, SDrop{}, s);
+}
+int t_attn_bwd_dropout(gitb200_student* c, const bf16* q, int ldq, int Lq, const bf16* kv, int kv_rows, int ldkv, int k_off, int v_off,
+                       int n_keys, int causal, const int* tokens, int tok_ld, int B, const bf16* dO, bf16* dq, int lddq, bf16* dkv, int lddkv,
+                       int dk_off, int dv_off, const SDrop& dr, cudaStream_t s) {
+  return attn_bwd_launch<true>(c, q, ldq, Lq, kv, kv_rows, ldkv, k_off, v_off, n_keys, causal, tokens, tok_ld, B, dO, dq, lddq, dkv, lddkv,
+                               dk_off, dv_off, dr, s);
+}
+
+int t_dropout_add_ln(gitb200_student* c, const bf16* x, const bf16* z, int rows, const float* g, const float* b, bf16* y, bf16* out,
+                     const SDrop& dr, cudaStream_t s) {
+  const int d = c->cfg.d_model;
+  if (d % 4 != 0) return sfail(c, GITB200_ERR_INVALID, "dropout-add-LayerNorm needs d_model %% 4 == 0, not %d", d);
+  dropout_add_ln_kernel<<<(rows * 32 + 255) / 256, 256, 0, s>>>(x, z, c->dp, rows, d, g, b, c->cfg.ln_eps, y, out, dr);
+  note_launch();
+  S_CUDA_OK(c, cudaGetLastError());
+  return 0;
+}
+
+int t_dropout_inplace(gitb200_student* c, bf16* h, int ld, int rows, int cols, const SDrop& dr, cudaStream_t s) {
+  if (cols % 4 != 0) return sfail(c, GITB200_ERR_INVALID, "dropout over %d columns (a multiple of 4)", cols);
+  const size_t quads = (size_t)rows * (cols / 4);
+  dropout_inplace_kernel<<<(unsigned)((quads + 255) / 256), 256, 0, s>>>(h, ld, rows, cols, dr);
   note_launch();
   S_CUDA_OK(c, cudaGetLastError());
   return 0;
@@ -455,6 +565,13 @@ int t_distill_loss(gitb200_student* c, const float* s_logits, int ld_s, const fl
 
 int t_relu_bwd(gitb200_student* c, const bf16* h, bf16* dh, size_t n, cudaStream_t s) {
   relu_bwd_kernel<<<(unsigned)((n + 255) / 256), 256, 0, s>>>(h, dh, n);
+  note_launch();
+  S_CUDA_OK(c, cudaGetLastError());
+  return 0;
+}
+
+int t_relu_bwd_dropout(gitb200_student* c, const bf16* h, bf16* dh, size_t n, float inv_keep, cudaStream_t s) {
+  relu_bwd_dropout_kernel<<<(unsigned)((n + 255) / 256), 256, 0, s>>>(h, dh, n, inv_keep);
   note_launch();
   S_CUDA_OK(c, cudaGetLastError());
   return 0;
@@ -512,7 +629,8 @@ void student_train_destroy(gitb200_student* c) {
   cudaFree(t->M2);
   for (auto& a : t->acts)
     for (auto* b : {&a.x0, &a.qkv, &a.a, &a.y1, &a.x1, &a.q2, &a.memkv, &a.a2, &a.y2, &a.x2, &a.h, &a.y3}) cudaFree(b->p);
-  for (auto* b : {&t->xo, &t->mem, &t->dlogits, &t->tA, &t->tB, &t->dx, &t->dy, &t->da, &t->dqkv, &t->dh, &t->dmemkv, &t->dmem}) cudaFree(b->p);
+  for (auto* b : {&t->xo, &t->mem, &t->dlogits, &t->tA, &t->tB, &t->dx, &t->dy, &t->da, &t->dqkv, &t->dh, &t->dmemkv, &t->dmem, &t->z, &t->dz})
+    cudaFree(b->p);
   cudaFree(t->logits.p);
   cudaFree(t->stats.p);
   cudaFree(t->loss.p);
@@ -662,6 +780,26 @@ long long gitb200_student_train_begin(gitb200_student* c, float lr, float beta1,
   return (long long)t->n_floats;
 }
 
+int gitb200_student_train_set_dropout(gitb200_student* c, float p, uint64_t seed, long long step) {
+  if (!c) return GITB200_ERR_INVALID;
+  if (!(p >= 0.f && p < 1.f) || step < 0)
+    return sfail(c, GITB200_ERR_INVALID, "dropout p must lie in [0, 1) and the step be >= 0 (got p = %g, step = %lld)", (double)p, step);
+  STrain* t = c->train;
+  if (!t) return sfail(c, GITB200_ERR_STATE, "call gitb200_student_train_begin first");
+  t->drop_p = p;
+  t->drop_seed = seed;
+  t->drop_step = step;
+  return GITB200_OK;
+}
+
+int gitb200_student_train_get_dropout(const gitb200_student* c, float* p, uint64_t* seed, long long* step) {
+  if (!c || !c->train) return GITB200_ERR_STATE;
+  if (p) *p = c->train->drop_p;
+  if (seed) *seed = c->train->drop_seed;
+  if (step) *step = c->train->drop_step;
+  return GITB200_OK;
+}
+
 long long gitb200_student_train_head_floats(const gitb200_student* c) { return (c && c->train) ? (long long)c->train->head_floats : -1; }
 
 // Forward with stored activations + loss + d loss / d logits.  tokens int32 [B, L]; memory fp32 [B, M, d_model]; teacher_logits fp32
@@ -710,6 +848,12 @@ int gitb200_student_train_forward(gitb200_student* c, const int32_t* tokens, con
   S_TRY(sensure(c, t->loss, (size_t)2 * R));
   S_TRY(sensure(c, t->nvalid, 1));
   S_TRY(sensure(c, t->toks, (size_t)R));
+  const bool drop = t->drop_p > 0.f;
+  if (drop) {
+    S_TRY(sensure(c, t->z, (size_t)R * dp));
+    S_TRY(sensure(c, t->dz, (size_t)R * dp));
+  }
+  auto site = [&](int l, int k) { return SDrop{t->drop_seed, (unsigned)t->drop_step, (unsigned)(6 * l + k), t->drop_p, 1.f / (1.f - t->drop_p)}; };
   S_CUDA_OK(c, cudaMemcpyAsync(t->toks.p, tokens, (size_t)R * sizeof(int), cudaMemcpyDeviceToDevice, s));  // the backward pass reads them again
   S_CUDA_OK(c, cast_f32_to_bf16(memory, Rm, d, d, t->mem.p, d, Rm, d, s));
   S_TRY(s_embed(c, t->toks.p, L, L, 0, R, t->acts[0].x0.p, s));
@@ -718,6 +862,21 @@ int gitb200_student_train_forward(gitb200_student* c, const int32_t* tokens, con
     LayerAct& A = t->acts[l];
     bf16* x3 = (l + 1 < k.n_layers) ? t->acts[l + 1].x0.p : t->xo.p;
     S_TRY(s_gemm(c, A.x0.p, dp, W.w_sa_in, d, R, 3 * dp, W.b_sa_in, nullptr, 0, ACT_NONE, A.qkv.p, 3 * dp, nullptr, 0, s));
+    if (drop) {  // the six sites of nn.TransformerDecoderLayer, in its call order: site 6 l + k
+      S_TRY(s_attn_dropout(c, A.qkv.p, 3 * dp, L, A.qkv.p, L, 3 * dp, dp, 2 * dp, L, 1, t->toks.p, L, R, A.a.p, dp, site(l, 0), s));
+      S_TRY(s_gemm(c, A.a.p, dp, W.w_sa_out, d, R, dp, W.b_sa_out, nullptr, 0, ACT_NONE, t->z.p, dp, nullptr, 0, s));
+      S_TRY(t_dropout_add_ln(c, A.x0.p, t->z.p, R, W.n1_g, W.n1_b, A.y1.p, A.x1.p, site(l, 1), s));
+      S_TRY(s_gemm(c, A.x1.p, dp, W.w_ca_q, d, R, dp, W.b_ca_q, nullptr, 0, ACT_NONE, A.q2.p, dp, nullptr, 0, s));
+      S_TRY(s_gemm(c, t->mem.p, d, W.w_ca_kv, d, Rm, 2 * dp, W.b_ca_kv, nullptr, 0, ACT_NONE, A.memkv.p, 2 * dp, nullptr, 0, s));
+      S_TRY(s_attn_dropout(c, A.q2.p, dp, L, A.memkv.p, M, 2 * dp, 0, dp, M, 0, nullptr, 0, R, A.a2.p, dp, site(l, 2), s));
+      S_TRY(s_gemm(c, A.a2.p, dp, W.w_ca_out, d, R, dp, W.b_ca_out, nullptr, 0, ACT_NONE, t->z.p, dp, nullptr, 0, s));
+      S_TRY(t_dropout_add_ln(c, A.x1.p, t->z.p, R, W.n2_g, W.n2_b, A.y2.p, A.x2.p, site(l, 3), s));
+      S_TRY(s_gemm(c, A.x2.p, dp, W.w_ff1, d, R, fp, W.b_ff1, nullptr, 0, ACT_RELU, A.h.p, fp, nullptr, 0, s));
+      S_TRY(t_dropout_inplace(c, A.h.p, fp, R, k.d_ffn, site(l, 4), s));
+      S_TRY(s_gemm(c, A.h.p, fp, W.w_ff2, fp, R, dp, W.b_ff2, nullptr, 0, ACT_NONE, t->z.p, dp, nullptr, 0, s));
+      S_TRY(t_dropout_add_ln(c, A.x2.p, t->z.p, R, W.n3_g, W.n3_b, A.y3.p, x3, site(l, 5), s));
+      continue;
+    }
     S_TRY(s_attn(c, A.qkv.p, 3 * dp, L, 0, A.qkv.p, L, 3 * dp, dp, 2 * dp, L, 1, t->toks.p, L, R, A.a.p, dp, s));
     S_TRY(s_gemm(c, A.a.p, dp, W.w_sa_out, d, R, dp, W.b_sa_out, A.x0.p, dp, ACT_NONE, A.y1.p, dp, nullptr, 0, s));
     S_TRY(s_ln(c, A.y1.p, dp, R, W.n1_g, W.n1_b, A.x1.p, dp, s));
@@ -734,6 +893,9 @@ int gitb200_student_train_forward(gitb200_student* c, const int32_t* tokens, con
   S_TRY(t_distill_loss(c, t->logits.p, vp, teacher_logits, ld_teacher, t->toks.p, B, L, temperature, t->nvalid.p, t->dlogits.p, t->loss.p,
                        loss_out, s));
   t->B = B; t->L = L; t->M = M;
+  t->fwd_drop = drop;
+  t->fwd_step = t->drop_step;
+  if (drop) t->drop_step += 1;
   t->have_forward = true;
   t->have_head = false;
   return GITB200_OK;
@@ -763,26 +925,44 @@ int gitb200_student_train_backward(gitb200_student* c, int phase, float* grads, 
     PEntry* e = find_entry(t, "embed.weight");
     S_CUDA_OK(c, cudaMemsetAsync(grads + e->off, 0, (size_t)e->rows_pad * e->cols_pad * sizeof(float), s));
   }
+  // dropout: the residual sites' LayerNorm backward also gives dz = D o dy, the gradient of the dropped addend, which feeds the
+  // out-projection's gradients; dy itself still goes to the residual addend.  Without dropout dz is dy.
+  const bool drop = t->fwd_drop;
+  const float inv_keep = drop ? 1.f / (1.f - t->drop_p) : 1.f;
+  auto site = [&](int l, int kk) { return SDrop{t->drop_seed, (unsigned)t->fwd_step, (unsigned)(6 * l + kk), t->drop_p, inv_keep}; };
+  bf16* dz = drop ? t->dz.p : t->dy.p;
+  auto ln_bwd = [&](const bf16* y, int l, int kk, const float* gamma, const std::string& name) {
+    float *dg = G_of(t, grads, name + ".weight"), *db = G_of(t, grads, name + ".bias");
+    return drop ? t_ln_bwd_dropout(c, y, t->dx.p, R, gamma, t->dy.p, dz, dg, db, t->stats.p, site(l, kk), s)
+                : t_ln_bwd(c, y, t->dx.p, R, gamma, t->dy.p, dg, db, t->stats.p, s);
+  };
   for (int l = k.n_layers - 1; l >= 0; --l) {
     const std::string p = "decoder.layers." + std::to_string(l) + ".";
     const SLayer& W = c->layers[l];
     const LayerT& T = t->lt[l];
     LayerAct& A = t->acts[l];
     // ---- x3 = norm3(y3), y3 = h W2^T + b2 + x2, h = relu(x2 W1^T + b1)              (dx holds d loss / d x3)
-    S_TRY(t_ln_bwd(c, A.y3.p, t->dx.p, R, W.n3_g, t->dy.p, G_of(t, grads, p + "norm3.weight"), G_of(t, grads, p + "norm3.bias"), t->stats.p, s));
-    S_TRY(t_weight_grad(c, t->dy.p, dp, dp, A.h.p, fp, fp, fp, R, G_of(t, grads, p + "linear2.weight"), t->tA.p, t->tB.p, s));
-    S_TRY(t_colsum(c, t->dy.p, dp, R, dp, G_of(t, grads, p + "linear2.bias"), s));
-    S_TRY(s_gemm(c, t->dy.p, dp, T.ff2, dp, R, fp, nullptr, nullptr, 0, ACT_NONE, t->dh.p, fp, nullptr, 0, s));
-    S_TRY(t_relu_bwd(c, A.h.p, t->dh.p, (size_t)R * fp, s));
+    S_TRY(ln_bwd(A.y3.p, l, 5, W.n3_g, p + "norm3"));
+    S_TRY(t_weight_grad(c, dz, dp, dp, A.h.p, fp, fp, fp, R, G_of(t, grads, p + "linear2.weight"), t->tA.p, t->tB.p, s));
+    S_TRY(t_colsum(c, dz, dp, R, dp, G_of(t, grads, p + "linear2.bias"), s));
+    S_TRY(s_gemm(c, dz, dp, T.ff2, dp, R, fp, nullptr, nullptr, 0, ACT_NONE, t->dh.p, fp, nullptr, 0, s));
+    if (drop)
+      S_TRY(t_relu_bwd_dropout(c, A.h.p, t->dh.p, (size_t)R * fp, inv_keep, s));
+    else
+      S_TRY(t_relu_bwd(c, A.h.p, t->dh.p, (size_t)R * fp, s));
     S_TRY(t_weight_grad(c, t->dh.p, fp, fp, A.x2.p, dp, dp, dp, R, G_of(t, grads, p + "linear1.weight"), t->tA.p, t->tB.p, s));
     S_TRY(t_colsum(c, t->dh.p, fp, R, fp, G_of(t, grads, p + "linear1.bias"), s));
     S_TRY(s_gemm(c, t->dh.p, fp, T.ff1, fp, R, dp, nullptr, t->dy.p, dp, ACT_NONE, t->dx.p, dp, nullptr, 0, s));  // d x2 = dh W1 + d y3
     // ---- x2 = norm2(y2), y2 = a2 Wo^T + bo + x1, a2 = attn(q2, memkv), q2 = x1 Wq^T + bq, memkv = mem Wkv^T + bkv
-    S_TRY(t_ln_bwd(c, A.y2.p, t->dx.p, R, W.n2_g, t->dy.p, G_of(t, grads, p + "norm2.weight"), G_of(t, grads, p + "norm2.bias"), t->stats.p, s));
-    S_TRY(t_weight_grad(c, t->dy.p, dp, dp, A.a2.p, dp, dp, dp, R, G_of(t, grads, p + "multihead_attn.out_proj.weight"), t->tA.p, t->tB.p, s));
-    S_TRY(t_colsum(c, t->dy.p, dp, R, dp, G_of(t, grads, p + "multihead_attn.out_proj.bias"), s));
-    S_TRY(s_gemm(c, t->dy.p, dp, T.ca_out, dp, R, dp, nullptr, nullptr, 0, ACT_NONE, t->da.p, dp, nullptr, 0, s));
-    S_TRY(t_attn_bwd(c, A.q2.p, dp, L, A.memkv.p, M, 2 * dp, 0, dp, M, 0, nullptr, 0, B, t->da.p, t->dqkv.p, dp, t->dmemkv.p, 2 * dp, 0, dp, s));
+    S_TRY(ln_bwd(A.y2.p, l, 3, W.n2_g, p + "norm2"));
+    S_TRY(t_weight_grad(c, dz, dp, dp, A.a2.p, dp, dp, dp, R, G_of(t, grads, p + "multihead_attn.out_proj.weight"), t->tA.p, t->tB.p, s));
+    S_TRY(t_colsum(c, dz, dp, R, dp, G_of(t, grads, p + "multihead_attn.out_proj.bias"), s));
+    S_TRY(s_gemm(c, dz, dp, T.ca_out, dp, R, dp, nullptr, nullptr, 0, ACT_NONE, t->da.p, dp, nullptr, 0, s));
+    if (drop)
+      S_TRY(t_attn_bwd_dropout(c, A.q2.p, dp, L, A.memkv.p, M, 2 * dp, 0, dp, M, 0, nullptr, 0, B, t->da.p, t->dqkv.p, dp, t->dmemkv.p, 2 * dp, 0,
+                               dp, site(l, 2), s));
+    else
+      S_TRY(t_attn_bwd(c, A.q2.p, dp, L, A.memkv.p, M, 2 * dp, 0, dp, M, 0, nullptr, 0, B, t->da.p, t->dqkv.p, dp, t->dmemkv.p, 2 * dp, 0, dp, s));
     S_TRY(t_weight_grad(c, t->dqkv.p, dp, dp, A.x1.p, dp, dp, dp, R, G_of(t, grads, p + "multihead_attn.in_proj_weight", 0), t->tA.p, t->tB.p, s));
     S_TRY(t_colsum(c, t->dqkv.p, dp, R, dp, G_of(t, grads, p + "multihead_attn.in_proj_bias", 0), s));
     S_TRY(s_gemm(c, t->dqkv.p, dp, T.ca_q, dp, R, dp, nullptr, t->dy.p, dp, ACT_NONE, t->dx.p, dp, nullptr, 0, s));  // d x1 = dq2 Wq + d y2
@@ -793,12 +973,16 @@ int gitb200_student_train_backward(gitb200_student* c, int phase, float* grads, 
     S_TRY(s_gemm(c, t->dmemkv.p, 2 * dp, T.ca_kv, 2 * dp, Rm, dp, nullptr, l + 1 < k.n_layers ? t->dmem.p : nullptr, dp, ACT_NONE, t->dmem.p, dp,
                  nullptr, 0, s));  // d memory accumulates over the layers
     // ---- x1 = norm1(y1), y1 = a Wo^T + bo + x0, a = self-attn(qkv), qkv = x0 Win^T + bin
-    S_TRY(t_ln_bwd(c, A.y1.p, t->dx.p, R, W.n1_g, t->dy.p, G_of(t, grads, p + "norm1.weight"), G_of(t, grads, p + "norm1.bias"), t->stats.p, s));
-    S_TRY(t_weight_grad(c, t->dy.p, dp, dp, A.a.p, dp, dp, dp, R, G_of(t, grads, p + "self_attn.out_proj.weight"), t->tA.p, t->tB.p, s));
-    S_TRY(t_colsum(c, t->dy.p, dp, R, dp, G_of(t, grads, p + "self_attn.out_proj.bias"), s));
-    S_TRY(s_gemm(c, t->dy.p, dp, T.sa_out, dp, R, dp, nullptr, nullptr, 0, ACT_NONE, t->da.p, dp, nullptr, 0, s));
-    S_TRY(t_attn_bwd(c, A.qkv.p, 3 * dp, L, A.qkv.p, L, 3 * dp, dp, 2 * dp, L, 1, t->toks.p, L, B, t->da.p, t->dqkv.p, 3 * dp, t->dqkv.p, 3 * dp, dp,
-                     2 * dp, s));
+    S_TRY(ln_bwd(A.y1.p, l, 1, W.n1_g, p + "norm1"));
+    S_TRY(t_weight_grad(c, dz, dp, dp, A.a.p, dp, dp, dp, R, G_of(t, grads, p + "self_attn.out_proj.weight"), t->tA.p, t->tB.p, s));
+    S_TRY(t_colsum(c, dz, dp, R, dp, G_of(t, grads, p + "self_attn.out_proj.bias"), s));
+    S_TRY(s_gemm(c, dz, dp, T.sa_out, dp, R, dp, nullptr, nullptr, 0, ACT_NONE, t->da.p, dp, nullptr, 0, s));
+    if (drop)
+      S_TRY(t_attn_bwd_dropout(c, A.qkv.p, 3 * dp, L, A.qkv.p, L, 3 * dp, dp, 2 * dp, L, 1, t->toks.p, L, B, t->da.p, t->dqkv.p, 3 * dp, t->dqkv.p,
+                               3 * dp, dp, 2 * dp, site(l, 0), s));
+    else
+      S_TRY(t_attn_bwd(c, A.qkv.p, 3 * dp, L, A.qkv.p, L, 3 * dp, dp, 2 * dp, L, 1, t->toks.p, L, B, t->da.p, t->dqkv.p, 3 * dp, t->dqkv.p, 3 * dp,
+                       dp, 2 * dp, s));
     // q | k | v blocks are adjacent in the layout ([3*dp, dp] fp32): one GEMM fills all three
     S_TRY(t_weight_grad(c, t->dqkv.p, 3 * dp, 3 * dp, A.x0.p, dp, dp, dp, R, G_of(t, grads, p + "self_attn.in_proj_weight", 0), t->tA.p, t->tB.p, s));
     S_TRY(t_colsum(c, t->dqkv.p, 3 * dp, R, 3 * dp, G_of(t, grads, p + "self_attn.in_proj_bias", 0), s));

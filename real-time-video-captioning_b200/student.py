@@ -10,7 +10,8 @@ The nn.Module tree only holds parameters; there is no torch forward and no CPU p
 The TinyViT image encoder (timm ``features_only`` model, :35-48) is not rebuilt: pass ``image_encoder=`` (any module that
 returns the list of stage feature maps like timm's) or call ``greedy_decode_from_memory`` / ``forward_decoder`` with the
 ``memory`` tensor [B, F, d_model] directly.  ``enable_training`` / ``distillation_step`` / ``DistillationTrainer`` run the
-reference's distillation step (model.py:880-983) for the decoder on the same library (csrc/student_train.cu).
+reference's distillation step (model.py:880-983) for the decoder on the same library (csrc/student_train.cu), with the
+reference's train-mode dropout when a ``dropout_seed`` is given.
 """
 from __future__ import annotations
 
@@ -105,6 +106,8 @@ class StudentCandidateV1(nn.Module):
         self._grads = None          # flat fp32 gradient vector (torch owns it so that torch.distributed can reduce it in place)
         self._head_floats = 0
         self._params_dirty = False  # the optimizer has moved the library's master weights past the nn.Parameters
+        self._dropout_seed = None   # Philox seed of the training step's dropout masks; None: no dropout
+        self._dropout_step = 0      # the library's dropout step as of the last call that read or set it
 
     # ---- engine plumbing
     def load_state_dict(self, state_dict, strict: bool = False, **kw):
@@ -150,6 +153,9 @@ class StudentCandidateV1(nn.Module):
             self._grads = torch.zeros(n, dtype=torch.float32, device=p.device)
             self._head_floats = int(lib.gitb200_student_train_head_floats(h))
             self._params_dirty = False
+            if self._dropout_seed is not None:
+                _check(lib.gitb200_student_train_set_dropout(h, ctypes.c_float(self.dropout), self._dropout_seed, self._dropout_step),
+                       lib, h, "gitb200_student_train_set_dropout")
         return h
 
     def close(self):
@@ -243,18 +249,54 @@ class StudentCandidateV1(nn.Module):
         return self.greedy_decode_from_memory(memory, max_len)
 
     # ---- distillation training of the decoder half (DistillationTrainer.training_step, model.py:880-983)
-    def enable_training(self, lr: float = 1e-4, betas=(0.9, 0.999), eps: float = 1e-8) -> None:
+    def enable_training(self, lr: float = 1e-4, betas=(0.9, 0.999), eps: float = 1e-8, dropout_seed: Optional[int] = None) -> None:
         """Switch the library context to training mode: fp32 master weights + torch.optim.Adam state (model.py:1105:
-        ``Adam(student.parameters(), lr)``) next to the bf16 operand copies.  Dropout is not applied."""
+        ``Adam(student.parameters(), lr)``) next to the bf16 operand copies.
+
+        Without ``dropout_seed`` the step applies no dropout.  With it, ``distillation_step`` applies the reference's
+        train-mode dropout with p = ``self.dropout`` at nn.TransformerDecoderLayer's six sites per layer, from the library's
+        Philox masks (include/gitb200.h, gitb200_student_train_set_dropout): a pure function of (seed, ``dropout_step``, site,
+        element), so a step can be replayed.  ``dropout_step`` starts at 0.  p = 0 gives the step without dropout, bit for bit."""
+        if dropout_seed is not None:
+            if not 0.0 <= float(self.dropout) < 1.0:
+                raise ValueError(f"dropout p = {self.dropout} is outside [0, 1)")
+            if not 0 <= int(dropout_seed) < 2 ** 64:
+                raise ValueError("dropout_seed must be an integer in [0, 2**64)")
+            dropout_seed = int(dropout_seed)
         self._train_cfg = (float(lr), float(betas[0]), float(betas[1]), float(eps))
+        self._dropout_seed, self._dropout_step = dropout_seed, 0
         self._stale = True
+
+    @property
+    def dropout_step(self) -> int:
+        """Number of dropout forwards since the seed was set: the step whose masks the next ``distillation_step`` uses.
+        Set it to resume a run or to replay a step (``dropout_step -= 1`` replays the previous one)."""
+        if self._h is not None and not self._stale and self._train_cfg is not None:
+            step = ctypes.c_longlong()
+            _check(self._lib.gitb200_student_train_get_dropout(self._h, None, None, ctypes.byref(step)), self._lib, self._h,
+                   "gitb200_student_train_get_dropout")
+            self._dropout_step = step.value
+        return self._dropout_step
+
+    @dropout_step.setter
+    def dropout_step(self, step: int) -> None:
+        if self._dropout_seed is None:
+            raise RuntimeError("dropout is off: call enable_training(..., dropout_seed=...) first")
+        if int(step) < 0:
+            raise ValueError("dropout_step must be >= 0")
+        self._dropout_step = int(step)
+        if self._h is not None and not self._stale:
+            _check(self._lib.gitb200_student_train_set_dropout(self._h, ctypes.c_float(self.dropout), self._dropout_seed, self._dropout_step),
+                   self._lib, self._h, "gitb200_student_train_set_dropout")
 
     def distillation_step(self, y: torch.Tensor, memory: torch.Tensor, teacher_logits: torch.Tensor, temperature: float = 1.0,
                           apply: bool = True, group=None, want_memory_grad: bool = False):
         """One training step on this rank's micro-batch: forward_decoder(y, memory) -> KL(batchmean) * T^2 + CE(ignore 0)
         (model.py:922-935, :983) -> backward -> gradient all-reduce over ``group`` (DDP average; the vocabulary-head bucket is
         reduced while the decoder layers are still in their backward pass) -> Adam.  Returns {'loss','kl','ce'} (device
-        scalars, this rank's micro-batch) and, on request, d loss / d memory [B, M, d_model] for an external image encoder."""
+        scalars, this rank's micro-batch) and, on request, d loss / d memory [B, M, d_model] for an external image encoder.
+        With ``enable_training(dropout_seed=...)`` the forward applies dropout with the masks of ``dropout_step``, the backward
+        replays them, and ``dropout_step`` advances by one."""
         if self._train_cfg is None:
             raise RuntimeError("call enable_training() first")
         from .dist import all_reduce_bucket, finish_all_reduce
@@ -276,6 +318,8 @@ class StudentCandidateV1(nn.Module):
         s = self._stream()
         _check(lib.gitb200_student_train_forward(h, _ptr(tok), _ptr(mem), _ptr(tl), tl.stride(0), B, L, mem.shape[1],
                                                  ctypes.c_float(temperature), _ptr(loss), s), lib, h, "gitb200_student_train_forward")
+        if self._dropout_seed is not None:
+            _ = self.dropout_step   # refreshes the host-side copy that an engine rebuild restores
         g = self._grads
         _check(lib.gitb200_student_train_backward(h, 0, _ptr(g), None, s), lib, h, "gitb200_student_train_backward(head)")
         w0 = all_reduce_bucket(g, 0, self._head_floats, group)            # overlaps phase 1
@@ -329,11 +373,16 @@ class DistillationTrainer:
     gives the teacher-forced logits (``forward_output_logits``, :896), the student's DECODER is trained on KL + CE (:983) with
     Adam (:1105) and a DDP gradient all-reduce (train.py:217-221).  The student's TinyViT image encoder is not part of the
     library: ``batch['memory']`` ([B, F, d_model], what ``forward_image_enc`` returns at :128) is supplied by the caller, and
-    ``d_memory`` comes back for it.  No Lightning: call ``training_step`` from your own loop."""
+    ``d_memory`` comes back for it.  No Lightning: call ``training_step`` from your own loop.
 
-    def __init__(self, teacher, student: StudentCandidateV1, lr: float = 1e-4, temperature: float = 1.0, group=None):
+    ``dropout_seed``: None trains without dropout.  An integer applies the reference's train-mode dropout (p = the student's
+    ``dropout``) from the library's Philox masks.  The masks do not depend on the rank: for independent masks per rank pass
+    ``dropout_seed = seed + rank``."""
+
+    def __init__(self, teacher, student: StudentCandidateV1, lr: float = 1e-4, temperature: float = 1.0, group=None,
+                 dropout_seed: Optional[int] = None):
         self.teacher, self.student, self.temperature, self.group = teacher, student, temperature, group
-        student.enable_training(lr=lr)
+        student.enable_training(lr=lr, dropout_seed=dropout_seed)
 
     @torch.no_grad()
     def teacher_logits(self, x: torch.Tensor, y: torch.Tensor) -> torch.Tensor:
