@@ -521,10 +521,16 @@ def op_layernorm(x: torch.Tensor, gamma: torch.Tensor, beta: torch.Tensor, eps: 
     return out
 
 
-def op_attention_groups(qkv: torch.Tensor, n_groups: int, group_len: int, heads: int, scale: float, legacy_mma: bool = False):
+def op_attention_groups(qkv: torch.Tensor, n_groups: int, group_len: int, heads: int, scale: float, legacy_mma: bool = False,
+                        out=None):
+    """out: None (a new tensor of qkv's rows), or a contiguous bf16 [n_groups * group_len, heads * 64] tensor to write into,
+    such as a row range of a larger buffer."""
     lib = _lib.load()
     qkv = qkv.contiguous()
-    out = torch.empty(qkv.shape[0], heads * 64, dtype=torch.bfloat16, device=qkv.device)
+    if out is None:
+        out = torch.empty(qkv.shape[0], heads * 64, dtype=torch.bfloat16, device=qkv.device)
+    elif not (out.dtype == torch.bfloat16 and out.is_contiguous() and out.shape == (n_groups * group_len, heads * 64)):
+        raise ValueError("op_attention_groups: out must be a contiguous bf16 [n_groups * group_len, heads * 64] tensor")
     s = ctypes.c_void_p(torch.cuda.current_stream(qkv.device).cuda_stream)
     fn = lib.gitb200_op_attention_groups_mma if legacy_mma else lib.gitb200_op_attention_groups
     check(fn(_ptr(qkv), _ptr(out), n_groups, group_len, heads, scale, s), None, "gitb200_op_attention_groups")

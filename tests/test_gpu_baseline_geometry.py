@@ -7,7 +7,8 @@ repeats the oracle comparison where the benchmark actually runs:
     an UNTIED head over 64 clips with a measured token match rate on margin-robust positions;
   * configs[2]  beam 4, max 20 tokens, 6 frames -- asserted, not only recorded;
   * configs[3]  GIT-large: ViT-L/14 with 6 frames (1542 keys, the shipped teacher config) and 24 frames (6168 keys, 97 key
-    blocks of the tcgen05 attention kernel) -- operator level and through forward_logits;
+    blocks of the tcgen05 attention kernel) through forward_logits (the attention operator at these geometries:
+    test_gpu_attention_groups.py);
   * GenerativeImageTextTeacher.forward's ``output`` (model.py:772-789) against the oracle's statement-by-statement
     restatement, and caption-metric parity through calculate_bleu_score_corpus (src/metrics.py:42-68).
 
@@ -197,29 +198,6 @@ def test_base_f6_beam4_max20_matches_oracle(g, base6, tied):
 
 
 # ------------------------------------------------------------------------------------------ configs[3]
-@pytest.mark.parametrize("n_groups,group_len,heads", [(2, 1542, 12), (1, 6168, 12), (1, 4097, 16)])
-def test_op_attention_long_groups(g, n_groups, group_len, heads):
-    """The decoder's visual block at the GIT-large geometries: 1542 keys (6 frames x 257, the shipped teacher config, 25 key
-    blocks) and 6168 keys (24 frames, 97 key blocks, 49 query tiles per head): operator against an fp32 softmax."""
-    from importlib import import_module
-    eng = import_module("real-time-video-captioning_b200.engine")
-    gen = torch.Generator(device="cuda").manual_seed(group_len)
-    W = heads * 64
-    qkv = torch.randn(n_groups * group_len, 3 * W, device="cuda", generator=gen).bfloat16()
-    out = eng.op_attention_groups(qkv, n_groups, group_len, heads, 0.125)
-    q, k, v = qkv.float().view(n_groups, group_len, 3, heads, 64).permute(2, 0, 3, 1, 4)
-    worst = 0.0
-    for h0 in range(0, heads, 4):  # 4 heads at a time: the fp32 score matrix of 6168 keys is 152 MB per head
-        p = torch.softmax(q[:, h0:h0 + 4] @ k[:, h0:h0 + 4].transpose(-1, -2) * 0.125, dim=-1)
-        ref = (p @ v[:, h0:h0 + 4]).permute(0, 2, 1, 3).reshape(n_groups * group_len, 4 * 64)
-        err = (out[:, h0 * 64:(h0 + 4) * 64].float() - ref).abs()
-        worst = max(worst, err.max().item())
-        assert (err <= 0.02 + 0.01 * ref.abs()).all(), (h0, err.max())
-    again = eng.op_attention_groups(qkv, n_groups, group_len, heads, 0.125)
-    assert torch.equal(out, again)
-    record("op_attention_long_groups", group_len=group_len, heads=heads, max_err=worst)
-
-
 @pytest.mark.parametrize("n_frames", [6, 24])
 def test_git_large_full_geometry_forward_matches_oracle(g, n_frames):
     """GIT-large as shipped (ViT-L/14, 6 frames -> 1542 visual tokens) and as BASELINE configs[3] benchmarks it (24 frames ->

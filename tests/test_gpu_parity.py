@@ -3,6 +3,7 @@ C ABI (ctypes) and checks it against the CPU oracle (oracle/) on the same seeded
 
 Stated tolerances (bf16 activations / fp32 accumulation against an fp32 oracle):
   * single GEMM / LayerNorm / attention operator: |err| <= 0.02 + 0.01*|ref|  (one bf16 rounding of the output)
+    (the group attention operator: test_gpu_attention_groups.py, against a per-element bound)
   * visual features (12 pre-LN ViT layers + ln_post):        relative Frobenius error < 2e-2
   * decoder hidden states (7 tensors):                       relative Frobenius error < 3e-2
   * logits: max |delta| < 0.15 sigma(logits), mean |delta| < 0.03 sigma (the bf16-autocast CPU run of the same model
@@ -160,24 +161,6 @@ def test_op_layernorm(g, rows, cols, eps):
     assert (err <= 0.02 + 0.01 * ref.abs()).all(), err.max()
 
 
-@pytest.mark.parametrize("legacy", [False, True])
-@pytest.mark.parametrize("n_groups,group_len,heads", [(3, 197, 12), (2, 257, 16), (1, 1182, 12), (2, 64, 12), (2, 65, 12), (5, 1, 12),
-                                                      (2, 128, 12), (3, 129, 12), (2, 200, 12)])
-def test_op_attention_groups(g, n_groups, group_len, heads, legacy):
-    from importlib import import_module
-    eng = import_module("real-time-video-captioning_b200.engine")
-    gen = torch.Generator(device="cuda").manual_seed(group_len)
-    W = heads * 64
-    qkv = torch.randn(n_groups * group_len, 3 * W, device="cuda", generator=gen).bfloat16()
-    out = eng.op_attention_groups(qkv, n_groups, group_len, heads, 0.125, legacy_mma=legacy)
-    q, k, v = qkv.float().view(n_groups, group_len, 3, heads, 64).permute(2, 0, 3, 1, 4)
-    p = torch.softmax(q @ k.transpose(-1, -2) * 0.125, dim=-1)
-    ref = (p @ v).permute(0, 2, 1, 3).reshape(n_groups * group_len, W)
-    err = (out.float() - ref).abs()
-    record("op_attention_groups", group_len=group_len, legacy=legacy, max_err=err.max().item())
-    assert (err <= 0.02 + 0.01 * ref.abs()).all(), err.max()
-
-
 def _text_attention_reference(q, vis, txt, anc, n_clips, rpc, heads, scale):
     """Plain fp32 torch: every row attends to its clip's visual keys and to the text keys of its ancestors' slots."""
     rows, W = q.shape
@@ -225,46 +208,6 @@ def test_op_text_attention(g, n_clips, rpc, heads, n_vis, n_text, splits, use_an
     assert (err <= 0.01 + 0.008 * ref.abs()).all(), err.max()
     again = eng.op_text_attention(q, vis, txt, anc, n_clips, rpc, heads, 0.125, splits)
     assert torch.equal(out, again)
-
-
-@pytest.mark.parametrize("group_len,heads", [(197, 12), (1182, 12), (257, 16), (70, 12)])
-def test_op_attention_deterministic_and_batch_invariant(g, group_len, heads):
-    """The kernel must be bit-reproducible run to run and a group's result must not depend on its position in the batch
-    (the two softmax warpgroups, the lazy rescale and the hand-off barriers leave no room for a timing dependence)."""
-    from importlib import import_module
-    eng = import_module("real-time-video-captioning_b200.engine")
-    gen = torch.Generator(device="cuda").manual_seed(group_len * 3 + 1)
-    W = heads * 64
-    n_groups = 37
-    qkv = (torch.randn(n_groups * group_len, 3 * W, device="cuda", generator=gen) * 1.5).bfloat16()
-    outs = [eng.op_attention_groups(qkv, n_groups, group_len, heads, 0.125).clone() for _ in range(4)]
-    for o in outs[1:]:
-        assert torch.equal(o, outs[0])
-    for gi in (0, 17, 36):
-        one = eng.op_attention_groups(qkv[gi * group_len:(gi + 1) * group_len].contiguous(), 1, group_len, heads, 0.125)
-        assert torch.equal(one, outs[0][gi * group_len:(gi + 1) * group_len])
-
-
-@pytest.mark.parametrize("n_groups,group_len,heads,gain", [(2, 197, 12, 16.0), (1, 1182, 12, 12.0), (2, 257, 16, 24.0), (3, 40, 12, 16.0)])
-def test_op_attention_growing_scores(g, n_groups, group_len, heads, gain):
-    """Keys whose magnitude grows along the group: every key block raises the row maximum by many powers of two, so the
-    kernel's lazy running-max path (rescale of the TMEM accumulator) runs on most blocks instead of almost never."""
-    from importlib import import_module
-    eng = import_module("real-time-video-captioning_b200.engine")
-    gen = torch.Generator(device="cuda").manual_seed(group_len + 7)
-    W = heads * 64
-    qkv = torch.randn(n_groups, group_len, 3, heads, 64, device="cuda", generator=gen)
-    ramp = torch.linspace(0.05, gain, group_len, device="cuda").view(1, group_len, 1, 1)
-    qkv[:, :, 1] *= ramp
-    qkv = qkv.reshape(n_groups * group_len, 3 * W).bfloat16()
-    out = eng.op_attention_groups(qkv, n_groups, group_len, heads, 0.125)
-    q, k, v = qkv.float().view(n_groups, group_len, 3, heads, 64).permute(2, 0, 3, 1, 4)
-    p = torch.softmax(q @ k.transpose(-1, -2) * 0.125, dim=-1)
-    ref = (p @ v).permute(0, 2, 1, 3).reshape(n_groups * group_len, W)
-    err = (out.float() - ref).abs()
-    record("op_attention_growing_scores", group_len=group_len, max_err=err.max().item())
-    assert torch.isfinite(out.float()).all()
-    assert (err <= 0.03 + 0.015 * ref.abs()).all(), err.max()
 
 
 @pytest.mark.parametrize("nb,keep,max_steps,eos_boost", [(1, 1, 6, 0.0), (1, 1, 15, 3.0), (4, 1, 15, 2.0), (4, 3, 10, 4.0), (3, 2, 8, 6.0)])
