@@ -55,7 +55,8 @@ typedef struct {
 
 /* The search's sampling / penalty arguments (model.py:479-480, :524-554).  top_k = 0 and top_p = 1 disable the filters;
  * temperature, top_k and top_p act only with do_sample.  seed is the Philox4x32-10 key of the draws: a clip's sample depends
- * only on (seed, its index in the call, its scores).  All-default values (do_sample 0, repetition_penalty 1,
+ * only on (seed, its index in the call, its scores).  gitb200_streams_caption_ext instead gives every stream its own key
+ * and leaves the index out of the counter, so a stream's sample does not depend on its position in the call.  All-default values (do_sample 0, repetition_penalty 1,
  * num_return_sequences 1) select exactly the calls without this struct. */
 typedef struct {
   int do_sample;              /* 0: beam / greedy; 1: sample per_node_beam_size words per beam row, without replacement */
@@ -254,6 +255,12 @@ int gitb200_stream_push_u8(gitb200_ctx* ctx, const uint8_t* frame_dev, int heigh
 int gitb200_stream_frames(const gitb200_ctx* ctx);
 int gitb200_stream_caption(gitb200_ctx* ctx, const gitb200_search_params* sp, int32_t* tokens_dev, float* logprobs_dev,
                            void* stream);
+/* gitb200_stream_caption with sampling, repetition penalty and num_return_sequences (sp_ext must not be NULL; sp_ext->seed is
+ * the Philox key): the result equals gitb200_decode_ext on the window's features, outputs and optional saved logits as there.
+ * An all-default sp_ext without logits_dev is gitb200_stream_caption.  Rejections as gitb200_decode_ext's, before anything is
+ * enqueued. */
+int gitb200_stream_caption_ext(gitb200_ctx* ctx, const gitb200_search_params* sp, const gitb200_sample_params* sp_ext,
+                               int32_t* tokens_dev, float* logprobs_dev, float* logits_dev, void* stream);
 
 /* ---- multi-stream pool: many cameras on one context ------------------------------------------------------------
  * A pool of n_streams windows next to the single window above (which it does not touch), each window the same ring of
@@ -284,6 +291,24 @@ int gitb200_streams_push_u8(gitb200_ctx* ctx, const int32_t* ids_host, int k, co
  * does not depend on which other streams share the call or in which order. */
 int gitb200_streams_caption(gitb200_ctx* ctx, const int32_t* ids_host, int k, const gitb200_search_params* sp,
                             int32_t* tokens_dev, float* logprobs_dev, void* stream);
+/* gitb200_streams_caption with sampling, repetition penalty and num_return_sequences, each stream drawing from its own
+ * Philox key.  sp_ext must not be NULL; sp_ext->seed is ignored.  keys_host uint64 [k] (required when sp_ext->do_sample,
+ * ignored otherwise): keys_host[j] is the key of stream ids_host[j] -- give a camera a fresh key for every caption (e.g. one
+ * derived from a seed, its id and its caption count) or its successive samples reuse the same uniforms.
+ * tokens_dev int32 [k*nrs, num_keep_best, max_steps], logprobs_dev fp32 [k*nrs, num_keep_best]: row j*nrs + r is sequence r
+ * of stream ids_host[j] (nrs = num_return_sequences).  logits_dev (optional) fp32 [max_steps-1, k*nrs*beam, logits_ld]: the
+ * pre-penalty scores, as in gitb200_decode_ext.
+ * The result for stream ids_host[j] depends only on its window, keys_host[j], the parameters and the number of rows in the
+ * call (a decode GEMM of <= 8 rows sums in another order than a larger one); not on the other streams in the call or their
+ * order.  With k = 1 it equals gitb200_decode_ext with seed = keys_host[0] on that window's features.
+ * Everything is checked on the host before anything is enqueued: what gitb200_streams_caption rejects, what
+ * gitb200_decode_ext rejects for k clips, and a NULL keys_host while sampling; a rejected call changes no window.  An
+ * all-default sp_ext without logits_dev is gitb200_streams_caption, bit for bit.  The key table is copied into a
+ * context-owned device buffer before any graph launch, so the CUDA graphs (keyed by shape and by the parameters other than
+ * keys and seed) replay for any keys.  Afterwards the context's current visual features are these k windows. */
+int gitb200_streams_caption_ext(gitb200_ctx* ctx, const int32_t* ids_host, int k, const gitb200_search_params* sp,
+                                const gitb200_sample_params* sp_ext, const uint64_t* keys_host, int32_t* tokens_dev,
+                                float* logprobs_dev, float* logits_dev, void* stream);
 /* Empties the windows of k distinct streams (the reference's frames.clear() after a caption, real_time_inference.py:61). */
 int gitb200_streams_reset(gitb200_ctx* ctx, const int32_t* ids_host, int k);
 /* Frames held by one stream's window (0 .. num_image_with_embedding); GITB200_ERR_INVALID for an unknown id. */

@@ -10,7 +10,7 @@ from ._lib import GitB200Error, LIB_PATH  # noqa: F401
 from .engine import Engine, SampleConfig, SearchConfig, make_config, preprocess_frames, VIT_CONFIGS  # noqa: F401
 from .model import (BeamHypotheses, CLIPVisionTower, GenerativeImageTextModel, GenerativeImageTextTeacher,  # noqa: F401
                     GeneratorWithBeamSearchV2, LazyLogits, MultiStreamCaptioner, StreamingCaptioner, SyntheticTokenizer, TransformerDecoderTextualHead,
-                    get_git_model)
+                    get_git_model, stream_key)
 from .student import DistillationTrainer, StudentCandidateV1  # noqa: F401
 from .metrics import calculate_bleu_score_corpus  # noqa: F401
 from .dist import all_reduce_bucket, caption_sharded, finish_all_reduce, shard_range  # noqa: F401
@@ -18,4 +18,4 @@ from .dist import all_reduce_bucket, caption_sharded, finish_all_reduce, shard_r
 __all__ = ["Engine", "SampleConfig", "SearchConfig", "GenerativeImageTextModel", "GenerativeImageTextTeacher",
            "GeneratorWithBeamSearchV2", "get_git_model", "calculate_bleu_score_corpus", "shard_range",
            "caption_sharded", "GitB200Error", "StudentCandidateV1", "DistillationTrainer", "all_reduce_bucket",
-           "finish_all_reduce", "MultiStreamCaptioner"]
+           "finish_all_reduce", "MultiStreamCaptioner", "stream_key"]

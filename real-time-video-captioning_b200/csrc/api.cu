@@ -175,6 +175,7 @@ struct gitb200_ctx {
   int pool_streams = 0;
   std::vector<int> pool_head, pool_count;
   Buf<int> pool_rows, pool_oldest;
+  Buf<unsigned long long> pool_keys;  // per-call table of a sampled caption (gitb200_streams_caption_ext): Philox key of each row
 
   // forward-hook taps on image_encoder.transformer.resblocks[i] (model.py:847): outputs copied out by the next encodes
   std::vector<int> tap_layers;
@@ -849,8 +850,9 @@ int make_search_state(gitb200_ctx* c, int n_clips, int V, int ldl, int sos_unuse
 // forced pass writes the K/V of the first P - 1 of them (every clip's visual K/V read once for the whole prompt), the K/V are
 // copied into the decode slots of all the clip's rows, and the search starts at t0 = P - 1 with the prompt as its history:
 // max_steps - P steps, saved logits [max_steps - P][rows][ld].  P = 0: no prompt (the search starts from SOS at t = 0).
+// keys (device, optional, sampling only): one Philox key per clip instead of the seed in seed_dev (SampleState::keys).
 int run_decode(gitb200_ctx* c, const gitb200_search_params& sp, int32_t* tokens_out, float* logprobs_out, float* logits_out,
-               cudaStream_t s, const gitb200_sample_params* smp = nullptr, int P = 0) {
+               cudaStream_t s, const gitb200_sample_params* smp = nullptr, int P = 0, const unsigned long long* keys = nullptr) {
   const gitb200_config& k = c->cfg;
   const int nrs = smp ? smp->num_return_sequences : 1;
   const int B = c->cur_clips, nb = sp.beam_size, entries = B * nrs, rows = entries * nb;
@@ -862,6 +864,7 @@ int run_decode(gitb200_ctx* c, const gitb200_search_params& sp, int32_t* tokens_
   if (smp) {
     ss.do_sample = smp->do_sample; ss.top_k = smp->top_k; ss.nrs = nrs; ss.pnb = sp.per_node_beam_size;
     ss.top_p = smp->top_p; ss.temperature = smp->temperature; ss.rp = smp->repetition_penalty; ss.seed = c->seed_dev.p;
+    ss.keys = keys;
   }
   if (!c->visual_pass_done) TRY(run_visual_pass(c, false, nullptr, 0, s));
   const int steps = sp.max_steps - 1;        // model.py:518: while cur_len < max_length, cur_len = t + 1
@@ -966,7 +969,7 @@ int run_decode(gitb200_ctx* c, const gitb200_search_params& sp, int32_t* tokens_
   for (int ts = t0; ts < steps; ts += seg) {
     const int n = steps - ts < seg ? steps - ts : seg;
     gitb200_ctx::GraphKey key;
-    key.kind = 5; key.i0 = B; key.i1 = ts; key.i2 = n; key.i3 = c->cur_nv; key.i4 = P; key.sp = sp; key.p0 = logits_out;
+    key.kind = 5; key.i0 = B; key.i1 = ts; key.i2 = n; key.i3 = c->cur_nv; key.i4 = P; key.sp = sp; key.p0 = logits_out; key.p1 = keys;
     if (smp) {
       key.smp = *smp;
       key.smp.seed = 0;
@@ -1012,7 +1015,7 @@ void free_workspaces(gitb200_ctx* c) {
   fr(c->tx); fr(c->tq); fr(c->ta); fr(c->tb); fr(c->tc); fr(c->tf); fr(c->logits); fr(c->partial); fr(c->vf_in_f32);
   fr(c->ibuf); fr(c->dbuf); fr(c->fbuf); fr(c->pos_arr); fr(c->ntext_arr); fr(c->tok_arr); fr(c->stage[0]); fr(c->stage[1]); fr(c->stage_u8[0]); fr(c->stage_u8[1]);
   fr(c->out_tok); fr(c->out_lp); fr(c->stats_a); fr(c->stats_b); fr(c->ring);
-  fr(c->pool); fr(c->pool_rows); fr(c->pool_oldest); fr(c->seed_dev);
+  fr(c->pool); fr(c->pool_rows); fr(c->pool_oldest); fr(c->pool_keys); fr(c->seed_dev);
   fr(c->prefix_dev); fr(c->prefix_kv);
 }
 
@@ -1793,29 +1796,53 @@ int gitb200_stream_push_u8(gitb200_ctx* c, const uint8_t* frame, int height, int
 
 int gitb200_stream_frames(const gitb200_ctx* c) { return c ? c->ring_count : 0; }
 
-int gitb200_stream_caption(gitb200_ctx* c, const gitb200_search_params* sp, int32_t* tokens, float* logprobs, void* stream) {
-  if (!c || !sp || !tokens || !logprobs) return fail(c, GITB200_ERR_INVALID, "bad stream_caption argument");
-  if (c->ring_count < 1) return fail(c, GITB200_ERR_STATE, "no frames in the streaming window: call gitb200_stream_push first");
-  CUDA_OK(c, cudaSetDevice(c->device));
-  cudaStream_t s = caller_stream(c, stream);
+// gitb200_stream_caption (smp == nullptr) and gitb200_stream_caption_ext (the seed already in seed_dev when smp is active)
+static int stream_caption_impl(gitb200_ctx* c, const gitb200_search_params* sp, const gitb200_sample_params* smp, int32_t* tokens,
+                               float* logprobs, float* logits, cudaStream_t s) {
   const int cap = c->cfg.num_image_with_embedding, n = c->ring_count, T = c->T, W = c->cfg.vit_width;
   ENSURE(c, c->vf, (size_t)n * T * W);
   const int first = (c->ring_head - n + cap) % cap;  // oldest frame -> temporal position 0
   gitb200_ctx::GraphKey key;
   key.kind = 2; key.p0 = tokens; key.p1 = logprobs; key.i0 = n; key.i1 = first; key.sp = *sp;
-  const int r = run_graphed(c, key, s, true, [&]() {
+  if (smp) {
+    key.smp = *smp;
+    key.smp.seed = 0;
+  }
+  // saved logits: eager (the step loop's early exit decides how many steps they hold, as in gitb200_decode)
+  const int r = run_graphed(c, key, s, logits == nullptr, [&]() {
     CUDA_OK(c, assemble_window(c->ring.p, first, cap, n, T, W, c->temporal, c->vf.p, s));
     c->cur_clips = 1;
     c->cur_nv = n * T;
     c->visual_pass_done = false;
     c->step_rows_per_clip = 0;
-    return run_decode(c, *sp, tokens, logprobs, nullptr, s);
+    return run_decode(c, *sp, tokens, logprobs, logits, s, smp);
   });
   if (r == 1) {
     c->cur_clips = 1; c->cur_nv = n * T; c->visual_pass_done = true; c->visual_pass_full = 0; c->step_rows_per_clip = 0;
     return GITB200_OK;
   }
   return r;
+}
+
+int gitb200_stream_caption(gitb200_ctx* c, const gitb200_search_params* sp, int32_t* tokens, float* logprobs, void* stream) {
+  if (!c || !sp || !tokens || !logprobs) return fail(c, GITB200_ERR_INVALID, "bad stream_caption argument");
+  if (c->ring_count < 1) return fail(c, GITB200_ERR_STATE, "no frames in the streaming window: call gitb200_stream_push first");
+  CUDA_OK(c, cudaSetDevice(c->device));
+  return stream_caption_impl(c, sp, nullptr, tokens, logprobs, nullptr, caller_stream(c, stream));
+}
+
+int gitb200_stream_caption_ext(gitb200_ctx* c, const gitb200_search_params* sp, const gitb200_sample_params* smp, int32_t* tokens,
+                               float* logprobs, float* logits, void* stream) {
+  if (!c || !sp || !smp || !tokens || !logprobs) return fail(c, GITB200_ERR_INVALID, "bad stream_caption_ext argument");
+  if (!c->finalized) return fail(c, GITB200_ERR_STATE, "call gitb200_finalize_weights first");
+  TRY(check_sample(c, *sp, *smp, c->cfg.vocab, 1, c->cfg.max_positions, true));
+  if (c->ring_count < 1) return fail(c, GITB200_ERR_STATE, "no frames in the streaming window: call gitb200_stream_push first");
+  const bool active = sample_active(*smp);
+  if (!active && logits == nullptr) return gitb200_stream_caption(c, sp, tokens, logprobs, stream);
+  CUDA_OK(c, cudaSetDevice(c->device));
+  cudaStream_t s = caller_stream(c, stream);
+  if (active) TRY(upload_seed(c, smp->seed, s));
+  return stream_caption_impl(c, sp, active ? smp : nullptr, tokens, logprobs, logits, s);
 }
 
 // ---- multi-stream pool: one window per camera stream, pushes and captions batched over streams
@@ -1855,17 +1882,18 @@ int gitb200_streams_configure(gitb200_ctx* c, int n_streams) {
   if (cap < 1) return fail(c, GITB200_ERR_STATE, "streaming needs num_image_with_embedding >= 1 (the window length)");
   CUDA_OK(c, cudaSetDevice(c->device));
   if (n_streams != c->pool_streams) {
-    for (void* p : {(void*)c->pool.p, (void*)c->pool_rows.p, (void*)c->pool_oldest.p})
+    for (void* p : {(void*)c->pool.p, (void*)c->pool_rows.p, (void*)c->pool_oldest.p, (void*)c->pool_keys.p})
       if (p) {
         CUDA_OK(c, cudaFree(p));
         c->ws_gen++;  // captured graphs hold the freed pointers
       }
-    c->pool = Buf<bf16>{}; c->pool_rows = Buf<int>{}; c->pool_oldest = Buf<int>{};
+    c->pool = Buf<bf16>{}; c->pool_rows = Buf<int>{}; c->pool_oldest = Buf<int>{}; c->pool_keys = Buf<unsigned long long>{};
     c->pool_streams = 0;
     c->pool_head.clear(); c->pool_count.clear();
     ENSURE(c, c->pool, (size_t)n_streams * cap * c->T * c->cfg.vit_width);
     ENSURE(c, c->pool_rows, (size_t)n_streams);
     ENSURE(c, c->pool_oldest, (size_t)n_streams);
+    ENSURE(c, c->pool_keys, (size_t)n_streams);
     c->pool_streams = n_streams;
   }
   c->pool_head.assign((size_t)n_streams, 0);
@@ -1914,19 +1942,24 @@ int gitb200_streams_push_u8(gitb200_ctx* c, const int32_t* ids, int k, const uin
   return streams_push_any(c, ids, k, nullptr, frames, height, width, stream);
 }
 
-int gitb200_streams_caption(gitb200_ctx* c, const int32_t* ids, int k, const gitb200_search_params* sp, int32_t* tokens,
-                            float* logprobs, void* stream) {
-  if (!c || !sp || !tokens || !logprobs) return fail(c, GITB200_ERR_INVALID, "bad streams_caption argument");
-  if (!c->finalized) return fail(c, GITB200_ERR_STATE, "call gitb200_finalize_weights first");
-  TRY(pool_check_ids(c, "gitb200_streams_caption", ids, k));
+// Host-side check of a caption's stream set (after pool_check_ids): every window holds frames, all the same number.
+static int pool_check_held(gitb200_ctx* c, const char* what, const int32_t* ids, int k) {
   const int n = c->pool_count[ids[0]];
   for (int j = 0; j < k; ++j) {
-    if (c->pool_count[ids[j]] < 1)
-      return fail(c, GITB200_ERR_STATE, "gitb200_streams_caption: stream id %d holds no frames: push first", ids[j]);
+    if (c->pool_count[ids[j]] < 1) return fail(c, GITB200_ERR_STATE, "%s: stream id %d holds no frames: push first", what, ids[j]);
     if (c->pool_count[ids[j]] != n)
-      return fail(c, GITB200_ERR_INVALID, "gitb200_streams_caption: stream id %d holds %d frames but stream id %d holds %d: "
-                  "windows of different lengths go in separate calls", ids[j], c->pool_count[ids[j]], ids[0], n);
+      return fail(c, GITB200_ERR_INVALID, "%s: stream id %d holds %d frames but stream id %d holds %d: "
+                  "windows of different lengths go in separate calls", what, ids[j], c->pool_count[ids[j]], ids[0], n);
   }
+  return 0;
+}
+
+// gitb200_streams_caption (smp == nullptr) and gitb200_streams_caption_ext (smp active; keys_host: one Philox key per id when
+// smp->do_sample).  Everything is validated by the caller.
+static int streams_caption_impl(gitb200_ctx* c, const int32_t* ids, int k, const gitb200_search_params* sp,
+                                const gitb200_sample_params* smp, const uint64_t* keys_host, int32_t* tokens, float* logprobs,
+                                float* logits, void* stream) {
+  const int n = c->pool_count[ids[0]];
   CUDA_OK(c, cudaSetDevice(c->device));
   const cudaStream_t s = (cudaStream_t)stream;
   TRY(pool_order_after_last_stream(c, s));
@@ -1936,6 +1969,12 @@ int gitb200_streams_caption(gitb200_ctx* c, const int32_t* ids, int k, const git
   std::vector<int> oldest((size_t)k);
   for (int j = 0; j < k; ++j) oldest[j] = ids[j] * cap + (c->pool_head[ids[j]] - n + cap) % cap;  // temporal position 0
   CUDA_OK(c, cudaMemcpyAsync(c->pool_oldest.p, oldest.data(), (size_t)k * sizeof(int), cudaMemcpyHostToDevice, s));
+  const unsigned long long* keys = nullptr;
+  if (smp && smp->do_sample) {
+    // (a pageable source: the copy is staged before cudaMemcpyAsync returns)
+    CUDA_OK(c, cudaMemcpyAsync(c->pool_keys.p, keys_host, (size_t)k * sizeof(unsigned long long), cudaMemcpyHostToDevice, s));
+    keys = c->pool_keys.p;
+  }
   auto assemble = [&]() -> int {
     CUDA_OK(c, assemble_windows(c->pool.p, c->pool_oldest.p, 0, k, n, cap, T, W, c->temporal, c->vf.p, nullptr, s));
     c->cur_clips = k; c->cur_nv = n * T; c->visual_pass_done = false; c->step_rows_per_clip = 0;
@@ -1945,9 +1984,14 @@ int gitb200_streams_caption(gitb200_ctx* c, const int32_t* ids, int k, const git
   key.i0 = k; key.i1 = n;
   if (k <= c->graph_max_clips) {  // latency mode: the whole call as one graph (k == 1, beam <= 4: the persistent decode kernel)
     key.kind = 12; key.p0 = tokens; key.p1 = logprobs; key.sp = *sp;
-    const int r = run_graphed(c, key, s, true, [&]() -> int {
+    if (smp) {  // the keys and the seed are read from device tables: the graph replays for any of them
+      key.smp = *smp;
+      key.smp.seed = 0;
+    }
+    // saved logits: eager (the step loop's early exit decides how many steps they hold, as in gitb200_decode)
+    const int r = run_graphed(c, key, s, logits == nullptr, [&]() -> int {
       TRY(assemble());
-      return run_decode(c, *sp, tokens, logprobs, nullptr, s);
+      return run_decode(c, *sp, tokens, logprobs, logits, s, smp, 0, keys);
     });
     if (r == 1) {  // replayed: host-side state the eager run would have left
       c->cur_clips = k; c->cur_nv = n * T; c->visual_pass_done = true; c->visual_pass_full = 0; c->step_rows_per_clip = 0;
@@ -1967,7 +2011,33 @@ int gitb200_streams_caption(gitb200_ctx* c, const int32_t* ids, int k, const git
   } else if (r != 0) {
     return r;
   }
-  return run_decode(c, *sp, tokens, logprobs, nullptr, s);
+  return run_decode(c, *sp, tokens, logprobs, logits, s, smp, 0, keys);
+}
+
+int gitb200_streams_caption(gitb200_ctx* c, const int32_t* ids, int k, const gitb200_search_params* sp, int32_t* tokens,
+                            float* logprobs, void* stream) {
+  if (!c || !sp || !tokens || !logprobs) return fail(c, GITB200_ERR_INVALID, "bad streams_caption argument");
+  if (!c->finalized) return fail(c, GITB200_ERR_STATE, "call gitb200_finalize_weights first");
+  TRY(pool_check_ids(c, "gitb200_streams_caption", ids, k));
+  TRY(pool_check_held(c, "gitb200_streams_caption", ids, k));
+  return streams_caption_impl(c, ids, k, sp, nullptr, nullptr, tokens, logprobs, nullptr, stream);
+}
+
+int gitb200_streams_caption_ext(gitb200_ctx* c, const int32_t* ids, int k, const gitb200_search_params* sp,
+                                const gitb200_sample_params* smp, const uint64_t* keys_host, int32_t* tokens, float* logprobs,
+                                float* logits, void* stream) {
+  const char* what = "gitb200_streams_caption_ext";
+  if (!c) return GITB200_ERR_INVALID;
+  if (!sp || !smp || !tokens || !logprobs) return fail(c, GITB200_ERR_INVALID, "%s: bad argument", what);
+  if (!c->finalized) return fail(c, GITB200_ERR_STATE, "call gitb200_finalize_weights first");
+  TRY(pool_check_ids(c, what, ids, k));
+  TRY(pool_check_held(c, what, ids, k));
+  TRY(check_sample(c, *sp, *smp, c->cfg.vocab, k, c->cfg.max_positions, true));
+  if (smp->do_sample && keys_host == nullptr)
+    return fail(c, GITB200_ERR_INVALID, "%s: keys_host is NULL while do_sample is set (one Philox key per stream id)", what);
+  const bool active = sample_active(*smp);
+  if (!active && logits == nullptr) return gitb200_streams_caption(c, ids, k, sp, tokens, logprobs, stream);
+  return streams_caption_impl(c, ids, k, sp, active ? smp : nullptr, keys_host, tokens, logprobs, logits, stream);
 }
 
 int gitb200_streams_reset(gitb200_ctx* c, const int32_t* ids, int k) {

@@ -194,6 +194,9 @@ struct SampleState {
   int do_sample, top_k, nrs, pnb;
   float top_p, temperature, rp;
   const unsigned long long* seed;  // device word: the Philox key
+  // Optional device table of one Philox key per clip (entry e draws with keys[e / nrs] and counter word 3 = 0, so a clip's
+  // draws do not depend on its position in the call).  nullptr: key *seed, counter word 3 = the clip index e / nrs.
+  const unsigned long long* keys;
 };
 // Bytes of dynamic shared memory a row of `V` logits needs (the limit the caller checks before enqueueing anything).
 size_t sample_step_smem(int V);

@@ -327,12 +327,14 @@ __global__ void __launch_bounds__(SS_THREADS) sample_rows_kernel(SearchState st,
   const float l = s.bc_f;
   const float bs = __ldcg(st.beam_scores + row);
   // ---- per_node_beam_size draws without replacement (model.py:540): the exponential race -- the largest
-  // (x - m) - log(-log u) in order, u = Philox4x32-10(counter (i / 4, step, j * nb + b, clip), key = seed) word i % 4.
+  // (x - m) - log(-log u) in order, u = Philox4x32-10(counter (i / 4, step, j * nb + b, clip), key = seed) word i % 4;
+  // with a key table, counter (i / 4, step, j * nb + b, 0) and key = keys[clip].
   // When the filters keep fewer tokens than per_node_beam_size (only a top-p cut can: check_sample rejects top-k below it),
   // the reference's torch.multinomial raises; here the missing draws are removed tokens in index order, with score -inf.
-  const unsigned long long seed = *p.seed;
+  const int clip = e / p.nrs;
+  const unsigned long long seed = p.keys ? p.keys[clip] : *p.seed;
   const uint32_t k0 = (uint32_t)seed, k1 = (uint32_t)(seed >> 32);
-  const uint32_t c2 = (uint32_t)((e % p.nrs) * nb + b), c3 = (uint32_t)(e / p.nrs);
+  const uint32_t c2 = (uint32_t)((e % p.nrs) * nb + b), c3 = p.keys ? 0u : (uint32_t)clip;
   float prev_s = INFINITY;
   int prev_i = -1;
   for (int r = 0; r < p.pnb; ++r) {
@@ -511,7 +513,7 @@ cudaError_t sample_step(const SearchState& s, const SampleState& p, const float*
                         cudaStream_t stream) {
   if (s.n_clips <= 0) return cudaSuccess;
   if (s.nb > MAX_NB || s.cand > MAX_CAND || cur_len + 1 > s.max_len || s.n_clips > 65535 || p.nrs < 1 || p.pnb < 1 ||
-      s.row_cand_score == nullptr || s.row_cand_idx == nullptr || (p.do_sample && p.seed == nullptr))
+      s.row_cand_score == nullptr || s.row_cand_idx == nullptr || (p.do_sample && p.seed == nullptr && p.keys == nullptr))
     return cudaErrorInvalidValue;
   const size_t smem = sample_step_smem(s.V);
   cudaError_t e = cudaFuncSetAttribute(sample_rows_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem);

@@ -37,7 +37,8 @@ class SearchConfig:
 class SampleConfig:
     """search() sampling keyword arguments (model.py:479-480) and the decoder's repetition_penalty / temperature
     (model.py:524-535), plus the seed of the device's counter-based RNG: a clip's sample depends only on (seed, its index
-    in the call, its scores).  top_k = 0 and top_p = 1.0 disable the filters."""
+    in the call, its scores).  The stream pool ignores the seed and takes one key per camera (``Engine.streams_caption``).
+    top_k = 0 and top_p = 1.0 disable the filters."""
     do_sample: bool = False
     top_k: int = 0
     top_p: float = 1.0
@@ -361,20 +362,40 @@ class Engine:
         check(self.lib.gitb200_stream_push_u8(self.h, _ptr(frame_u8), h, w, self._stream()), self.h, "gitb200_stream_push_u8")
         return int(self.lib.gitb200_stream_frames(self.h))
 
-    def stream_caption(self, sp: SearchConfig):
+    def _window_outputs(self, attr: str, k: int, sp: SearchConfig, sample: Optional[SampleConfig]):
         # persistent output buffers: identical call signatures let the library replay its captured CUDA graph
-        key = (sp.num_keep_best, sp.max_steps)
-        if not hasattr(self, "_stream_out"):
-            self._stream_out = {}
-        if key not in self._stream_out:
-            self._stream_out[key] = (torch.empty(1, sp.num_keep_best, sp.max_steps, dtype=torch.int32, device=self.device),
-                                     torch.empty(1, sp.num_keep_best, dtype=torch.float32, device=self.device))
-        tokens, logprobs = self._stream_out[key]
+        n = k * (sample.num_return_sequences if sample is not None else 1)
+        key = (n, sp.num_keep_best, sp.max_steps)
+        bufs = self.__dict__.setdefault(attr, {})
+        if key not in bufs:
+            bufs[key] = (torch.empty(n, sp.num_keep_best, sp.max_steps, dtype=torch.int32, device=self.device),
+                         torch.empty(n, sp.num_keep_best, dtype=torch.float32, device=self.device))
+        return bufs[key]
+
+    def _saved_logits(self, n_rows: int, sp: SearchConfig, save_logits: bool, sample: Optional[SampleConfig]):
+        if save_logits and sample is None:
+            raise GitB200Error("save_logits needs sample (a SampleConfig; SampleConfig() for plain beam search)")
+        return torch.empty(sp.max_steps - 1, n_rows * sp.beam_size, self.ld, dtype=torch.float32,
+                           device=self.device) if save_logits else None
+
+    def stream_caption(self, sp: SearchConfig, sample: Optional[SampleConfig] = None, save_logits: bool = False):
+        """Caption the single streaming window: (tokens int32 [1, keep, max_steps], logprobs [1, keep]).  With ``sample``
+        (its seed is the Philox key) the result equals ``decode(1, sp, sample=sample)`` on the window's features and the
+        call returns (tokens [nrs, keep, max_steps], logprobs [nrs, keep], logits or None) as ``decode`` does."""
+        tokens, logprobs = self._window_outputs("_stream_out", 1, sp, sample)
         c = sp.to_c()
-        check(self.lib.gitb200_stream_caption(self.h, ctypes.byref(c), _ptr(tokens), _ptr(logprobs), self._stream()), self.h,
-              "gitb200_stream_caption")
+        if sample is None:
+            check(self.lib.gitb200_stream_caption(self.h, ctypes.byref(c), _ptr(tokens), _ptr(logprobs), self._stream()), self.h,
+                  "gitb200_stream_caption")
+        else:
+            logits = self._saved_logits(tokens.shape[0], sp, save_logits, sample)
+            x = sample.to_c()
+            check(self.lib.gitb200_stream_caption_ext(self.h, ctypes.byref(c), ctypes.byref(x), _ptr(tokens), _ptr(logprobs),
+                                                      _ptr(logits), self._stream()), self.h, "gitb200_stream_caption_ext")
         self._cur_clips, self._cur_nv, self._step_rows = 1, int(self.lib.gitb200_stream_frames(self.h)) * self.T, 0
-        return tokens.clone(), logprobs.clone()
+        if sample is None:
+            return tokens.clone(), logprobs.clone()
+        return tokens.clone(), logprobs.clone(), logits[: self.last_decode_steps()] if logits is not None else None
 
     # ---- multi-stream pool: one window per camera, pushes and captions batched over cameras
     @staticmethod
@@ -404,23 +425,36 @@ class Engine:
         check(self.lib.gitb200_streams_push_u8(self.h, arr, k, _ptr(frames_u8), h, w, self._stream()), self.h,
               "gitb200_streams_push_u8")
 
-    def streams_caption(self, ids, sp: SearchConfig):
+    def streams_caption(self, ids, sp: SearchConfig, sample: Optional[SampleConfig] = None, keys=None,
+                        save_logits: bool = False):
         """Caption the windows of the streams ``ids`` (all holding the same number of frames) as one decode batch:
-        (tokens int32 [k, keep, max_steps], logprobs [k, keep]), row j = stream ids[j]."""
+        (tokens int32 [k, keep, max_steps], logprobs [k, keep]), row j = stream ids[j].
+
+        With ``sample`` (its seed is ignored), ``keys`` gives the Philox key of each stream (one int per id, required when
+        sampling; see model.stream_key) and the call returns (tokens [k*nrs, keep, max_steps], logprobs [k*nrs, keep],
+        logits or None): row j*nrs + r is sequence r of stream ids[j].  A stream's result depends on its window, its key,
+        the parameters and the number of rows in the call, not on the other streams or their order."""
         arr, k = self._ids(ids)
-        # persistent output buffers: identical call signatures let the library replay its captured CUDA graph
-        key = (k, sp.num_keep_best, sp.max_steps)
-        if not hasattr(self, "_streams_out"):
-            self._streams_out = {}
-        if key not in self._streams_out:
-            self._streams_out[key] = (torch.empty(k, sp.num_keep_best, sp.max_steps, dtype=torch.int32, device=self.device),
-                                      torch.empty(k, sp.num_keep_best, dtype=torch.float32, device=self.device))
-        tokens, logprobs = self._streams_out[key]
+        tokens, logprobs = self._window_outputs("_streams_out", k, sp, sample)
         c = sp.to_c()
-        check(self.lib.gitb200_streams_caption(self.h, arr, k, ctypes.byref(c), _ptr(tokens), _ptr(logprobs), self._stream()),
-              self.h, "gitb200_streams_caption")
+        if sample is None:
+            check(self.lib.gitb200_streams_caption(self.h, arr, k, ctypes.byref(c), _ptr(tokens), _ptr(logprobs),
+                                                   self._stream()), self.h, "gitb200_streams_caption")
+        else:
+            logits = self._saved_logits(tokens.shape[0], sp, save_logits, sample)
+            if keys is not None:
+                keys = [int(x) & (2 ** 64 - 1) for x in keys]
+                if len(keys) != k:
+                    raise GitB200Error(f"streams_caption: {len(keys)} keys for {k} stream ids")
+            key_arr = (ctypes.c_uint64 * k)(*keys) if keys is not None else None
+            x = sample.to_c()
+            check(self.lib.gitb200_streams_caption_ext(self.h, arr, k, ctypes.byref(c), ctypes.byref(x), key_arr, _ptr(tokens),
+                                                       _ptr(logprobs), _ptr(logits), self._stream()), self.h,
+                  "gitb200_streams_caption_ext")
         self._cur_clips, self._cur_nv, self._step_rows = k, self.streams_frames(int(ids[0])) * self.T, 0
-        return tokens.clone(), logprobs.clone()
+        if sample is None:
+            return tokens.clone(), logprobs.clone()
+        return tokens.clone(), logprobs.clone(), logits[: self.last_decode_steps()] if logits is not None else None
 
     def streams_reset(self, ids) -> None:
         arr, k = self._ids(ids)

@@ -18,6 +18,7 @@ Differences from the reference, all deliberate (DESIGN.md):
 """
 from __future__ import annotations
 
+import dataclasses
 import functools
 from typing import Callable, Dict, List, Optional, Sequence
 
@@ -753,15 +754,62 @@ class GenerativeImageTextTeacher(nn.Module):
         return tokens[:, 0].long()
 
 
+_M64 = 2 ** 64 - 1
+_SAMPLE_KEYS = ("do_sample", "top_k", "top_p", "temperature", "repetition_penalty", "num_return_sequences", "seed")
+
+
+def _splitmix64(x: int) -> int:
+    """splitmix64 (Steele, Lea, Flood 2014): a bijection of 64-bit words with full avalanche."""
+    z = (x + 0x9E3779B97F4A7C15) & _M64
+    z = ((z ^ (z >> 30)) * 0xBF58476D1CE4E5B9) & _M64
+    z = ((z ^ (z >> 27)) * 0x94D049BB133111EB) & _M64
+    return z ^ (z >> 31)
+
+
+def stream_key(seed: int, stream_id: int, n: int) -> int:
+    """The Philox key of camera ``stream_id``'s ``n``-th sampled caption (n = 0, 1, ...) under ``seed``:
+    splitmix64(splitmix64(seed) ^ ((stream_id + 1) << 32 | n)).  splitmix64 is a bijection, so under one seed two different
+    (stream_id, n) pairs never share a key (stream_id < 2^31 - 1, n < 2^32)."""
+    stream_id, n = int(stream_id), int(n)
+    if not (0 <= stream_id < 2 ** 31 - 1 and 0 <= n < 2 ** 32):
+        raise ValueError(f"stream_key: stream_id {stream_id} or caption count {n} out of range")
+    return _splitmix64(_splitmix64(int(seed) & _M64) ^ ((stream_id + 1) << 32 | n))
+
+
+def _sample_config(sample: Optional[dict]):
+    """The captioners' ``sample`` dict (search_param names) -> (SampleConfig, seed), or (None, None)."""
+    if sample is None:
+        return None, None
+    unknown = set(sample) - set(_SAMPLE_KEYS)
+    if unknown:
+        raise ValueError(f"unknown sample keys {sorted(unknown)} (expected some of {list(_SAMPLE_KEYS)})")
+    top_k, top_p = sample.get("top_k"), sample.get("top_p")
+    cfg = SampleConfig(bool(sample.get("do_sample", False)), int(top_k or 0), 1.0 if top_p is None else float(top_p),
+                       float(sample.get("temperature", 1.0)), float(sample.get("repetition_penalty", 1.0)),
+                       int(sample.get("num_return_sequences", 1)))
+    return cfg, int(sample.get("seed", 0))
+
+
+def _decode_rows(tokenizer, rows, nrs: int):
+    """Token rows [k*nrs, max_steps] -> k captions: a string each, or with nrs > 1 a list of nrs strings each."""
+    texts = [tokenizer.decode(r, skip_special_tokens=True) for r in rows]
+    return texts if nrs == 1 else [texts[i:i + nrs] for i in range(0, len(texts), nrs)]
+
+
 class StreamingCaptioner:
     """The webcam loop of src/real_time_inference.py:38-61 on the GPU: every `stride`-th frame is preprocessed
     (image_transform, :16-28) and its ViT features are computed as it arrives; once `window` frames are held the caption
     is decoded -- only ONE frame's ViT stands between the last frame and its caption.  ``sliding=False`` reproduces the
     reference (``frames.clear()`` after each caption, :61); ``sliding=True`` re-captions on every new frame with
-    per-frame feature reuse."""
+    per-frame feature reuse.
+
+    ``sample`` (a dict with search_param's names: do_sample, top_k, top_p, temperature, repetition_penalty,
+    num_return_sequences, seed) samples / penalises in the fused device search; the n-th caption draws with the key
+    ``stream_key(seed, 0, n)``, so every window gets fresh uniforms.  With num_return_sequences > 1 a caption is a list of
+    strings."""
 
     def __init__(self, teacher: GenerativeImageTextTeacher, stride: int = 3, max_len: int = 25, beam_size: int = 1,
-                 sliding: bool = False):
+                 sliding: bool = False, sample: Optional[dict] = None):
         from .engine import preprocess_frames
         self._pre = preprocess_frames
         self.teacher, self.stride, self.sliding = teacher, stride, sliding
@@ -771,6 +819,8 @@ class StreamingCaptioner:
         self.search = SearchConfig(beam_size=beam_size, max_steps=max_len + 1, length_penalty=d.length_penalty,
                                    per_node_beam_size=d.per_node_beam_size, num_keep_best=1)
         self._counter = 0
+        self.sample, self.seed = _sample_config(sample)
+        self._n_captions = 0
         self._raw, self._raw_key = None, None
         self.latest_caption = ""
         self.engine.stream_reset()
@@ -793,8 +843,14 @@ class StreamingCaptioner:
         held = self.engine.stream_push_u8(self._raw)
         if held < self.window:
             return None
-        tokens, _ = self.engine.stream_caption(self.search)
-        self.latest_caption = self.teacher.tokenizer.decode(tokens[0, 0].tolist(), skip_special_tokens=True)
+        if self.sample is None:
+            tokens, _ = self.engine.stream_caption(self.search)
+            self.latest_caption = self.teacher.tokenizer.decode(tokens[0, 0].tolist(), skip_special_tokens=True)
+        else:
+            x = dataclasses.replace(self.sample, seed=stream_key(self.seed, 0, self._n_captions))
+            self._n_captions += 1
+            tokens, _, _ = self.engine.stream_caption(self.search, sample=x)
+            self.latest_caption = _decode_rows(self.teacher.tokenizer, tokens[:, 0].tolist(), x.num_return_sequences)[0]
         if not self.sliding:
             self.engine.stream_reset()
         return self.latest_caption
@@ -807,10 +863,16 @@ class MultiStreamCaptioner:
     encoded as one ViT batch per frame size, and the windows that completed are captioned as one decode batch per
     held-frame count.  ``sliding=False`` reproduces the reference (``frames.clear()`` after each caption, :61);
     ``sliding=True`` re-captions a camera on every frame it pushes, reusing the other frames' features.
-    The constructor (re)configures the engine's pool: one captioner per engine."""
+    The constructor (re)configures the engine's pool: one captioner per engine.
+
+    ``sample`` (a dict with search_param's names: do_sample, top_k, top_p, temperature, repetition_penalty,
+    num_return_sequences, seed) samples / penalises in the pool's fused device search.  Each camera counts the captions it
+    has received since the captioner was built (``reset`` keeps the count), and camera i's n-th caption draws with the key
+    ``stream_key(seed, i, n)``: its samples depend neither on which cameras share a call nor on earlier windows' uniforms.
+    With num_return_sequences > 1 a camera's caption is a list of strings."""
 
     def __init__(self, teacher: GenerativeImageTextTeacher, n_streams: int, stride: int = 3, max_len: int = 25, beam_size: int = 1,
-                 sliding: bool = False):
+                 sliding: bool = False, sample: Optional[dict] = None):
         if n_streams < 1 or stride < 1:
             raise ValueError("n_streams and stride must be >= 1")
         self.teacher, self.n_streams, self.stride, self.sliding = teacher, n_streams, stride, sliding
@@ -820,6 +882,8 @@ class MultiStreamCaptioner:
         self.search = SearchConfig(beam_size=beam_size, max_steps=max_len + 1, length_penalty=d.length_penalty,
                                    per_node_beam_size=d.per_node_beam_size, num_keep_best=1)
         self._counter = [0] * n_streams
+        self.sample, self.seed = _sample_config(sample)
+        self._n_captions = [0] * n_streams
         self._raw = {}  # (k, H, W) -> persistent device buffer: repeated shapes replay the library's CUDA graphs
         self.latest_caption = [""] * n_streams
         self.engine.streams_configure(n_streams)
@@ -858,9 +922,17 @@ class MultiStreamCaptioner:
         ready = [sid for sid, _ in due if self.engine.streams_frames(sid) >= self.window]
         out = {}
         for _, ids in _group_by(ready, self.engine.streams_frames).items():
-            tokens, _ = self.engine.streams_caption(ids, self.search)
-            for sid, row in zip(ids, tokens[:, 0].tolist()):
-                out[sid] = self.latest_caption[sid] = self.teacher.tokenizer.decode(row, skip_special_tokens=True)
+            if self.sample is None:
+                tokens, _ = self.engine.streams_caption(ids, self.search)
+                captions = [self.teacher.tokenizer.decode(row, skip_special_tokens=True) for row in tokens[:, 0].tolist()]
+            else:
+                keys = [stream_key(self.seed, sid, self._n_captions[sid]) for sid in ids]
+                for sid in ids:
+                    self._n_captions[sid] += 1
+                tokens, _, _ = self.engine.streams_caption(ids, self.search, sample=self.sample, keys=keys)
+                captions = _decode_rows(self.teacher.tokenizer, tokens[:, 0].tolist(), self.sample.num_return_sequences)
+            for sid, caption in zip(ids, captions):
+                out[sid] = self.latest_caption[sid] = caption
             if not self.sliding:
                 self.engine.streams_reset(ids)
         return out
