@@ -261,6 +261,14 @@ int gitb200_stream_caption(gitb200_ctx* ctx, const gitb200_search_params* sp, in
  * enqueued. */
 int gitb200_stream_caption_ext(gitb200_ctx* ctx, const gitb200_search_params* sp, const gitb200_sample_params* sp_ext,
                                int32_t* tokens_dev, float* logprobs_dev, float* logits_dev, void* stream);
+/* gitb200_stream_caption with a prompt, prefix_host int32 [1, P] on the HOST (sp_ext may be NULL; with sampling its seed is the
+ * Philox key): the result equals gitb200_decode_prefix on the window's features, outputs and optional saved logits
+ * [max_steps-P, nrs*beam, logits_ld] as there; tokens include the prompt.  Rejections as gitb200_decode_prefix's for one
+ * clip, before anything is enqueued.  One window with beam <= 4, no sampling and no saved logits takes the persistent decode
+ * kernel from step P - 1.  The CUDA graph is keyed by P, not by the prompt's tokens. */
+int gitb200_stream_caption_prefix(gitb200_ctx* ctx, const gitb200_search_params* sp, const gitb200_sample_params* sp_ext,
+                                  const int32_t* prefix_host, int P, int32_t* tokens_dev, float* logprobs_dev,
+                                  float* logits_dev, void* stream);
 
 /* ---- multi-stream pool: many cameras on one context ------------------------------------------------------------
  * A pool of n_streams windows next to the single window above (which it does not touch), each window the same ring of
@@ -309,6 +317,21 @@ int gitb200_streams_caption(gitb200_ctx* ctx, const int32_t* ids_host, int k, co
 int gitb200_streams_caption_ext(gitb200_ctx* ctx, const int32_t* ids_host, int k, const gitb200_search_params* sp,
                                 const gitb200_sample_params* sp_ext, const uint64_t* keys_host, int32_t* tokens_dev,
                                 float* logprobs_dev, float* logits_dev, void* stream);
+/* Prompted captions of k windows: gitb200_decode_prefix (batch['prefix'], model.py:432-437) on the k windows' features.
+ * prefix_host int32 [prefix_rows, P] on the HOST, prefix_rows = 1 (one prompt for every stream) or k (row j is the prompt of
+ * stream ids_host[j]); every stream of one call has a prompt of the same length P (group cameras by prompt length as by
+ * held-frame count).  sp_ext may be NULL; with sampling, stream ids_host[j] draws with keys_host[j] at Philox step P - 1 as
+ * gitb200_streams_caption_ext draws without a prompt.  Outputs as gitb200_streams_caption_ext's, the tokens including the
+ * prompt, saved logits [max_steps-P, k*nrs*beam, logits_ld].  Everything is checked on the host before anything is enqueued:
+ * what gitb200_streams_caption_ext rejects and what gitb200_decode_prefix rejects for k clips; a rejected call changes no
+ * window.  The prompt and the key table are copied into context-owned device buffers before any graph launch, so the CUDA
+ * graphs (keyed by shape and P) replay for any prompt tokens, ids and keys.  One window with beam <= 4, no sampling and no
+ * saved logits takes the persistent decode kernel from step P - 1.  P = 1 with the SOS token gives exactly what
+ * gitb200_streams_caption / _ext give. */
+int gitb200_streams_caption_prefix(gitb200_ctx* ctx, const int32_t* ids_host, int k, const gitb200_search_params* sp,
+                                   const gitb200_sample_params* sp_ext, const uint64_t* keys_host, const int32_t* prefix_host,
+                                   int prefix_rows, int P, int32_t* tokens_dev, float* logprobs_dev, float* logits_dev,
+                                   void* stream);
 /* Empties the windows of k distinct streams (the reference's frames.clear() after a caption, real_time_inference.py:61). */
 int gitb200_streams_reset(gitb200_ctx* ctx, const int32_t* ids_host, int k);
 /* Frames held by one stream's window (0 .. num_image_with_embedding); GITB200_ERR_INVALID for an unknown id. */

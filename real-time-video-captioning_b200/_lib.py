@@ -117,12 +117,16 @@ SIGNATURES = {
     "gitb200_stream_caption": (c_int, [c_void_p, POINTER(SearchParams), c_void_p, c_void_p, c_void_p]),
     "gitb200_stream_caption_ext": (c_int, [c_void_p, POINTER(SearchParams), POINTER(SampleParams), c_void_p, c_void_p, c_void_p,
                                            c_void_p]),
+    "gitb200_stream_caption_prefix": (c_int, [c_void_p, POINTER(SearchParams), POINTER(SampleParams), c_void_p, c_int, c_void_p,
+                                              c_void_p, c_void_p, c_void_p]),
     "gitb200_streams_configure": (c_int, [c_void_p, c_int]),
     "gitb200_streams_push": (c_int, [c_void_p, c_void_p, c_int, c_void_p, c_void_p]),
     "gitb200_streams_push_u8": (c_int, [c_void_p, c_void_p, c_int, c_void_p, c_int, c_int, c_void_p]),
     "gitb200_streams_caption": (c_int, [c_void_p, c_void_p, c_int, POINTER(SearchParams), c_void_p, c_void_p, c_void_p]),
     "gitb200_streams_caption_ext": (c_int, [c_void_p, c_void_p, c_int, POINTER(SearchParams), POINTER(SampleParams), c_void_p,
                                             c_void_p, c_void_p, c_void_p, c_void_p]),
+    "gitb200_streams_caption_prefix": (c_int, [c_void_p, c_void_p, c_int, POINTER(SearchParams), POINTER(SampleParams), c_void_p,
+                                               c_void_p, c_int, c_int, c_void_p, c_void_p, c_void_p, c_void_p]),
     "gitb200_streams_reset": (c_int, [c_void_p, c_void_p, c_int]),
     "gitb200_streams_frames": (c_int, [c_void_p, c_int]),
     "gitb200_streams_window": (c_int, [c_void_p, c_int, c_void_p, c_void_p]),

@@ -1532,6 +1532,13 @@ static int caption_eager(gitb200_ctx* c, const float* frames, int n_clips, int n
   return gitb200_decode(c, sp, tokens, logprobs, logits, stream);
 }
 
+// Decode steps a replayed whole-call graph ran: a graph is captured without the early-exit poll, so every step from the search's
+// first cur_len (P with a prompt, 1 without) to max_steps.
+static int replayed_decode_steps(const gitb200_search_params& sp, int P) {
+  const int first = P > 0 ? P : 1;
+  return sp.max_steps > first ? sp.max_steps - first : 0;
+}
+
 // gitb200_caption (smp == nullptr) and gitb200_caption_ext with active sampling parameters (the seed already in seed_dev);
 // P > 0: gitb200_caption_prefix (the prompt already in prefix_dev, see run_decode)
 static int caption_impl(gitb200_ctx* c, const float* frames, int n_clips, int n_frames, const gitb200_search_params* sp,
@@ -1552,8 +1559,7 @@ static int caption_impl(gitb200_ctx* c, const float* frames, int n_clips, int n_
     if (r == 1) {  // replayed: host-side state the eager path would have left behind
       const int F = (c->cfg.num_image_with_embedding > 0 && n_frames > c->cfg.num_image_with_embedding) ? c->cfg.num_image_with_embedding : n_frames;
       c->cur_clips = n_clips; c->cur_nv = F * c->T; c->visual_pass_done = true; c->visual_pass_full = 0; c->step_rows_per_clip = 0;
-      const int first = P > 0 ? P : 1;  // the search's first cur_len
-      c->last_decode_steps = sp->max_steps > first ? sp->max_steps - first : 0;
+      c->last_decode_steps = replayed_decode_steps(*sp, P);
       return GITB200_OK;
     }
     return r;
@@ -1796,14 +1802,15 @@ int gitb200_stream_push_u8(gitb200_ctx* c, const uint8_t* frame, int height, int
 
 int gitb200_stream_frames(const gitb200_ctx* c) { return c ? c->ring_count : 0; }
 
-// gitb200_stream_caption (smp == nullptr) and gitb200_stream_caption_ext (the seed already in seed_dev when smp is active)
+// gitb200_stream_caption (smp == nullptr) and gitb200_stream_caption_ext (the seed already in seed_dev when smp is active);
+// P > 0: gitb200_stream_caption_prefix (the prompt already in prefix_dev, see run_decode)
 static int stream_caption_impl(gitb200_ctx* c, const gitb200_search_params* sp, const gitb200_sample_params* smp, int32_t* tokens,
-                               float* logprobs, float* logits, cudaStream_t s) {
+                               float* logprobs, float* logits, cudaStream_t s, int P = 0) {
   const int cap = c->cfg.num_image_with_embedding, n = c->ring_count, T = c->T, W = c->cfg.vit_width;
   ENSURE(c, c->vf, (size_t)n * T * W);
   const int first = (c->ring_head - n + cap) % cap;  // oldest frame -> temporal position 0
   gitb200_ctx::GraphKey key;
-  key.kind = 2; key.p0 = tokens; key.p1 = logprobs; key.i0 = n; key.i1 = first; key.sp = *sp;
+  key.kind = 2; key.p0 = tokens; key.p1 = logprobs; key.i0 = n; key.i1 = first; key.i2 = P; key.sp = *sp;
   if (smp) {
     key.smp = *smp;
     key.smp.seed = 0;
@@ -1815,10 +1822,11 @@ static int stream_caption_impl(gitb200_ctx* c, const gitb200_search_params* sp, 
     c->cur_nv = n * T;
     c->visual_pass_done = false;
     c->step_rows_per_clip = 0;
-    return run_decode(c, *sp, tokens, logprobs, logits, s, smp);
+    return run_decode(c, *sp, tokens, logprobs, logits, s, smp, P);
   });
   if (r == 1) {
     c->cur_clips = 1; c->cur_nv = n * T; c->visual_pass_done = true; c->visual_pass_full = 0; c->step_rows_per_clip = 0;
+    c->last_decode_steps = replayed_decode_steps(*sp, P);
     return GITB200_OK;
   }
   return r;
@@ -1843,6 +1851,22 @@ int gitb200_stream_caption_ext(gitb200_ctx* c, const gitb200_search_params* sp, 
   cudaStream_t s = caller_stream(c, stream);
   if (active) TRY(upload_seed(c, smp->seed, s));
   return stream_caption_impl(c, sp, active ? smp : nullptr, tokens, logprobs, logits, s);
+}
+
+int gitb200_stream_caption_prefix(gitb200_ctx* c, const gitb200_search_params* sp, const gitb200_sample_params* smp,
+                                  const int32_t* prefix_host, int P, int32_t* tokens, float* logprobs, float* logits, void* stream) {
+  if (!c || !sp || !tokens || !logprobs) return fail(c, GITB200_ERR_INVALID, "bad stream_caption_prefix argument");
+  if (!c->finalized) return fail(c, GITB200_ERR_STATE, "call gitb200_finalize_weights first");
+  const gitb200_sample_params& x = smp ? *smp : kDefaultSample;
+  TRY(check_sample(c, *sp, x, c->cfg.vocab, 1, c->cfg.max_positions, true));
+  if (c->ring_count < 1) return fail(c, GITB200_ERR_STATE, "no frames in the streaming window: call gitb200_stream_push first");
+  TRY(check_prefix(c, prefix_host, 1, P, 1, c->cfg.vocab, c->cfg.max_positions));
+  CUDA_OK(c, cudaSetDevice(c->device));
+  cudaStream_t s = caller_stream(c, stream);
+  const bool active = sample_active(x);
+  if (active) TRY(upload_seed(c, x.seed, s));
+  TRY(upload_prefix(c, prefix_host, 1, P, 1, s));
+  return stream_caption_impl(c, sp, active ? &x : nullptr, tokens, logprobs, logits, s, P);
 }
 
 // ---- multi-stream pool: one window per camera stream, pushes and captions batched over streams
@@ -1955,10 +1979,12 @@ static int pool_check_held(gitb200_ctx* c, const char* what, const int32_t* ids,
 }
 
 // gitb200_streams_caption (smp == nullptr) and gitb200_streams_caption_ext (smp active; keys_host: one Philox key per id when
-// smp->do_sample).  Everything is validated by the caller.
+// smp->do_sample); P > 0: gitb200_streams_caption_prefix (prefix_host [prefix_rows][P], copied into prefix_dev before any
+// graph launch, see run_decode).  Everything is validated by the caller.
 static int streams_caption_impl(gitb200_ctx* c, const int32_t* ids, int k, const gitb200_search_params* sp,
                                 const gitb200_sample_params* smp, const uint64_t* keys_host, int32_t* tokens, float* logprobs,
-                                float* logits, void* stream) {
+                                float* logits, void* stream, const int32_t* prefix_host = nullptr, int prefix_rows = 0,
+                                int P = 0) {
   const int n = c->pool_count[ids[0]];
   CUDA_OK(c, cudaSetDevice(c->device));
   const cudaStream_t s = (cudaStream_t)stream;
@@ -1975,13 +2001,14 @@ static int streams_caption_impl(gitb200_ctx* c, const int32_t* ids, int k, const
     CUDA_OK(c, cudaMemcpyAsync(c->pool_keys.p, keys_host, (size_t)k * sizeof(unsigned long long), cudaMemcpyHostToDevice, s));
     keys = c->pool_keys.p;
   }
+  if (P > 0) TRY(upload_prefix(c, prefix_host, prefix_rows, P, k, s));
   auto assemble = [&]() -> int {
     CUDA_OK(c, assemble_windows(c->pool.p, c->pool_oldest.p, 0, k, n, cap, T, W, c->temporal, c->vf.p, nullptr, s));
     c->cur_clips = k; c->cur_nv = n * T; c->visual_pass_done = false; c->step_rows_per_clip = 0;
     return 0;
   };
   gitb200_ctx::GraphKey key;
-  key.i0 = k; key.i1 = n;
+  key.i0 = k; key.i1 = n; key.i2 = P;
   if (k <= c->graph_max_clips) {  // latency mode: the whole call as one graph (k == 1, beam <= 4: the persistent decode kernel)
     key.kind = 12; key.p0 = tokens; key.p1 = logprobs; key.sp = *sp;
     if (smp) {  // the keys and the seed are read from device tables: the graph replays for any of them
@@ -1991,11 +2018,11 @@ static int streams_caption_impl(gitb200_ctx* c, const int32_t* ids, int k, const
     // saved logits: eager (the step loop's early exit decides how many steps they hold, as in gitb200_decode)
     const int r = run_graphed(c, key, s, logits == nullptr, [&]() -> int {
       TRY(assemble());
-      return run_decode(c, *sp, tokens, logprobs, logits, s, smp, 0, keys);
+      return run_decode(c, *sp, tokens, logprobs, logits, s, smp, P, keys);
     });
     if (r == 1) {  // replayed: host-side state the eager run would have left
       c->cur_clips = k; c->cur_nv = n * T; c->visual_pass_done = true; c->visual_pass_full = 0; c->step_rows_per_clip = 0;
-      c->last_decode_steps = sp->max_steps - 1;
+      c->last_decode_steps = replayed_decode_steps(*sp, P);
       return GITB200_OK;
     }
     return r;
@@ -2011,7 +2038,7 @@ static int streams_caption_impl(gitb200_ctx* c, const int32_t* ids, int k, const
   } else if (r != 0) {
     return r;
   }
-  return run_decode(c, *sp, tokens, logprobs, logits, s, smp, 0, keys);
+  return run_decode(c, *sp, tokens, logprobs, logits, s, smp, P, keys);
 }
 
 int gitb200_streams_caption(gitb200_ctx* c, const int32_t* ids, int k, const gitb200_search_params* sp, int32_t* tokens,
@@ -2038,6 +2065,25 @@ int gitb200_streams_caption_ext(gitb200_ctx* c, const int32_t* ids, int k, const
   const bool active = sample_active(*smp);
   if (!active && logits == nullptr) return gitb200_streams_caption(c, ids, k, sp, tokens, logprobs, stream);
   return streams_caption_impl(c, ids, k, sp, active ? smp : nullptr, keys_host, tokens, logprobs, logits, stream);
+}
+
+int gitb200_streams_caption_prefix(gitb200_ctx* c, const int32_t* ids, int k, const gitb200_search_params* sp,
+                                   const gitb200_sample_params* smp, const uint64_t* keys_host, const int32_t* prefix_host,
+                                   int prefix_rows, int P, int32_t* tokens, float* logprobs, float* logits, void* stream) {
+  const char* what = "gitb200_streams_caption_prefix";
+  if (!c) return GITB200_ERR_INVALID;
+  if (!sp || !tokens || !logprobs) return fail(c, GITB200_ERR_INVALID, "%s: bad argument", what);
+  if (!c->finalized) return fail(c, GITB200_ERR_STATE, "call gitb200_finalize_weights first");
+  TRY(pool_check_ids(c, what, ids, k));
+  TRY(pool_check_held(c, what, ids, k));
+  const gitb200_sample_params& x = smp ? *smp : kDefaultSample;
+  TRY(check_sample(c, *sp, x, c->cfg.vocab, k, c->cfg.max_positions, true));
+  if (x.do_sample && keys_host == nullptr)
+    return fail(c, GITB200_ERR_INVALID, "%s: keys_host is NULL while do_sample is set (one Philox key per stream id)", what);
+  TRY(check_prefix(c, prefix_host, prefix_rows, P, k, c->cfg.vocab, c->cfg.max_positions));
+  const bool active = sample_active(x);
+  return streams_caption_impl(c, ids, k, sp, active ? &x : nullptr, keys_host, tokens, logprobs, logits, stream, prefix_host,
+                              prefix_rows, P);
 }
 
 int gitb200_streams_reset(gitb200_ctx* c, const int32_t* ids, int k) {

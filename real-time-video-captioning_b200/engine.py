@@ -372,19 +372,31 @@ class Engine:
                          torch.empty(n, sp.num_keep_best, dtype=torch.float32, device=self.device))
         return bufs[key]
 
-    def _saved_logits(self, n_rows: int, sp: SearchConfig, save_logits: bool, sample: Optional[SampleConfig]):
+    def _saved_logits(self, n_rows: int, sp: SearchConfig, save_logits: bool, sample: Optional[SampleConfig], P: int = 1):
         if save_logits and sample is None:
             raise GitB200Error("save_logits needs sample (a SampleConfig; SampleConfig() for plain beam search)")
-        return torch.empty(sp.max_steps - 1, n_rows * sp.beam_size, self.ld, dtype=torch.float32,
+        return torch.empty(max(0, sp.max_steps - P), n_rows * sp.beam_size, self.ld, dtype=torch.float32,
                            device=self.device) if save_logits else None
 
-    def stream_caption(self, sp: SearchConfig, sample: Optional[SampleConfig] = None, save_logits: bool = False):
+    def stream_caption(self, sp: SearchConfig, sample: Optional[SampleConfig] = None, save_logits: bool = False,
+                       prefix: Optional[torch.Tensor] = None):
         """Caption the single streaming window: (tokens int32 [1, keep, max_steps], logprobs [1, keep]).  With ``sample``
         (its seed is the Philox key) the result equals ``decode(1, sp, sample=sample)`` on the window's features and the
-        call returns (tokens [nrs, keep, max_steps], logprobs [nrs, keep], logits or None) as ``decode`` does."""
+        call returns (tokens [nrs, keep, max_steps], logprobs [nrs, keep], logits or None) as ``decode`` does.
+        ``prefix`` (batch['prefix'], int [1, P], host or device): the result equals ``decode(1, sp, prefix=prefix)`` on the
+        window's features (the tokens include the prompt, the logits hold max_steps - P steps); the return form is the same."""
         tokens, logprobs = self._window_outputs("_stream_out", 1, sp, sample)
         c = sp.to_c()
-        if sample is None:
+        if prefix is not None:
+            pre = _prefix_host(prefix)
+            if pre.shape[0] != 1:
+                raise GitB200Error(f"stream_caption: prefix must have one row (got {pre.shape[0]})")
+            logits = self._saved_logits(tokens.shape[0], sp, save_logits, sample, pre.shape[1])
+            x = sample.to_c() if sample is not None else None
+            check(self.lib.gitb200_stream_caption_prefix(self.h, ctypes.byref(c), ctypes.byref(x) if x is not None else None,
+                                                         _ptr(pre), pre.shape[1], _ptr(tokens), _ptr(logprobs), _ptr(logits),
+                                                         self._stream()), self.h, "gitb200_stream_caption_prefix")
+        elif sample is None:
             check(self.lib.gitb200_stream_caption(self.h, ctypes.byref(c), _ptr(tokens), _ptr(logprobs), self._stream()), self.h,
                   "gitb200_stream_caption")
         else:
@@ -425,28 +437,45 @@ class Engine:
         check(self.lib.gitb200_streams_push_u8(self.h, arr, k, _ptr(frames_u8), h, w, self._stream()), self.h,
               "gitb200_streams_push_u8")
 
+    @staticmethod
+    def _keys(keys, k: int):
+        if keys is None:
+            return None
+        keys = [int(x) & (2 ** 64 - 1) for x in keys]
+        if len(keys) != k:
+            raise GitB200Error(f"streams_caption: {len(keys)} keys for {k} stream ids")
+        return (ctypes.c_uint64 * k)(*keys)
+
     def streams_caption(self, ids, sp: SearchConfig, sample: Optional[SampleConfig] = None, keys=None,
-                        save_logits: bool = False):
+                        save_logits: bool = False, prefix: Optional[torch.Tensor] = None):
         """Caption the windows of the streams ``ids`` (all holding the same number of frames) as one decode batch:
         (tokens int32 [k, keep, max_steps], logprobs [k, keep]), row j = stream ids[j].
 
         With ``sample`` (its seed is ignored), ``keys`` gives the Philox key of each stream (one int per id, required when
         sampling; see model.stream_key) and the call returns (tokens [k*nrs, keep, max_steps], logprobs [k*nrs, keep],
         logits or None): row j*nrs + r is sequence r of stream ids[j].  A stream's result depends on its window, its key,
-        the parameters and the number of rows in the call, not on the other streams or their order."""
+        the parameters and the number of rows in the call, not on the other streams or their order.
+
+        ``prefix`` (batch['prefix'], int [1 or k, P], host or device; row j is the prompt of stream ids[j]): the result
+        equals ``decode(k, sp, sample=..., prefix=prefix)`` on the windows' features, each stream drawing with its key;
+        the tokens include the prompt and the logits hold max_steps - P steps.  The return form is the same as without it."""
         arr, k = self._ids(ids)
         tokens, logprobs = self._window_outputs("_streams_out", k, sp, sample)
         c = sp.to_c()
-        if sample is None:
+        if prefix is not None:
+            pre = _prefix_host(prefix)
+            logits = self._saved_logits(tokens.shape[0], sp, save_logits, sample, pre.shape[1])
+            x = sample.to_c() if sample is not None else None
+            check(self.lib.gitb200_streams_caption_prefix(self.h, arr, k, ctypes.byref(c), ctypes.byref(x) if x is not None else None,
+                                                          self._keys(keys, k), _ptr(pre), pre.shape[0], pre.shape[1], _ptr(tokens),
+                                                          _ptr(logprobs), _ptr(logits), self._stream()), self.h,
+                  "gitb200_streams_caption_prefix")
+        elif sample is None:
             check(self.lib.gitb200_streams_caption(self.h, arr, k, ctypes.byref(c), _ptr(tokens), _ptr(logprobs),
                                                    self._stream()), self.h, "gitb200_streams_caption")
         else:
             logits = self._saved_logits(tokens.shape[0], sp, save_logits, sample)
-            if keys is not None:
-                keys = [int(x) & (2 ** 64 - 1) for x in keys]
-                if len(keys) != k:
-                    raise GitB200Error(f"streams_caption: {len(keys)} keys for {k} stream ids")
-            key_arr = (ctypes.c_uint64 * k)(*keys) if keys is not None else None
+            key_arr = self._keys(keys, k)
             x = sample.to_c()
             check(self.lib.gitb200_streams_caption_ext(self.h, arr, k, ctypes.byref(c), ctypes.byref(x), key_arr, _ptr(tokens),
                                                        _ptr(logprobs), _ptr(logits), self._stream()), self.h,

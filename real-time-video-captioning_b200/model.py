@@ -790,6 +790,34 @@ def _sample_config(sample: Optional[dict]):
     return cfg, int(sample.get("seed", 0))
 
 
+def _prompt_ids(prompt, vocab: int, max_steps: int):
+    """A camera's prompt (token ids starting with SOS, as one row of batch['prefix']: a list, a 1-D tensor or a [1, P] tensor)
+    -> a tuple of ints, or None for None.  Rejects an empty prompt, a token outside [0, vocab) and a prompt that leaves the
+    search no step (P >= max_steps = max_len + 1)."""
+    if prompt is None:
+        return None
+    if isinstance(prompt, torch.Tensor):
+        if prompt.dtype.is_floating_point or prompt.dtype.is_complex or prompt.dtype == torch.bool:
+            raise ValueError(f"prompt must hold integer token ids (got {prompt.dtype})")
+        if prompt.dim() == 2 and prompt.shape[0] == 1:
+            prompt = prompt[0]
+        if prompt.dim() != 1:
+            raise ValueError(f"prompt must be one row of token ids (got shape {tuple(prompt.shape)})")
+        ids = tuple(int(t) for t in prompt.tolist())
+    else:
+        ids = tuple(prompt)
+        if not all(isinstance(t, int) and not isinstance(t, bool) for t in ids):
+            raise ValueError(f"prompt must hold integer token ids (got {prompt!r})")
+    if not ids:
+        raise ValueError("prompt must hold at least one token (start it with SOS)")
+    bad = [t for t in ids if not 0 <= t < vocab]
+    if bad:
+        raise ValueError(f"prompt token {bad[0]} lies outside the vocabulary [0, {vocab})")
+    if len(ids) >= max_steps:
+        raise ValueError(f"a prompt of {len(ids)} tokens leaves no caption token within max_len {max_steps - 1}")
+    return ids
+
+
 def _decode_rows(tokenizer, rows, nrs: int):
     """Token rows [k*nrs, max_steps] -> k captions: a string each, or with nrs > 1 a list of nrs strings each."""
     texts = [tokenizer.decode(r, skip_special_tokens=True) for r in rows]
@@ -806,10 +834,14 @@ class StreamingCaptioner:
     ``sample`` (a dict with search_param's names: do_sample, top_k, top_p, temperature, repetition_penalty,
     num_return_sequences, seed) samples / penalises in the fused device search; the n-th caption draws with the key
     ``stream_key(seed, 0, n)``, so every window gets fresh uniforms.  With num_return_sequences > 1 a caption is a list of
-    strings."""
+    strings.
+
+    ``prompt`` (token ids starting with SOS, as one row of batch['prefix']) starts every caption's search from that prompt,
+    e.g. a question; the caption is the text after it (the reference's strip, ``predicted[:, P:]``).  ``set_prompt``
+    changes or clears it."""
 
     def __init__(self, teacher: GenerativeImageTextTeacher, stride: int = 3, max_len: int = 25, beam_size: int = 1,
-                 sliding: bool = False, sample: Optional[dict] = None):
+                 sliding: bool = False, sample: Optional[dict] = None, prompt=None):
         from .engine import preprocess_frames
         self._pre = preprocess_frames
         self.teacher, self.stride, self.sliding = teacher, stride, sliding
@@ -823,7 +855,12 @@ class StreamingCaptioner:
         self._n_captions = 0
         self._raw, self._raw_key = None, None
         self.latest_caption = ""
+        self.set_prompt(prompt)
         self.engine.stream_reset()
+
+    def set_prompt(self, prompt) -> None:
+        """The prompt of the following captions (None: none); checked here, before any frame is captioned."""
+        self.prompt = _prompt_ids(prompt, self.engine.cfg.vocab, self.search.max_steps) if prompt is not None else None
 
     @torch.no_grad()
     def push(self, frame_bgr_u8: torch.Tensor) -> Optional[str]:
@@ -843,14 +880,16 @@ class StreamingCaptioner:
         held = self.engine.stream_push_u8(self._raw)
         if held < self.window:
             return None
+        P = len(self.prompt) if self.prompt is not None else 0
+        kw = {"prefix": torch.tensor([self.prompt], dtype=torch.int32)} if self.prompt is not None else {}
         if self.sample is None:
-            tokens, _ = self.engine.stream_caption(self.search)
-            self.latest_caption = self.teacher.tokenizer.decode(tokens[0, 0].tolist(), skip_special_tokens=True)
+            tokens, _ = self.engine.stream_caption(self.search, **kw)
+            self.latest_caption = self.teacher.tokenizer.decode(tokens[0, 0, P:].tolist(), skip_special_tokens=True)
         else:
             x = dataclasses.replace(self.sample, seed=stream_key(self.seed, 0, self._n_captions))
             self._n_captions += 1
-            tokens, _, _ = self.engine.stream_caption(self.search, sample=x)
-            self.latest_caption = _decode_rows(self.teacher.tokenizer, tokens[:, 0].tolist(), x.num_return_sequences)[0]
+            tokens, _, _ = self.engine.stream_caption(self.search, sample=x, **kw)
+            self.latest_caption = _decode_rows(self.teacher.tokenizer, tokens[:, 0, P:].tolist(), x.num_return_sequences)[0]
         if not self.sliding:
             self.engine.stream_reset()
         return self.latest_caption
@@ -869,10 +908,16 @@ class MultiStreamCaptioner:
     num_return_sequences, seed) samples / penalises in the pool's fused device search.  Each camera counts the captions it
     has received since the captioner was built (``reset`` keeps the count), and camera i's n-th caption draws with the key
     ``stream_key(seed, i, n)``: its samples depend neither on which cameras share a call nor on earlier windows' uniforms.
-    With num_return_sequences > 1 a camera's caption is a list of strings."""
+    With num_return_sequences > 1 a camera's caption is a list of strings.
+
+    ``prompt`` (token ids starting with SOS, as one row of batch['prefix']) is every camera's default prompt, e.g. a
+    question; ``set_prompt(id, prompt)`` gives one camera its own (None: none).  A prompted caption is the text after the
+    prompt (the reference's strip, ``predicted[:, P:]``).  The windows due are captioned as one pool call per (held frames,
+    prompt length), with the group's prompts as a [k, P] prefix; cameras without a prompt make exactly the calls they make
+    without this option."""
 
     def __init__(self, teacher: GenerativeImageTextTeacher, n_streams: int, stride: int = 3, max_len: int = 25, beam_size: int = 1,
-                 sliding: bool = False, sample: Optional[dict] = None):
+                 sliding: bool = False, sample: Optional[dict] = None, prompt=None):
         if n_streams < 1 or stride < 1:
             raise ValueError("n_streams and stride must be >= 1")
         self.teacher, self.n_streams, self.stride, self.sliding = teacher, n_streams, stride, sliding
@@ -886,7 +931,16 @@ class MultiStreamCaptioner:
         self._n_captions = [0] * n_streams
         self._raw = {}  # (k, H, W) -> persistent device buffer: repeated shapes replay the library's CUDA graphs
         self.latest_caption = [""] * n_streams
+        prompt = _prompt_ids(prompt, self.engine.cfg.vocab, self.search.max_steps) if prompt is not None else None
+        self._prompts = [prompt] * n_streams
         self.engine.streams_configure(n_streams)
+
+    def set_prompt(self, stream_id: int, prompt) -> None:
+        """Camera ``stream_id``'s prompt for its following captions (None: none); checked here, before any frame is captioned."""
+        if not 0 <= stream_id < self.n_streams:
+            raise KeyError(f"unknown stream id {stream_id} (this captioner has ids 0..{self.n_streams - 1})")
+        self._prompts[stream_id] = (_prompt_ids(prompt, self.engine.cfg.vocab, self.search.max_steps)
+                                    if prompt is not None else None)
 
     def reset(self, stream_ids) -> None:
         """Empty the windows (and stride counters) of these cameras, e.g. after a scene cut or a reconnect."""
@@ -921,16 +975,21 @@ class MultiStreamCaptioner:
             self.engine.streams_push_u8(ids, buf)
         ready = [sid for sid, _ in due if self.engine.streams_frames(sid) >= self.window]
         out = {}
-        for _, ids in _group_by(ready, self.engine.streams_frames).items():
+        def group(sid):
+            p = self._prompts[sid]
+            return self.engine.streams_frames(sid), len(p) if p is not None else 0
+
+        for (_, P), ids in _group_by(ready, group).items():
+            kw = {"prefix": torch.tensor([self._prompts[sid] for sid in ids], dtype=torch.int32)} if P else {}
             if self.sample is None:
-                tokens, _ = self.engine.streams_caption(ids, self.search)
-                captions = [self.teacher.tokenizer.decode(row, skip_special_tokens=True) for row in tokens[:, 0].tolist()]
+                tokens, _ = self.engine.streams_caption(ids, self.search, **kw)
+                captions = [self.teacher.tokenizer.decode(row, skip_special_tokens=True) for row in tokens[:, 0, P:].tolist()]
             else:
                 keys = [stream_key(self.seed, sid, self._n_captions[sid]) for sid in ids]
                 for sid in ids:
                     self._n_captions[sid] += 1
-                tokens, _, _ = self.engine.streams_caption(ids, self.search, sample=self.sample, keys=keys)
-                captions = _decode_rows(self.teacher.tokenizer, tokens[:, 0].tolist(), self.sample.num_return_sequences)
+                tokens, _, _ = self.engine.streams_caption(ids, self.search, sample=self.sample, keys=keys, **kw)
+                captions = _decode_rows(self.teacher.tokenizer, tokens[:, 0, P:].tolist(), self.sample.num_return_sequences)
             for sid, caption in zip(ids, captions):
                 out[sid] = self.latest_caption[sid] = caption
             if not self.sliding:
